@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU path
+    python bench.py ... --dump-outputs DIR                    # also write a sample of the last step's PCM
 
 For N > 1 the driver launches it under torchrun (one rank per GPU, NCCL); RANK /
 LOCAL_RANK / WORLD_SIZE come from the environment.  One JSON line is printed by rank 0.
@@ -64,7 +65,42 @@ def parse_args():
     ap.add_argument("--no-extras", action="store_true", help="skip the mixed / worst-case legs (N=1 only)")
     ap.add_argument("--strong", action="store_true", help="strong scaling: --captures is the TOTAL, split over the ranks")
     ap.add_argument("--no-long", action="store_true", help="skip the one-hour time-sharded capture (BASELINE configs[4])")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed, seeded sample of the last timed step's PCM to DIR/pcm.npy (with its "
+                         "[capture, sample] positions in DIR/pcm_index.npy), so that two builds can be compared")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the CUDA path's PCM; --impl reference keeps none")
+    return args
+
+
+# at most this many PCM samples are dumped: 8 MB of float32 values + 32 MB of float64 positions
+DUMP_SAMPLES = 1 << 21
+DUMP_SEED = 20241020
+
+
+def dump_pcm_sample(np, torch, bufs, out_dir):
+    """Write a seeded sample of the PCM in `bufs` (a list of [C, n] int16 device tensors, read as one array of
+    len(bufs) * C rows) as float32 to out_dir/pcm.npy and its (row, sample) positions as float64 to
+    out_dir/pcm_index.npy.  The positions depend only on the shape, so runs of the same arguments line up."""
+    rows, n = sum(b.shape[0] for b in bufs), bufs[0].shape[1]
+    total = rows * n
+    k = min(total, DUMP_SAMPLES)
+    # one position drawn in each of k equal strata: sorted, distinct, O(k) memory whatever the total
+    edges = np.arange(k + 1, dtype=np.int64) * total // k
+    flat = edges[:-1] + (np.random.default_rng(DUMP_SEED).random(k) * np.diff(edges)).astype(np.int64)
+    vals, r0 = [], 0
+    for b in bufs:
+        sel = flat[(flat >= r0 * n) & (flat < (r0 + b.shape[0]) * n)] - r0 * n
+        idx = torch.from_numpy(sel).to(b.device)
+        vals.append(b.reshape(-1)[idx].float().cpu().numpy())
+        r0 += b.shape[0]
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "pcm.npy", np.concatenate(vals).astype(np.float32))
+    np.save(out / "pcm_index.npy", np.stack([flat // n, flat % n], axis=1).astype(np.float64))
 
 
 def workload_name(captures, seconds):
@@ -449,6 +485,8 @@ def main_b200(args):
     drain()
     ms_step, kern, launches, clk, pcm = timed_steps(args.steps, with_clocks=True)
     value = world * samples_per_step / (ms_step * 1e-3) / 1e6
+    if args.dump_outputs and rank == 0:                   # before the legs below reuse the PCM buffers
+        dump_pcm_sample(np, torch, [pcm] if world == 1 else [g.view(torch.int16) for g in gathered], args.dump_outputs)
     pcm_main = pcm.clone() if world > 1 else pcm          # (double-buffered: keep the last step's result)
 
     # ---- end to end through fmrx_process(): pinned host in, pinned host out ----

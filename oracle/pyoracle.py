@@ -46,9 +46,28 @@ def build_port(force: bool = False) -> Path:
     return PORT_SO
 
 
+def reference_missing_reason() -> str | None:
+    """Why the reference cannot be used here, or None when it can."""
+    if REF_SO.exists():
+        return None
+    try:
+        if (REF_ROOT / "src" / "filter.cpp").is_file():
+            return None
+    except OSError as e:                  # e.g. a checkout the current user may not read
+        return f"{REF_ROOT} is not readable ({e.strerror}) and oracle/_ref is not built"
+    return f"no reference sources under {REF_ROOT} and oracle/_ref is not built"
+
+
+def _reference_sources_present() -> bool:
+    try:
+        return (REF_ROOT / "src" / "filter.cpp").is_file()
+    except OSError:
+        return False
+
+
 def build_reference() -> Path | None:
     """Compile the reference where it lies (only when it is present)."""
-    if (REF_ROOT / "src" / "filter.cpp").exists():
+    if _reference_sources_present():
         subprocess.run(["make", "-s", "-C", str(HERE), "ref", f"REF={REF_ROOT}"],
                        check=True, stdout=subprocess.DEVNULL)
     return REF_SO if REF_SO.exists() else None
@@ -289,7 +308,7 @@ class Reference(_OpsMixin):
 
     @staticmethod
     def available() -> bool:
-        return REF_SO.exists() or (REF_ROOT / "src" / "filter.cpp").exists()
+        return reference_missing_reason() is None
 
     def pll(self, x, freq, Fs, scale, phase_adjust, norm_bw, state=None):
         """Returns (nco, None, new_state) -- the reference exposes no trigArg."""

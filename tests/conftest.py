@@ -53,9 +53,14 @@ def port():
 
 @pytest.fixture(scope="session")
 def reference():
+    """The reference's own compiled code, or None: then tests/reference_vectors.py compares with what it
+    computed, stored in tests/golden/reference_vectors.npz."""
+    import warnings
     import pyoracle
-    if not pyoracle.Reference.available():
-        pytest.skip("oracle/_ref not built and no reference checkout on this box")
+    why = pyoracle.reference_missing_reason()
+    if why is not None:
+        warnings.warn(f"reference not available ({why}): comparing with the stored reference vectors")
+        return None
     return pyoracle.Reference()
 
 

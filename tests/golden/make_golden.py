@@ -15,6 +15,15 @@ Fixtures (tests/golden/*.npz):
                               reference block loop exposes (float32, bit patterns).
   taps.npz                  : impulseResponseLPF/BPF outputs for every tap set used.
   pll_kat.npz               : PLL known-answer: pilot in, ncoOut + final state out.
+  reference_vectors.npz     : inputs and outputs of every comparison the tests make with the
+                              reference's compiled code (tests/reference_vectors.py CASES), for
+                              boxes without the reference.
+
+    python tests/golden/make_golden.py --vectors-from-oracle
+rewrites reference_vectors.npz alone from the oracle (oracle/fmrx_oracle.c), for when the
+reference is not at hand.  Those tests, run live against the reference, hold the oracle
+bit-identical to it on every one of these cases, and the oracle reproduces every fixture above
+(tests/test_golden.py).  The file records which of the two wrote it ("meta|source").
 """
 import hashlib
 import importlib
@@ -28,7 +37,10 @@ ROOT = HERE.parent.parent
 sys.path.insert(0, str(ROOT))
 sys.path.insert(0, str(ROOT / "oracle"))
 
+sys.path.insert(0, str(ROOT / "tests"))
+
 import pyoracle  # noqa: E402
+import reference_vectors as rv  # noqa: E402
 
 synth = importlib.import_module("software-defined-radio-course-project_b200").synth
 
@@ -40,8 +52,21 @@ CHAINS = [(0, 51, 12, 7, True), (0, 101, 6, 8, True), (0, 301, 4, 9, True), (1, 
           (2, 51, 2, 11, False), (3, 51, 1, 12, False)]
 
 
+def write_reference_vectors(impl, source):
+    port = pyoracle.Port()
+    out = {"meta|source": np.array(source)}
+    for case, fn, args in rv.CASES:
+        out.update(rv.encode(case, fn(port, synth, impl, *args)))
+    np.savez_compressed(rv.VECTORS, **out)
+    print("reference vectors", len(rv.CASES), "cases from the", source, rv.VECTORS.stat().st_size, "bytes")
+
+
 def main():
+    if "--vectors-from-oracle" in sys.argv:
+        write_reference_vectors(pyoracle.Port(), "oracle")
+        return
     ref = pyoracle.Reference()
+    write_reference_vectors(ref, "reference")
     port_modes = pyoracle.Port()          # only for the mode table (sizes), not for any signal
     for mode, taps, nb, seed, store in CHAINS:
         info = port_modes.mode(mode, taps)

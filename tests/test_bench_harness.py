@@ -7,6 +7,7 @@ import sys
 from pathlib import Path
 
 import numpy as np
+import pytest
 
 ROOT = Path(__file__).resolve().parent.parent
 
@@ -35,6 +36,32 @@ def test_parity_full_counts_differences(port, synth):
     assert bad["samples_differ"] == 2 and bad["max_abs_lsb"] == 3 and bad["captures_gt_1lsb"] == 1
     assert bad["first_difference"] == {"capture": 1, "pcm_index": 1000}
     assert good["input_sha256"] == bad["input_sha256"]
+
+
+def test_dump_pcm_sample_is_seeded_and_bounded(tmp_path):
+    torch = pytest.importorskip("torch")
+    b = _bench()
+    rng = np.random.default_rng(3)
+    parts = [rng.integers(-32768, 32768, size=(3, 1000000), dtype=np.int16) for _ in range(2)]
+    b.dump_pcm_sample(np, torch, [torch.from_numpy(p) for p in parts], tmp_path / "a")
+    b.dump_pcm_sample(np, torch, [torch.from_numpy(np.concatenate(parts))], tmp_path / "b")
+    pcm, pos = np.load(tmp_path / "a" / "pcm.npy"), np.load(tmp_path / "a" / "pcm_index.npy")
+    assert pcm.dtype == np.float32 and pos.dtype == np.float64
+    assert len(pcm) == min(6 * 1000000, b.DUMP_SAMPLES) and pos.shape == (len(pcm), 2)
+    flat = pos[:, 0] * 1000000 + pos[:, 1]
+    assert np.all(np.diff(flat) > 0) and flat[0] >= 0 and flat[-1] < 6 * 1000000
+    assert pcm.nbytes + pos.nbytes <= 64 << 20
+    whole = np.concatenate(parts)
+    assert np.array_equal(pcm, whole[pos[:, 0].astype(np.int64), pos[:, 1].astype(np.int64)].astype(np.float32))
+    for name in ("pcm.npy", "pcm_index.npy"):      # the same rows split differently: the same sample
+        assert np.array_equal(np.load(tmp_path / "a" / name), np.load(tmp_path / "b" / name))
+
+
+@pytest.mark.parametrize("args,flag", [(["--steps", "0"], "--steps"),
+                                       (["--impl", "reference", "--dump-outputs", "d"], "--dump-outputs")])
+def test_bad_arguments_are_refused(args, flag):
+    r = subprocess.run([sys.executable, str(ROOT / "bench.py"), *args], capture_output=True, text=True, timeout=120)
+    assert r.returncode != 0 and flag in r.stderr
 
 
 def test_golden_fixtures_cover_the_bench_batch():

@@ -6,6 +6,7 @@ are rounded to float where the reference rounds; see DESIGN.md for the residual
 import numpy as np
 import pytest
 
+import reference_vectors as rv
 from conftest import assert_bits_equal
 from pll_inputs import KINDS, hostile_pilot
 
@@ -134,6 +135,7 @@ def test_pll_hostile_inputs_bitwise(fm, port, kind):
     o, _, os_ = port.pll(x, 19000, 240e3, 2, 0, 0.01)
     assert_bits_equal(g, o, f"pll nco ({kind})")
     assert_bits_equal(gs, os_, f"pll state ({kind})")
+    rv.check_stored(f"pll hostile {kind}", {"input": x, "nco": g, "state": gs})    # and the stored reference vectors
     # and again from the carried state, in pieces that are not multiples of anything
     pieces, st_g, st_o, at = [], gs, os_, 0
     for m in (1, 15, 16, 17, 1023, 1024, 1025, 5000):

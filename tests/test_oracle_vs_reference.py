@@ -4,109 +4,61 @@ src/iofunc.cpp behind oracle/ref_shim.cpp) and against its binary.
 
 The reference's own tests hold no vector for this path (SURVEY.md section 4),
 so this comparison -- plus the fixtures in tests/golden/ generated from the same
-library -- is the pin.  Runs wherever oracle/_ref exists (built from
-/root/reference in this container; the prebuilt files travel to the GPU box)."""
+library -- is the pin.  Where the reference is not at hand, each comparison is made
+with what it computed, stored in tests/golden/reference_vectors.npz (tests/reference_vectors.py)."""
 import subprocess
 
 import numpy as np
 import pytest
 
 import pyoracle
-from conftest import assert_bits_equal
-from pll_inputs import KINDS, hostile_pilot
+import reference_vectors as rv
+from pll_inputs import KINDS
 
 TAP_SETS = (51, 101, 301)
 
 
 @pytest.mark.parametrize("taps", TAP_SETS)
-def test_tap_design_bitwise(port, reference, taps):
-    for fs in (2.4e6, 1.152e6, 2.304e6):
-        assert_bits_equal(port.lpf_taps(fs, 100e3, taps, 1), reference.lpf_taps(fs, 100e3, taps, 1), f"rf lpf {fs}")
-    for fs in (240e3, 288e3, 256e3):
-        assert_bits_equal(port.lpf_taps(fs, 16e3, taps, 1), reference.lpf_taps(fs, 16e3, taps, 1), f"audio lpf {fs}")
-        for fb, fe in ((22e3, 54e3), (18.5e3, 19.5e3)):
-            assert_bits_equal(port.bpf_taps(fs, fb, fe, taps), reference.bpf_taps(fs, fb, fe, taps), f"bpf {fs} {fb}")
-    for fs, up in ((35.28e6, 147), (112.896e6, 441)):
-        assert_bits_equal(port.lpf_taps(fs, 16e3, taps * up, up), reference.lpf_taps(fs, 16e3, taps * up, up),
-                          f"polyphase lpf x{up}")
+def test_tap_design_bitwise(port, synth, reference, taps):
+    rv.compare(f"taps {taps}", port, synth, reference)
 
 
-def test_operators_bitwise(port, reference):
-    rng = np.random.default_rng(5)
-    x = rng.standard_normal(4000).astype(np.float32)
-    y = rng.standard_normal(4000).astype(np.float32)
-    c = port.lpf_taps(240e3, 16e3, 51, 1)
-    for up, down in ((1, 1), (1, 5), (1, 10), (3, 7), (147, 800)):
-        cc = port.lpf_taps(240e3 * up, 16e3, 51 * up, up)
-        st = rng.standard_normal(51 * up - 1).astype(np.float32)
-        xin = x if len(x) >= 51 * up - 1 else rng.standard_normal(51 * up + 500).astype(np.float32)
-        po, ps = port.resample(xin, st, cc, up, down)      # reference needs in_len >= taps-1
-        ro, rs = reference.resample(xin, st, cc, up, down)
-        assert_bits_equal(po, ro, f"resample {up}/{down}")
-        assert_bits_equal(ps, rs, f"resample state {up}/{down}")
-    pd, pi, pq = port.fmdemod(x, y, 0.25, -0.5)
-    rd, ri, rq = reference.fmdemod(x, y, 0.25, -0.5)
-    assert_bits_equal(pd, rd, "fmdemod")
-    assert (pi, pq) == (ri, rq)
-    z = np.zeros(8, np.float32)
-    assert_bits_equal(port.fmdemod(z, z)[0], reference.fmdemod(z, z)[0], "fmdemod zero denominator")
-    assert_bits_equal(port.mixer(x, y), reference.mixer(x, y), "mixer")
-    for a, b in zip(port.lr_extract(x, y), reference.lr_extract(x, y)):
-        assert_bits_equal(a, b, "lr_extract")
-    del c
+def test_operators_bitwise(port, synth, reference):
+    rv.compare("operators", port, synth, reference)
 
 
-def test_pll_bitwise_including_saturation(port, reference):
-    t = np.arange(200000, dtype=np.float64)
-    pilot = (0.1 * np.sin(2 * np.pi * 19000.3 / 240e3 * t + 0.4)).astype(np.float32)
-    pn, _, ps = port.pll(pilot, 19000, 240e3, 2, 0, 0.01)
-    rn, _, rs = reference.pll(pilot, 19000, 240e3, 2, 0, 0.01)
-    assert_bits_equal(pn, rn, "pll nco")
-    assert_bits_equal(ps, rs, "pll state")
-    # float trigOffset saturates at 2^24 (SURVEY.md H5): start just below it
-    st = np.array([1e-4, 3.0, 0.3, -0.95, 1.0, 16777216.0 - 300.0], np.float32)
-    pn, _, ps = port.pll(pilot[:1000], 19000, 240e3, 2, 0, 0.01, st)
-    rn, _, rs = reference.pll(pilot[:1000], 19000, 240e3, 2, 0, 0.01, st)
-    assert_bits_equal(pn, rn, "pll nco (saturating counter)")
-    assert_bits_equal(ps, rs, "pll state (saturating counter)")
-    assert ps[5] == 16777216.0
+def test_pll_bitwise_including_saturation(port, synth, reference):
+    got = rv.compare("pll saturation", port, synth, reference)
+    assert got["state (saturating counter)"][5] == 16777216.0
 
 
 @pytest.mark.parametrize("kind", KINDS)
-def test_pll_hostile_inputs_bitwise(port, reference, kind):
+def test_pll_hostile_inputs_bitwise(port, synth, reference, kind):
     """The inputs the GPU parity tests use against the oracle (tests/pll_inputs.py): zeros, subnormals,
     noise, huge amplitudes -- the oracle must follow the compiled reference there too (atan2 of signed
     zeros, float overflow in the products)."""
-    x = hostile_pilot(kind)
-    pn, _, ps = port.pll(x, 19000, 240e3, 2, 0, 0.01)
-    rn, _, rs = reference.pll(x, 19000, 240e3, 2, 0, 0.01)
-    assert_bits_equal(pn, rn, f"pll nco ({kind})")
-    assert_bits_equal(ps, rs, f"pll state ({kind})")
+    rv.compare(f"pll hostile {kind}", port, synth, reference)
 
 
 @pytest.mark.parametrize("mode,taps,nblocks", [(0, 51, 40), (0, 101, 12), (0, 301, 8), (1, 51, 24),
                                                (2, 51, 2), (3, 51, 2)])
-def test_chain_all_stages_bitwise(port, reference, synth, mode, taps, nblocks):
-    info = port.mode(mode, taps)
-    iq = synth.synth_iq(nblocks * info.block_size // 2, info.rf_fs, seed=mode + 10)
-    pcm, d = port.chain(mode, taps).run(iq, pyoracle.STAGES)
-    rpcm, rd, rst = reference.chain_run(mode, taps, iq, pyoracle.STAGES, info)
-    for s in rd:
-        assert_bits_equal(d[s], rd[s], f"mode {mode} taps {taps} stage {s}")
-    assert np.array_equal(pcm, rpcm)
-    assert np.abs(pcm).max() > 1000          # the chain decodes audio, not silence
+def test_chain_all_stages_bitwise(port, synth, reference, mode, taps, nblocks):
+    got = rv.compare(f"chain m{mode} t{taps} x{nblocks}", port, synth, reference)
+    assert np.abs(got["pcm"]).max() > 1000          # the chain decodes audio, not silence
 
 
 @pytest.mark.parametrize("taps", [51, 101])
-def test_reference_binary_pcm_is_prefix(port, synth, taps):
+def test_reference_binary_pcm_is_prefix(port, synth, reference, taps):
     """End to end against the reference's own `project` binary: its stdout is an exact
     prefix of the oracle's PCM, short by the 0..4 blocks it loses at EOF (SURVEY.md H7: a race between
-    its two threads at exit, so how many -- possibly none -- varies from run to run)."""
+    its two threads at exit, so how many -- possibly none -- varies from run to run).  Without the binary,
+    the oracle's PCM equals the reference's over the whole blocks of the same input (stored)."""
     exe = pyoracle.Reference.binary(taps)
     if exe is None:
-        pytest.skip("reference binary not built")
+        rv.compare(f"binary t{taps}", port, synth, reference)
+        return
     info = port.mode(0, taps)
-    iq = synth.synth_iq(60 * info.block_size // 2 + 777, info.rf_fs, seed=3)   # ragged tail
+    iq = rv.binary_input(port, synth, taps)
     r = subprocess.run([str(exe), "0", "2"], input=iq.tobytes(), capture_output=True, timeout=120)
     assert r.returncode == 1 and b"End of input stream reached!" in r.stderr
     out = np.frombuffer(r.stdout, np.int16)

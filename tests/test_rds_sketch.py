@@ -6,42 +6,20 @@ import numpy as np
 import pytest
 
 import pyoracle
+import reference_vectors as rv
 from conftest import assert_bits_equal
 
 
-def _demod_with_rds(port, synth, n_blocks, seed=0):
-    """Demodulated FM (the chain's own `demod` stage) with a 57 kHz BPSK-ish subcarrier added, so that the sketch's
-    squarer finds a 114 kHz line to lock its PLL to."""
-    info = port.mode(0, 51)
-    iq = synth.synth_iq_exact(n_blocks * info.block_size // 2, float(info.rf_fs), station=seed)
-    _, d = port.chain(0, 51).run(iq, ("demod",))
-    x = d["demod"]
-    t = np.arange(len(x), dtype=np.float64) / info.if_fs
-    rng = np.random.default_rng(seed)
-    bits = rng.integers(0, 2, len(x) // 202 + 2) * 2 - 1                   # 1187.5 baud at 240 kHz: 202 samples per bit
-    data = np.repeat(bits, 202)[:len(x)].astype(np.float64)
-    return (x + 0.05 * data * np.cos(2 * np.pi * 57000.0 * t)).astype(np.float32), info
-
-
 @pytest.mark.parametrize("taps,delay", [(51, 5), (101, 12)])
-def test_oracle_rds_sketch_matches_reference_operators(port, reference, synth, taps, delay):
-    x, info = _demod_with_rds(port, synth, 40)
-    a = pyoracle.RdsSketch(port, float(info.if_fs), taps, delay)
-    b = pyoracle.RdsSketch(reference, float(info.if_fs), taps, delay)
-    for blk in range(40):
-        seg = x[blk * info.if_per_block:(blk + 1) * info.if_per_block]
-        oa, ca, na = a.block(seg)
-        ob, cb, nb = b.block(seg)
-        assert_bits_equal(ca, cb, f"channel, block {blk}")
-        assert_bits_equal(na, nb, f"carrier after the PLL, block {blk}")
-        assert_bits_equal(oa, ob, f"mixer, block {blk}")
-    assert np.abs(oa).max() > 0
+def test_oracle_rds_sketch_matches_reference_operators(port, synth, reference, taps, delay):
+    got = rv.compare(f"rds t{taps} d{delay}", port, synth, reference)
+    assert np.abs(got["mixer"][-640:]).max() > 0
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("taps,delay,block_mult", [(51, 5, 1), (101, 12, 3), (51, 0, 2)])
 def test_cuda_rds_sketch_matches_oracle(fm, port, synth, taps, delay, block_mult):
-    x, info = _demod_with_rds(port, synth, 60, seed=3)
+    x, info = rv.demod_with_rds(port, synth, 60, seed=3)
     ref = pyoracle.RdsSketch(port, float(info.if_fs), taps, delay)
     n = info.if_per_block * block_mult
     with fm.RdsFront(float(info.if_fs), taps, delay) as rds:

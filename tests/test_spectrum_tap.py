@@ -8,30 +8,21 @@ upper bins -- so: within 0.01 dB on the bins within 30 dB of the strongest, 0.25
 import numpy as np
 import pytest
 
+import reference_vectors as rv
 from conftest import assert_bits_equal
 
 
-def _signal(n, seed=0):
-    rng = np.random.default_rng(seed)
-    t = np.arange(n)
-    return (0.5 * np.sin(2 * np.pi * 19000 / 240e3 * t) + 0.2 * np.sin(2 * np.pi * 57000 / 240e3 * t + 1.0)
-            + 0.01 * rng.standard_normal(n)).astype(np.float32)
-
-
 @pytest.mark.parametrize("bins,segments", [(256, 8), (64, 20), (100, 5)])
-def test_oracle_psd_is_bit_identical_to_reference_fourier(port, reference, bins, segments):
-    x = _signal(bins * segments + 17, seed=bins)              # a ragged tail is ignored (:63)
-    fo, po = port.estimate_psd(x, bins, 240e3)
-    fr, pr = reference.estimate_psd(x, bins, 240e3)
-    assert_bits_equal(fo, fr, "freq")
-    assert_bits_equal(po, pr, "psd")
+def test_oracle_psd_is_bit_identical_to_reference_fourier(port, synth, reference, bins, segments):
+    got = rv.compare(f"psd {bins}x{segments}", port, synth, reference)
+    fo, po = got["freq"], got["psd"]
     assert abs(fo[np.argmax(po)] - 19000.0) <= 240e3 / bins
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("bins,segments", [(256, 40), (1024, 6), (2048, 3), (100, 30)])
 def test_cuda_psd_matches_oracle_within_float_accuracy(fm, port, bins, segments):
-    x = _signal(bins * segments + 5, seed=bins)
+    x = rv.psd_signal(bins * segments + 5, seed=bins)
     fo, po = port.estimate_psd(x, bins, 240e3)
     fg, pg = fm.estimatePSD(x, bins, 240e3)
     assert_bits_equal(fg, fo, "freq")
