@@ -136,7 +136,9 @@ int fmrx_reset(fmrx_pipeline *p);
 
 /* Process n_blocks whole blocks of every capture.  HOST buffers:
  *   iq : capture c starts at iq + c*iq_stride (bytes), n_blocks*block_size u8
- *        interleaved I,Q (what the reference reads from stdin);
+ *        interleaved I,Q (what the reference reads from stdin).  iq_stride 0:
+ *        every capture reads the same stream (several stations of one
+ *        capture, fmrx_set_tuning); it is copied to the device once;
  *   pcm: capture c at pcm + c*pcm_stride (int16 elements),
  *        n_blocks*2*audio_per_block int16, interleaved R,L (what the reference
  *        writes to stdout).
@@ -146,13 +148,32 @@ int fmrx_reset(fmrx_pipeline *p);
 int fmrx_process(fmrx_pipeline *p, const uint8_t *iq, size_t iq_stride,
                  size_t n_blocks, int16_t *pcm, size_t pcm_stride);
 
-/* Same, DEVICE buffers on the pipeline's device.  Work is ordered after
- * everything already enqueued on `stream` (a cudaStream_t; NULL = default
- * stream) and `stream` is made to wait for the result; the call itself does
- * not synchronise the host. */
+/* Same, DEVICE buffers on the pipeline's device (iq_stride 0 as above).
+ * Work is ordered after everything already enqueued on `stream` (a
+ * cudaStream_t; NULL = default stream) and `stream` is made to wait for the
+ * result; the call itself does not synchronise the host. */
 int fmrx_process_device(fmrx_pipeline *p, const uint8_t *iq_dev, size_t iq_stride,
                         size_t n_blocks, int16_t *pcm_dev, size_t pcm_stride,
                         void *stream);
+
+/* Tune `capture` to the station offset_hz above its stream's centre
+ * frequency (negative: below); |offset_hz| < rf_fs/2, else FMRX_ERR_ARG.
+ * The chain then runs on x * e^{-j theta(n)} instead of the raw pairs x(n):
+ *   inc   = (uint32) llrint(offset_hz * 2^32 / rf_fs), in double, mod 2^32;
+ *   n     = pair index from the stream's first pair (0 after create or reset;
+ *           it continues across calls, chunks and state blobs);
+ *   ph    = (uint32)(n * inc) in uint32 arithmetic, k = ph >> 16;
+ *   cos_t[k] = (float)cos(a), sin_t[k] = (float)sin(a), a = 2 pi k / 65536
+ *           (double), 65536 entries each;
+ *   I' = i*cos_t[k] + q*sin_t[k],  Q' = q*cos_t[k] - i*sin_t[k]
+ *           (i, q = (u8-128)/128; one IEEE float operation each, no FMA).
+ * The zero history in front of the first pair is not rotated; the rest of
+ * the chain is unchanged.  Offset 0 is bit-identical to no tuning and
+ * restores it.  Tuning is configuration, not state: it survives
+ * fmrx_reset and is not in the state blob.  Only at the start of the
+ * capture's stream (after create or reset), else FMRX_ERR_STATE; to resume
+ * a tuned checkpoint: fmrx_create, fmrx_set_tuning, fmrx_set_state. */
+int fmrx_set_tuning(fmrx_pipeline *p, int capture, double offset_hz);
 
 /* Stage intermediates of the LAST fmrx_process* call (keep_stages=1 only). */
 typedef enum {

@@ -38,7 +38,7 @@ ABI_SYMBOLS = (
     "fmrx_process", "fmrx_process_device", "fmrx_read_stage",
     "fmrx_state_size", "fmrx_get_state", "fmrx_set_state", "fmrx_get_pll_state",
     "fmrx_host_alloc", "fmrx_host_free", "fmrx_kernel_launches", "fmrx_set_timing",
-    "fmrx_last_timing",
+    "fmrx_last_timing", "fmrx_set_tuning",
     "fmrx_long_create", "fmrx_long_destroy", "fmrx_long_shard", "fmrx_long_process", "fmrx_long_process_device",
     "fmrx_long_last_ms", "fmrx_long_pll_state",
     "fmrx_rds_create", "fmrx_rds_destroy", "fmrx_rds_reset", "fmrx_rds_process", "fmrx_rds_pll_state",
@@ -129,6 +129,7 @@ def load() -> C.CDLL:
     L.fmrx_estimate_psd.argtypes = [_f32p, _f32p, _f32p, C.c_size_t, C.c_int, C.c_float]
     L.fmrx_set_timing.argtypes = [C.c_void_p, C.c_int]
     L.fmrx_last_timing.argtypes = [C.c_void_p, _f32p]
+    L.fmrx_set_tuning.argtypes = [C.c_void_p, C.c_int, C.c_double]
     _lib = L
     return L
 
@@ -238,10 +239,11 @@ def pcm_pack(left, right) -> np.ndarray:
 # ---- fused pipeline -----------------------------------------------------------
 
 class Pipeline:
-    """The block loop of src/project.cpp for ``n_captures`` captures at once."""
+    """The block loop of src/project.cpp for ``n_captures`` captures at once.  ``tune_hz``: the station's offset from
+    the capture's centre frequency (fmrx_set_tuning), one for all captures or one per capture; None: untuned."""
 
     def __init__(self, mode: int = 0, taps: int = 51, n_captures: int = 1, device: int = -1,
-                 chunk_blocks: int = 0, keep_stages: bool = False):
+                 chunk_blocks: int = 0, keep_stages: bool = False, tune_hz=None):
         self._L = load()
         cfg = ConfigStruct(mode, taps, n_captures, device, chunk_blocks, int(keep_stages))
         h = C.c_void_p()
@@ -252,6 +254,18 @@ class Pipeline:
         self.info = ModeInfo(s)
         self.n_captures = n_captures
         self._last_nb = 0
+        if tune_hz is not None:
+            hz = list(tune_hz) if np.ndim(tune_hz) else [tune_hz] * n_captures
+            if len(hz) != n_captures:
+                self.close()
+                raise ValueError(f"tune_hz: {len(hz)} offsets for {n_captures} captures")
+            for c, f in enumerate(hz):
+                self.set_tuning(c, f)
+
+    def set_tuning(self, capture: int, hz: float):
+        """Tune ``capture`` to the station ``hz`` above its stream's centre (negative: below); only at the start of
+        its stream (after creation or reset)."""
+        _check(self._L.fmrx_set_tuning(self._h, capture, float(hz)), "fmrx_set_tuning")
 
     def close(self):
         if getattr(self, "_h", None):
@@ -286,6 +300,19 @@ class Pipeline:
         if nb:
             _check(self._L.fmrx_process(self._h, iq.ctypes.data, iq.strides[0], nb, pcm.ctypes.data,
                                         pcm.shape[1]), "fmrx_process")
+        return pcm
+
+    def process_shared(self, iq: np.ndarray) -> np.ndarray:
+        """One host IQ stream (uint8, 1-D) read by every capture (``iq_stride`` 0): with each capture tuned to its
+        own station, several stations of one capture.  Returns int16 ``[n_captures, n_blocks*2*audio_per_block]``."""
+        iq = np.ascontiguousarray(iq, np.uint8)
+        assert iq.ndim == 1
+        nb = len(iq) // self.info.block_size
+        pcm = np.zeros((self.n_captures, nb * 2 * self.info.audio_per_block), np.int16)
+        self._last_nb = nb
+        if nb:
+            _check(self._L.fmrx_process(self._h, iq.ctypes.data, 0, nb, pcm.ctypes.data, pcm.shape[1]),
+                   "fmrx_process")
         return pcm
 
     def process_raw(self, iq_ptr: int, iq_stride: int, n_blocks: int, pcm_ptr: int, pcm_stride: int):

@@ -13,6 +13,7 @@
 // previous chunk is kept in small per-capture "tail" arrays owned by the stream
 // that produces the data, and copied in front of the next chunk's buffer.
 #include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstring>
 #include <new>
@@ -376,7 +377,14 @@ struct fmrx_pipeline {
     cudaStream_t s_h2d = nullptr;   // host path: the H2D copies, so that chunk i+1 comes in under K1/K2 of chunk i
     cudaEvent_t ev_in = nullptr, ev_out = nullptr;
     std::vector<long long> blocks_done;   // per capture: blocks since the start of ITS stream (state blobs carry it)
+    long long blocks_run = 0;             // blocks the chunk loop has run since create/reset (the same for every capture)
     long long chunk_counter = 0;
+    // tuning (fmrx_set_tuning): configuration, not state.  tune[c] is mirrored in d_tune for K1 and written only
+    // while the device is idle (create, reset, fmrx_set_tuning, fmrx_set_state), so a call never uploads it.
+    std::vector<RfTune> tune;
+    RfTune *d_tune = nullptr;             // [C]
+    float2 *d_tune_cs = nullptr;          // the mixer table (65536 cos, sin), allocated when a capture is first tuned
+    bool tuned = false;                   // some capture has a nonzero phase step: K1 runs its tuned variant
     size_t mem_pitch = 0;       // cudaDeviceProp::memPitch: the largest pitch cudaMemcpy2D takes
     uint64_t launches = 0;
 
@@ -402,6 +410,7 @@ void free_pipeline(fmrx_pipeline *p)
     auto F = [](void *q) { if (q) cudaFree(q); };
     F(p->d_rf_taps); F(p->d_pilot_taps); F(p->d_chan_taps); F(p->d_audio_pm);
     F(p->d_hist_iq); F(p->d_tail_demod); F(p->d_tail_chan); F(p->d_tail_trig); F(p->d_pll_state);
+    F(p->d_tune); F(p->d_tune_cs);
     for (auto &s : p->sets) {
         F(s.iq); F(s.demod); F(s.chan); F(s.trig); F(s.pilot); F(s.pcm);
         if (s.front_done) cudaEventDestroy(s.front_done);
@@ -436,6 +445,10 @@ int reset_state(fmrx_pipeline *p)
     }
     CU(cudaMemcpy(p->d_pll_state, st.data(), st.size() * sizeof(float), cudaMemcpyHostToDevice));
     p->blocks_done.assign(C, 0);
+    p->blocks_run = 0;
+    for (auto &t : p->tune)
+        t.pair_offset = 0;
+    CU(cudaMemcpy(p->d_tune, p->tune.data(), C * sizeof(RfTune), cudaMemcpyHostToDevice));
     return FMRX_OK;
 }
 
@@ -505,6 +518,8 @@ int create_impl(fmrx_pipeline *p, const fmrx_config *cfg)
     CU(dalloc(&p->d_tail_chan, C * p->H));
     CU(dalloc(&p->d_tail_trig, C * p->H));
     CU(dalloc(&p->d_pll_state, C * 8));
+    CU(dalloc(&p->d_tune, C));
+    p->tune.assign(C, RfTune{ 0, 0 });
     for (auto &s : p->sets) {
         CU(dalloc(&s.demod, C * p->if_stride));
         CU(dalloc(&s.chan, C * p->if_stride));
@@ -579,6 +594,16 @@ cudaError_t copy2d(void *dst, size_t dpitch, const void *src, size_t spitch, siz
     return cudaMemcpy2DAsync(dst, dpitch, src, spitch, width, rows, kind, s);
 }
 
+// `rows` contiguous device rows of `width` bytes, each a copy of one source row: one copy, then doubling
+// (what copy2d cannot do: cudaMemcpy2DAsync refuses a source pitch of 0).
+cudaError_t broadcast_rows(uint8_t *dst, const uint8_t *src, size_t width, size_t rows, cudaStream_t s)
+{
+    cudaError_t e = cudaMemcpyAsync(dst, src, width, cudaMemcpyDeviceToDevice, s);
+    for (size_t k = 1; k < rows && e == cudaSuccess; k *= 2)
+        e = cudaMemcpyAsync(dst + k * width, dst, std::min(k, rows - k) * width, cudaMemcpyDeviceToDevice, s);
+    return e;
+}
+
 // The chunk loop shared by the host- and device-pointer entry points.
 // feedforward_only: K1 and K2 only -- what a time shard runs over the blocks in FRONT of its own (its halo), from the
 // zero state, to arrive at the IQ / demod / channel histories the stream has at the shard's first block.
@@ -647,12 +672,13 @@ int run(fmrx_pipeline *p, const uint8_t *iq, size_t iq_stride, size_t n_blocks, 
         size_t iq_dev_stride;
         if (host_io) {
             iq_dev = S.iq;
-            iq_dev_stride = static_cast<size_t>(p->chunk_blocks) * mi.block_size;
+            // iq_stride 0: every capture reads one stream, which crosses the host link once
+            iq_dev_stride = iq_stride ? static_cast<size_t>(p->chunk_blocks) * mi.block_size : 0;
             // on its own stream: the copy of a chunk only waits for the staging buffer (read for the
             // last time by K1 three chunks ago), not for K1/K2 of the chunk before
             if (S.iq_free_pending)
                 CU(cudaStreamWaitEvent(p->s_h2d, S.iq_free, 0));
-            CU(copy2d(S.iq, iq_dev_stride, iq + b0 * mi.block_size, iq_stride, chunk_bytes, C,
+            CU(copy2d(S.iq, iq_dev_stride, iq + b0 * mi.block_size, iq_stride, chunk_bytes, iq_stride ? C : 1,
                       p->s_h2d, cudaMemcpyHostToDevice, p->mem_pitch));
             CU(cudaEventRecord(S.h2d_done, p->s_h2d));
             CU(cudaStreamWaitEvent(p->s_front, S.h2d_done, 0));
@@ -682,14 +708,19 @@ int run(fmrx_pipeline *p, const uint8_t *iq, size_t iq_stride, size_t n_blocks, 
                 a.stage_stride = p->stage_if_len;
                 a.stage_off = b0 * mi.if_per_block;
             }
-            CU(launch_rf_demod(a, C, p->s_front));
+            const RfTuneArgs tu{ p->d_tune_cs, p->d_tune, p->blocks_run * (mi.block_size / 2) };
+            CU(launch_rf_demod(a, C, p->s_front, p->tuned ? &tu : nullptr));
             p->launches++;
         }
         if (te) CU(cudaEventRecord(te[1], p->s_front));
-        // IQ history for the next chunk: the last hist_pairs pairs of this chunk
-        CU(copy2d(p->d_hist_iq, 2 * static_cast<size_t>(p->hist_pairs),
-                  iq_dev + chunk_bytes - 2 * static_cast<size_t>(p->hist_pairs), iq_dev_stride,
-                  2 * static_cast<size_t>(p->hist_pairs), C, p->s_front));
+        // IQ history for the next chunk: the last hist_pairs pairs of this chunk (per capture, also when the
+        // captures share one stream: state blobs are per capture)
+        const size_t hist_bytes = 2 * static_cast<size_t>(p->hist_pairs);
+        if (iq_dev_stride)
+            CU(copy2d(p->d_hist_iq, hist_bytes, iq_dev + chunk_bytes - hist_bytes, iq_dev_stride, hist_bytes, C,
+                      p->s_front));
+        else
+            CU(broadcast_rows(p->d_hist_iq, iq_dev + chunk_bytes - hist_bytes, hist_bytes, C, p->s_front));
         if (host_io) {
             CU(cudaEventRecord(S.iq_free, p->s_front));
             S.iq_free_pending = true;
@@ -805,6 +836,7 @@ int run(fmrx_pipeline *p, const uint8_t *iq, size_t iq_stride, size_t n_blocks, 
 
         for (auto &bd : p->blocks_done)
             bd += nb;
+        p->blocks_run += nb;
         p->chunk_counter++;
     }
 
@@ -836,8 +868,8 @@ int check_io(const fmrx_pipeline *p, const void *iq, size_t iq_stride, size_t n_
     if ((reinterpret_cast<uintptr_t>(iq) & 1u) || (reinterpret_cast<uintptr_t>(pcm) & 3u))
         return FMRX_ERR_ARG;
     // the strides only matter with more than one capture (a single capture may be a truncated file of
-    // any length: the trailing partial block is the caller's to drop)
-    if (p->C > 1 && (iq_stride < need_iq || pcm_stride < need_pcm || (iq_stride & 1u) || (pcm_stride & 1u)))
+    // any length: the trailing partial block is the caller's to drop); iq_stride 0 = one stream for all
+    if (p->C > 1 && ((iq_stride && iq_stride < need_iq) || pcm_stride < need_pcm || (iq_stride & 1u) || (pcm_stride & 1u)))
         return FMRX_ERR_ARG;
     return FMRX_OK;
 }
@@ -1033,7 +1065,30 @@ extern "C" int fmrx_set_state(fmrx_pipeline *p, int capture, const void *blob, s
         CU(cudaMemcpy(p->d_pll_state + 8 * static_cast<size_t>(capture), b_pll, 8 * sizeof(float),
                       cudaMemcpyHostToDevice));
         p->blocks_done[capture] = h.blocks_done;
+        p->tune[capture].pair_offset = (h.blocks_done - p->blocks_run) * (p->mi.block_size / 2);
+        CU(cudaMemcpy(p->d_tune + capture, &p->tune[capture], sizeof(RfTune), cudaMemcpyHostToDevice));
     }
+    return FMRX_OK;
+}
+
+extern "C" int fmrx_set_tuning(fmrx_pipeline *p, int capture, double offset_hz)
+{
+    if (!p || capture < 0 || capture >= p->C || !(std::fabs(offset_hz) < 0.5 * p->mi.rf_fs))
+        return FMRX_ERR_ARG;
+    if (p->blocks_done[capture] != 0)
+        return FMRX_ERR_STATE;   // FIR history mixed with another offset: retuning mid-stream is not supported
+    const uint32_t inc = static_cast<uint32_t>(std::llrint(offset_hz * 4294967296.0 / p->mi.rf_fs));
+    CU(cudaSetDevice(p->device));
+    CU(cudaDeviceSynchronize());   // K1 of calls still in flight reads d_tune
+    if (inc && !p->d_tune_cs) {
+        std::vector<float> cs(2 * 65536);
+        mixer_table(cs.data());
+        CU(dalloc(&p->d_tune_cs, cs.size() / 2));
+        CU(cudaMemcpy(p->d_tune_cs, cs.data(), cs.size() * sizeof(float), cudaMemcpyHostToDevice));
+    }
+    p->tune[capture].inc = inc;
+    CU(cudaMemcpy(p->d_tune + capture, &p->tune[capture], sizeof(RfTune), cudaMemcpyHostToDevice));
+    p->tuned = std::any_of(p->tune.begin(), p->tune.end(), [](const RfTune &t) { return t.inc != 0; });
     return FMRX_OK;
 }
 

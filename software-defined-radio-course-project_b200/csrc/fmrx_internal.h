@@ -31,7 +31,20 @@ struct RfDemodArgs {
     size_t stage_stride;
     size_t stage_off;
 };
-cudaError_t launch_rf_demod(const RfDemodArgs &a, int n_captures, cudaStream_t s);
+// K1 tuned to stations off the capture's centre (fmrx_set_tuning): pair n of a capture's stream, counted from its
+// first pair, is mixed by cs[(uint32)(n * inc) >> 16].
+struct RfTune {             // per capture
+    long long pair_offset;  // the capture's pair index minus the pipeline's pairs_run (nonzero after fmrx_set_state)
+    uint32_t inc;           // phase step per pair, 2^-32 turns
+};
+struct RfTuneArgs {
+    const float2 *cs;       // the mixer's table: 65536 (cos, sin) pairs
+    const RfTune *cap;      // [n_captures]
+    long long pairs_run;    // pairs in front of this chunk, counted by the pipeline since create/reset
+};
+// tune == nullptr: the untuned kernel (a capture's centre)
+cudaError_t launch_rf_demod(const RfDemodArgs &a, int n_captures, cudaStream_t s, const RfTuneArgs *tune = nullptr);
+void mixer_table(float *cs);   // fmrx_taps.cpp: 65536 (cos, sin) pairs, 2^-16 turns apart
 
 // K2: pilot (18.5-19.5 kHz) and stereo-band (22-54 kHz) band-pass FIRs over one demod tile.
 struct BandpassArgs {

@@ -18,6 +18,7 @@
 // attainable ceiling of these kernels is half the FFMA peak by construction.
 #include <cstddef>
 #include <mutex>
+#include <type_traits>
 
 #include "fmrx_internal.h"
 #ifdef FMRX_PLL_PROFILE   // development build: k_pll prints its cycle accounting for capture 0 of every launch
@@ -32,7 +33,7 @@ namespace fmrx {
 // opt-in shared memory is keyed by the device ordinal and guarded by a mutex.
 constexpr int kMaxDevices = 64;
 struct DeviceCfg {
-    size_t rf_smem[3] = { 0, 0, 0 };       // k_rf_demod_win<10>, <4>, <9>: configured dynamic shared memory
+    size_t rf_smem[2][3] = {};             // k_rf_demod_win<10|4|9, untuned|tuned>: configured dynamic shared memory
     size_t audio_smem = 0;                 // k_audio
     size_t bp_smem = 0;                    // k_bandpass_pair
     size_t pll_ring_only = 0, pll_whole_sm = 0;
@@ -88,7 +89,25 @@ template <int D> struct RfWin {
     static __host__ __device__ int wp_max(int T) { return (RF_COMPUTED - 1) * D + T + (tpad(T) - T) + 1; }   // staged pairs (one more if the window starts on an odd pair)
     static __host__ __device__ int words(int T) { return (wp_max(T) + 1) / 2 + (wp_max(T) + 1) / SEG + 2; }  // 32-bit words of the padded tile
     static size_t smem_bytes(int T) { return sizeof(uint32_t) * (size_t)2 * words(T) + sizeof(float) * ((size_t)2 * RF_COMPUTED + tpad(T)); }   // two tiles
+    // tuned: one float2 per staged pair, one float2 of padding per SEG pairs (lane stride SEG + 1 float2: conflict-free)
+    static __host__ __device__ int words_tuned(int T) { return 2 * (wp_max(T) + wp_max(T) / SEG + 1); }
+    static size_t smem_bytes_tuned(int T) { return sizeof(uint32_t) * (size_t)2 * words_tuned(T) + sizeof(float) * ((size_t)2 * RF_COMPUTED + tpad(T)); }
 };
+
+// Tuned K1 (fmrx_set_tuning): the tile is staged already mixed to the station, I' = i cos + q sin, Q' = q cos - i sin
+// with (cos, sin) = cs[ph >> 16], ph = (uint32)(n * inc) at absolute pair n, as two floats per pair -- round 1's float
+// staging -- and the delay line loads those floats instead of converting bytes.  Rotating at use instead would cost a
+// table lookup per tap and thread.  The staging is plain loads (it computes), so there is no cp.async on this path.
+__device__ __forceinline__ void rf_pair(uint32_t v, float &i, float &q)
+{
+    i = unpack_u8_byte<0>(v);
+    q = unpack_u8_byte<1>(v);
+}
+__device__ __forceinline__ void rf_pair(float2 v, float &i, float &q)
+{
+    i = v.x;
+    q = v.y;
+}
 
 // A CTA takes RFW_TILES_MAX (fewer on short chunks) consecutive tiles of one capture and keeps two raw tiles in shared
 // memory: the bytes of tile i+1 arrive by cp.async (4 bytes per request: the tile starts on an arbitrary IQ pair, and
@@ -96,15 +115,19 @@ template <int D> struct RfWin {
 // its time at 51 taps waiting for the tile it was about to compute (ncu source view, profiles/r02_ncu_summary.md).
 constexpr int RFW_TILES_MAX = 8;
 
-template <int D> __global__ void __launch_bounds__(RFW_THREADS) k_rf_demod_win(const RfDemodArgs a, const int tiles_per_cta)
+template <int D, bool Tuned>
+__global__ void __launch_bounds__(RFW_THREADS) k_rf_demod_win(const RfDemodArgs a, const int tiles_per_cta, const RfTuneArgs tu)
 {
     using W = RfWin<D>;
     constexpr int L = W::L, SEG = W::SEG, R = RFW_R;
+    using Elem = typename std::conditional<Tuned, float2, unsigned short>::type;   // one staged pair
+    using Val = typename std::conditional<Tuned, float2, uint32_t>::type;
+    constexpr int PADE = Tuned ? 1 : 2;     // padding elements per SEG staged pairs
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int T = a.T;
     const int Tpad = (T + L - 1) / L * L;
-    const int words = W::words(T);
-    uint32_t *s_buf = reinterpret_cast<uint32_t *>(smem_raw);               // two raw tiles, two pairs per word, padded
+    const int words = Tuned ? W::words_tuned(T) : W::words(T);
+    uint32_t *s_buf = reinterpret_cast<uint32_t *>(smem_raw);               // two tiles (raw: two pairs per word), padded
     float *o_i = reinterpret_cast<float *>(s_buf + 2 * words);              // [RF_COMPUTED]
     float *o_q = o_i + RF_COMPUTED;
     float *s_c = o_q + RF_COMPUTED;                                         // [Tpad]
@@ -139,14 +162,32 @@ template <int D> __global__ void __launch_bounds__(RFW_THREADS) k_rf_demod_win(c
         const int padl = tile_padl(tile);
         const long long m_first = (long long)(tile * RF_REAL - 1) * D - (T - 1) - padl;
         const int Wp = (RF_COMPUTED - 1) * D + T + padl;
-        const int n_words = (Wp + 1) >> 1;
-        for (int j = tid; j < n_words; j += RFW_THREADS) {
-            const long long m0 = m_first + 2 * (long long)j;
-            uint32_t *dst = s_w + j + j / (SEG / 2);
-            if (m0 >= 0 && m0 + 1 < n_pairs) {
-                asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"((unsigned)__cvta_generic_to_shared(dst)), "l"(iq16 + m0) : "memory");
-            } else {             // words that straddle the chunk (history in front, nothing behind): assembled pair by pair
-                *dst = pair_at(m0) | (pair_at(m0 + 1) << 16);
+        if constexpr (Tuned) {
+            float2 *s_f = reinterpret_cast<float2 *>(s_w);
+            const RfTune cap = tu.cap[c];
+            const long long n_first = cap.pair_offset + tu.pairs_run + m_first;    // absolute index of staged pair 0
+            const uint32_t ph_first = (uint32_t)((unsigned long long)n_first * cap.inc);
+            for (int l = tid; l < Wp; l += RFW_THREADS) {
+                float xi, xq;
+                rf_pair(pair_at(m_first + l), xi, xq);
+                if (n_first + l >= 0) {      // the zero history in front of the stream's first pair is not rotated
+                    const float2 cs = tu.cs[(ph_first + (uint32_t)l * cap.inc) >> 16];
+                    const float ri = fadd(fmul(xi, cs.x), fmul(xq, cs.y));
+                    xq = fsub(fmul(xq, cs.x), fmul(xi, cs.y));
+                    xi = ri;
+                }
+                s_f[l + l / SEG] = make_float2(xi, xq);
+            }
+        } else {
+            const int n_words = (Wp + 1) >> 1;
+            for (int j = tid; j < n_words; j += RFW_THREADS) {
+                const long long m0 = m_first + 2 * (long long)j;
+                uint32_t *dst = s_w + j + j / (SEG / 2);
+                if (m0 >= 0 && m0 + 1 < n_pairs) {
+                    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"((unsigned)__cvta_generic_to_shared(dst)), "l"(iq16 + m0) : "memory");
+                } else {             // words that straddle the chunk (history in front, nothing behind): assembled pair by pair
+                    *dst = pair_at(m0) | (pair_at(m0 + 1) << 16);
+                }
             }
         }
         asm volatile("cp.async.commit_group;" ::: "memory");
@@ -164,23 +205,22 @@ template <int D> __global__ void __launch_bounds__(RFW_THREADS) k_rf_demod_win(c
         }
         __syncthreads();
 
-        const unsigned short *s_p = reinterpret_cast<const unsigned short *>(s_w);
+        const Elem *s_p = reinterpret_cast<const Elem *>(s_w);
         const int n0 = tile * RF_REAL;              // first demod sample of the tile
         const int padl = tile_padl(tile);
         // this thread: computed outputs o0..o0+3, o0 = 4 tid.  Output o0 at tap k reads staged pair tid*SEG + r0 - k,
-        // r0 = T - 1 + padl (the same for every thread); pair l' sits at 16-bit position l' + 2 (l' / SEG), i.e. for
-        // l' = tid*SEG + e at tid*(SEG + 2) + e + 2 (e / SEG)
+        // r0 = T - 1 + padl (the same for every thread); pair l' sits at element l' + PADE (l' / SEG), i.e. for
+        // l' = tid*SEG + e at tid*(SEG + PADE) + e + PADE (e / SEG)
         const int o0 = tid * R;
         const int r0 = T - 1 + padl;
-        const unsigned short *tp = s_p + tid * (SEG + 2);
+        const Elem *tp = s_p + tid * (SEG + PADE);
 
         float di[L], dq[L];                         // delay lines: slot (k mod L) holds the sample of tap k
 #pragma unroll
         for (int m = 1; m <= L; m++) {              // "taps" -m: the samples above tap 0's, for outputs o0+1..o0+3
             const int e = r0 + m;
-            const uint32_t v = tp[e + 2 * (e / SEG)];
-            di[L - m] = unpack_u8_byte<0>(v);
-            dq[L - m] = unpack_u8_byte<1>(v);
+            const Val v = tp[e + PADE * (e / SEG)];
+            rf_pair(v, di[L - m], dq[L - m]);
         }
         float ai[R], aq[R];
 #pragma unroll
@@ -192,13 +232,14 @@ template <int D> __global__ void __launch_bounds__(RFW_THREADS) k_rf_demod_win(c
             // within a trip e = e_trip - j crosses at most one padding boundary: e / SEG = q - (j > rem)
             const int e_trip = r0 - k0;             // >= 0 by construction of padl
             const int q = e_trip / SEG, rem = e_trip - q * SEG;
-            const unsigned short *tq = tp + e_trip + 2 * q;
+            const Elem *tq = tp + e_trip + PADE * q;
 #pragma unroll
             for (int j = 0; j < L; j++) {
-                const uint32_t v = tq[-j - (j > rem ? 2 : 0)];
+                const Val v = tq[-j - (j > rem ? PADE : 0)];
                 const float ck = s_c[k0 + j];
                 const float old_i = di[j], old_q = dq[j];          // tap k - L: output 3's sample
-                const float xi = unpack_u8_byte<0>(v), xq = unpack_u8_byte<1>(v);
+                float xi, xq;
+                rf_pair(v, xi, xq);
                 di[j] = xi;
                 dq[j] = xq;
                 ai[0] = fadd(ai[0], fmul(ck, xi));
@@ -236,17 +277,18 @@ template <int D> __global__ void __launch_bounds__(RFW_THREADS) k_rf_demod_win(c
     }
 }
 
-template <int D> static cudaError_t launch_rf_demod_win(const RfDemodArgs &a, int n_captures, cudaStream_t s)
+template <int D, bool Tuned> static cudaError_t launch_rf_demod_win(const RfDemodArgs &a, int n_captures, cudaStream_t s,
+                                                                   const RfTuneArgs &tu)
 {
-    const size_t smem = RfWin<D>::smem_bytes(a.T);
+    const size_t smem = Tuned ? RfWin<D>::smem_bytes_tuned(a.T) : RfWin<D>::smem_bytes(a.T);
     DeviceCfg *cfg = device_cfg();
     if (!cfg)
         return cudaErrorInvalidDevice;
     {
         std::lock_guard<std::mutex> lock(g_cfg_mutex);
-        size_t &configured = cfg->rf_smem[D == 10 ? 0 : D == 4 ? 1 : 2];
+        size_t &configured = cfg->rf_smem[Tuned][D == 10 ? 0 : D == 4 ? 1 : 2];
         if (smem > configured) {
-            cudaError_t e = cudaFuncSetAttribute(k_rf_demod_win<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            cudaError_t e = cudaFuncSetAttribute(k_rf_demod_win<D, Tuned>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
             if (e != cudaSuccess)
                 return e;
             configured = smem;
@@ -259,20 +301,25 @@ template <int D> static cudaError_t launch_rf_demod_win(const RfDemodArgs &a, in
     while (per > 1 && (long long)((tiles + per - 1) / per) * n_captures < 4 * 148)
         per >>= 1;
     dim3 grid((tiles + per - 1) / per, n_captures);
-    k_rf_demod_win<D><<<grid, RFW_THREADS, smem, s>>>(a, per);
+    k_rf_demod_win<D, Tuned><<<grid, RFW_THREADS, smem, s>>>(a, per, tu);
     return cudaGetLastError();
 }
 
-cudaError_t launch_rf_demod(const RfDemodArgs &a, int n_captures, cudaStream_t s)
+template <bool Tuned> static cudaError_t launch_rf_demod_d(const RfDemodArgs &a, int n_captures, cudaStream_t s, const RfTuneArgs &tu)
 {
     // the reference's modes decimate by 10, 4 and 9 (src/project.cpp:327-362); fmrx_mode_table yields nothing else
     if (a.decim == 10)
-        return launch_rf_demod_win<10>(a, n_captures, s);
+        return launch_rf_demod_win<10, Tuned>(a, n_captures, s, tu);
     if (a.decim == 4)
-        return launch_rf_demod_win<4>(a, n_captures, s);
+        return launch_rf_demod_win<4, Tuned>(a, n_captures, s, tu);
     if (a.decim == 9)
-        return launch_rf_demod_win<9>(a, n_captures, s);
+        return launch_rf_demod_win<9, Tuned>(a, n_captures, s, tu);
     return cudaErrorInvalidValue;
+}
+
+cudaError_t launch_rf_demod(const RfDemodArgs &a, int n_captures, cudaStream_t s, const RfTuneArgs *tune)
+{
+    return tune ? launch_rf_demod_d<true>(a, n_captures, s, *tune) : launch_rf_demod_d<false>(a, n_captures, s, RfTuneArgs{});
 }
 
 // ============================================================================

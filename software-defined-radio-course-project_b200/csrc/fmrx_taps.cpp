@@ -74,6 +74,19 @@ extern "C" int fmrx_impulse_response_bpf(float *h, float fs, float fb, float fe,
     return FMRX_OK;
 }
 
+// fmrx_set_tuning's mixer table: cs[2k] = (float)cos(a), cs[2k+1] = (float)sin(a), a = 2 pi k / 65536, k < 65536.
+// The phase is quantised to 16 bits (spurs near -96 dBc, under the 8-bit input's floor).
+namespace fmrx {
+void mixer_table(float *cs)
+{
+    for (int k = 0; k < 65536; k++) {
+        const double a = 6.283185307179586 * static_cast<double>(k) / 65536.0;
+        cs[2 * k] = static_cast<float>(std::cos(a));
+        cs[2 * k + 1] = static_cast<float>(std::sin(a));
+    }
+}
+}  // namespace fmrx
+
 // src/project.cpp:304-364
 extern "C" int fmrx_mode_table(int mode, int taps, fmrx_mode_info *out)
 {

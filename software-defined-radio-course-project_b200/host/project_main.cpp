@@ -1,7 +1,10 @@
 // project_main.cpp -- the `project` command line on the B200 pipeline.
 //
 //   project                      mode 0 (message says "mono", like the reference)
-//   project <mode 0-3> <1|2|m|s> [--taps N] [--chunk-blocks K] [--device D] [--stats]
+//   project <mode 0-3> <1|2|m|s> [--taps N] [--chunk-blocks K] [--device D] [--tune HZ] [--stats]
+//
+// --tune HZ: decode the station HZ (an integer, may be negative) above the capture's centre
+// frequency (fmrx_set_tuning); |HZ| < rf_fs/2 of the mode, else the usage message and exit 1.
 //
 // stdin : raw interleaved u8 I/Q at the mode's RF rate
 // stdout: raw s16le PCM, interleaved R,L, 48 or 44.1 kS/s -- for either channel
@@ -74,6 +77,7 @@ bool write_full(int fd, const uint8_t *src, size_t n)
 int main(int argc, char *argv[])
 {
     int mode = 0, channels = 1, taps = 51, chunk_blocks = 0, device = -1;
+    long long tune_hz = 0;
     bool stats = false;
     // positional part, as src/project.cpp:278-299
     int npos = 0;
@@ -87,6 +91,12 @@ int main(int argc, char *argv[])
         if (a == "--taps") next(taps);
         else if (a == "--chunk-blocks") next(chunk_blocks);
         else if (a == "--device") next(device);
+        else if (a == "--tune") {
+            if (i + 1 >= argc) usage(argv[0]);
+            char *end = nullptr;
+            tune_hz = std::strtoll(argv[++i], &end, 10);
+            if (end == argv[i] || *end) usage(argv[0]);
+        }
         else if (a == "--stats") stats = true;
         else if (npos < 2) pos[npos++] = argv[i];
         else usage(argv[0]);
@@ -114,6 +124,8 @@ int main(int argc, char *argv[])
         std::fprintf(stderr, "Invalid taps: %d!\n", taps);
         return 1;
     }
+    if (!(std::llabs(tune_hz) < mi.rf_fs / 2))
+        usage(argv[0]);
     if (chunk_blocks <= 0) {
         // about 0.2 s of signal per call: low latency for a live rtl_sdr pipe
         chunk_blocks = static_cast<int>(0.2 * mi.rf_fs * 2 / mi.block_size);
@@ -130,6 +142,10 @@ int main(int argc, char *argv[])
     int rc = fmrx_create(&p, &cfg);
     if (rc != FMRX_OK) {
         std::fprintf(stderr, "fmrx_create: %s (%s)\n", fmrx_strerror(rc), fmrx_last_error());
+        return 1;
+    }
+    if (tune_hz && (rc = fmrx_set_tuning(p, 0, static_cast<double>(tune_hz))) != FMRX_OK) {
+        std::fprintf(stderr, "fmrx_set_tuning: %s (%s)\n", fmrx_strerror(rc), fmrx_last_error());
         return 1;
     }
     const size_t in_bytes = static_cast<size_t>(chunk_blocks) * mi.block_size;

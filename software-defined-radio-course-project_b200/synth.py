@@ -263,3 +263,111 @@ def synth_iq_exact_torch(n_pairs: int, n_captures: int, device, rf_fs: float = 2
             row[2 * s:2 * e:2] = torch.clamp(i, 0, 255).to(torch.uint8)
             row[2 * s + 1:2 * e:2] = torch.clamp(q, 0, 255).to(torch.uint8)
     return out
+
+
+# ----------------------------------------------------------------------------------------
+# Several stations in one stream (what one RTL-SDR capture of the FM band holds)
+# ----------------------------------------------------------------------------------------
+#
+# Station s is ExactSynth's carrier for (station_index, kind), moved to offset_hz from the
+# stream's centre by one more phase term, n * rint(offset/fs * 2^40) in 2^-40 turns (int64
+# wrap), and scaled by gain/256: it adds (cos14[idx] * gain) >> 8 to I and the same of sin14
+# to Q.  The stream carries one noise term, that of the first station's (index, kind).  One
+# station at offset 0 with gain 256 is byte for byte synth_iq_exact.  The helpers below take
+# the backend's int64 arrays (numpy or torch) and its cumulative sum, so that both backends
+# run the same statements.
+
+def _multi_plans(rf_fs: float, stations):
+    plans = []
+    for off, idx, kind, gain in stations:
+        if not abs(off) < rf_fs / 2:
+            raise ValueError(f"offset {off} outside +-rf_fs/2")
+        plans.append((_exact_plan(rf_fs, idx, kind, None, None, None), int(round(off / rf_fs * 2.0 ** 40)), int(gain)))
+    if not plans:
+        raise ValueError("no stations")
+    return plans
+
+
+def _multi_iq(n, plans, carries, tables, consts, cumsum):
+    """I and Q (before clipping) of pairs ``n`` and the carried phase sums: int64 in, int64 out."""
+    sin12, cos14, sin14 = tables
+    gold, mix1, mix2, seed_mix0 = consts
+    acc_i = acc_q = 0
+    new_carries = []
+    for (p, off_inc, gain), carry in zip(plans, carries):
+        def tone(inc):
+            return sin12[((n * inc) & 0xFFFFFFFF) >> 20]
+        sl, sr, sp, s38 = tone(p["inc_l"]), tone(p["inc_r"]), tone(p["inc_p"]), tone(p["inc_38"])
+        mpx = (p["a"] * (sl + sr) + p["b"] * sp) * 32768 + p["a"] * (sl - sr) * s38
+        dphi = ((mpx * p["kdev"] + (1 << 62)) >> 25) - (1 << 37)
+        phi = cumsum(dphi) + carry
+        new_carries.append(phi[-1])
+        idx = ((phi + n * off_inc) >> 26) & 16383
+        acc_i = acc_i + p["carrier"] * ((cos14[idx] * gain) >> 8)
+        acc_q = acc_q + p["carrier"] * ((sin14[idx] * gain) >> 8)
+    p0 = plans[0][0]
+    h = n * gold + seed_mix0
+    h = (h ^ ((h >> 30) & ((1 << 34) - 1))) * mix1
+    h = (h ^ ((h >> 27) & ((1 << 37) - 1))) * mix2
+    h = h ^ ((h >> 31) & ((1 << 33) - 1))
+
+    def noise(shift):
+        b = ((h >> shift) & 255) + ((h >> (shift + 8)) & 255) + ((h >> (shift + 16)) & 255) + ((h >> (shift + 24)) & 255)
+        return (((b - 510) * p0["noise_mul"] + (1 << 40)) >> 8) - (1 << 32)
+    base = 128 * 256 + 128
+    return (base + acc_i + noise(0)) >> 8, (base + acc_q + noise(32)) >> 8, new_carries
+
+
+class ExactMultiSynth:
+    """Stateful numpy generator of several stations in one stream: ``stations`` is a list of
+    ``(offset_hz, station_index, kind, gain)``; ``read(n_pairs)`` returns the next ``2*n_pairs``
+    bytes (any split into reads gives the same bytes)."""
+
+    def __init__(self, rf_fs: float, stations):
+        self.plans = _multi_plans(rf_fs, stations)
+        self.tables = _exact_tables()
+        self.consts = tuple(np.int64(_s64(v)) for v in (_GOLD, _MIX1, _MIX2, self.plans[0][0]["seed_mix"]))
+        self.pos = 0
+        self.carries = [np.int64(0)] * len(self.plans)
+
+    def read(self, n_pairs: int, out: np.ndarray | None = None, chunk: int = 1 << 22) -> np.ndarray:
+        if out is None:
+            out = np.empty(2 * n_pairs, np.uint8)
+        with np.errstate(over="ignore"):
+            for s in range(0, n_pairs, chunk):
+                e = min(n_pairs, s + chunk)
+                n = np.arange(self.pos + s, self.pos + e, dtype=np.int64)
+                i, q, self.carries = _multi_iq(n, self.plans, self.carries, self.tables, self.consts,
+                                               lambda x: np.cumsum(x, dtype=np.int64))
+                out[2 * s:2 * e:2] = np.clip(i, 0, 255).astype(np.uint8)
+                out[2 * s + 1:2 * e:2] = np.clip(q, 0, 255).astype(np.uint8)
+        self.pos += n_pairs
+        return out
+
+
+def synth_iq_exact_multi(n_pairs: int, rf_fs: float, stations, chunk: int = 1 << 22,
+                         out: np.ndarray | None = None) -> np.ndarray:
+    """``2*n_pairs`` uint8 of one stream holding ``stations`` (see ExactMultiSynth), numpy.
+    Bit-identical to synth_iq_exact_multi_torch."""
+    return ExactMultiSynth(rf_fs, stations).read(n_pairs, out=out, chunk=chunk)
+
+
+def synth_iq_exact_multi_torch(n_pairs: int, rf_fs: float, stations, device, chunk: int = 1 << 23, out=None):
+    """``2*n_pairs`` uint8 on ``device``, byte for byte ``synth_iq_exact_multi(n_pairs, rf_fs, stations)``."""
+    import torch
+
+    dev = torch.device(device)
+    plans = _multi_plans(rf_fs, stations)
+    tables = tuple(torch.from_numpy(t).to(dev) for t in _exact_tables())
+    consts = tuple(torch.tensor(_s64(v), dtype=torch.int64, device=dev)
+                   for v in (_GOLD, _MIX1, _MIX2, plans[0][0]["seed_mix"]))
+    if out is None:
+        out = torch.empty(2 * n_pairs, dtype=torch.uint8, device=dev)
+    carries = [torch.zeros((), dtype=torch.int64, device=dev)] * len(plans)
+    for s in range(0, n_pairs, chunk):
+        e = min(n_pairs, s + chunk)
+        n = torch.arange(s, e, dtype=torch.int64, device=dev)
+        i, q, carries = _multi_iq(n, plans, carries, tables, consts, lambda x: torch.cumsum(x, 0))
+        out[2 * s:2 * e:2] = torch.clamp(i, 0, 255).to(torch.uint8)
+        out[2 * s + 1:2 * e:2] = torch.clamp(q, 0, 255).to(torch.uint8)
+    return out
