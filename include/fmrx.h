@@ -289,6 +289,63 @@ int fmrx_rds_pll_state(fmrx_rds *h, float out[6]);
 int fmrx_estimate_psd(float *freq, float *psd, const float *samples, size_t n,
                       int freq_bins, float Fs);
 
+/* ---------------------------------------------------------------------- */
+/* Band scan: where the stations of an IQ capture are, as offsets from its  */
+/* centre frequency (what fmrx_set_tuning takes).                           */
+/* ---------------------------------------------------------------------- */
+/* The spectrum is Welch's averaged periodogram of the complex baseband:
+ * scipy.signal.welch(x, fs=rf_fs, window="hann", nperseg=N, noverlap=N/2,
+ * detrend=False, return_onesided=False, scaling="density"), bins fft-shifted.
+ *   x[n] = (I[n]-128)/128 + j (Q[n]-128)/128, n = pair index from the stream's
+ *          first pair (0 after create or reset; it continues across calls);
+ *   N    = n_fft, a power of two in 256..16384; hop N/2;
+ *   segment j covers pairs [j N/2, j N/2 + N); only whole segments count:
+ *          after P pairs, n_seg = P < N ? 0 : (P - N)/(N/2) + 1;
+ *   w[k] = 0.5 - 0.5 cos(2 pi k/N)  (periodic Hann);
+ *   PSD[m] = sum_j |sum_k w[k] x[jN/2+k] e^{-2 pi i k m'/N}|^2
+ *            / (n_seg rf_fs sum_k w[k]^2)   in full-scale^2/Hz,
+ *          m' = (m - N/2) mod N: output m is f_m = (m - N/2) rf_fs/N, DC at N/2.
+ * Accuracy: |P - P_exact| <= 1e-4 P_exact + 1e-7 max(P_exact) per bin (float
+ * FFT, double sums; a diagnostic off the PCM path like fmrx_estimate_psd).
+ * The same bytes in the same calls give the same bits (no atomics). */
+typedef struct fmrx_scan fmrx_scan;
+/* device -1 = current.  FMRX_ERR_NO_DEVICE without a CUDA device. */
+int fmrx_scan_create(fmrx_scan **out, int n_fft, double rf_fs, int device);
+int fmrx_scan_destroy(fmrx_scan *s);
+/* Back to pair 0, no segments. */
+int fmrx_scan_reset(fmrx_scan *s);
+/* HOST buffer, n_pairs interleaved I,Q pairs; copied to the device with
+ * cudaMemcpyAsync (pinned or not).  Returns when iq may be reused. */
+int fmrx_scan_process(fmrx_scan *s, const uint8_t *iq, size_t n_pairs);
+/* DEVICE buffer on the scanner's device.  Ordered after everything already
+ * enqueued on `stream` (a cudaStream_t; NULL = default stream), and `stream`
+ * is made to wait for it; the call does not synchronise the host. */
+int fmrx_scan_process_device(fmrx_scan *s, const uint8_t *iq_dev, size_t n_pairs, void *stream);
+/* psd: n_fft doubles, fft-shifted, full-scale^2/Hz (zeros while *n_segments == 0);
+ * n >= n_fft; n_segments may be NULL.  Waits for the device. */
+int fmrx_scan_read(fmrx_scan *s, double *psd, size_t n, uint64_t *n_segments);
+
+/* Station finder over a spectrum of n_fft bins as fmrx_scan_read gives it.
+ * Host code, double, deterministic; no device needed.
+ *   df = rf_fs/N; h = floor(channel_hz/(2 df) + 0.5), h >= 1 and 2h+1 <= N
+ *   (else FMRX_ERR_ARG);
+ *   floor = sorted(PSD)[floor(0.1 (N-1))]  (10th percentile, lower rank);
+ *   mean(m) = mean of PSD[m-h .. m+h] for centres m in [h, N-1-h];
+ *   candidates: mean(m) >= floor 10^(threshold_db/10) and mean(m) > 0;
+ *   visited by descending mean (ties: lower m first), a candidate is accepted
+ *   when |m - a| df >= channel_hz for every accepted centre a;
+ *   each accepted centre: offset_hz = sum f_k q_k / sum q_k over its window,
+ *   q_k = max(PSD_k - floor, 0) (the power centroid: an FM signal's long-run
+ *   spectrum follows its instantaneous frequency, whose mean is the carrier);
+ *   level_db = 10 log10(sum PSD_k df); snr_db = 10 log10(mean(m)/floor).
+ * Writes min(found, max_out) stations in ascending offset, *n_found = found.
+ * threshold_db <= 0 -> 10; channel_hz <= 0 -> 200e3; non-finite: FMRX_ERR_ARG. */
+typedef struct {
+    double offset_hz, level_db, snr_db;
+} fmrx_station;
+int fmrx_find_stations(const double *psd, int n_fft, double rf_fs, double threshold_db, double channel_hz,
+                       fmrx_station *out, int max_out, int *n_found);
+
 #ifdef __cplusplus
 }
 #endif

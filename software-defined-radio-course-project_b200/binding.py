@@ -9,6 +9,7 @@ if the CUDA extension is missing or no B200 is visible, calls raise
 from __future__ import annotations
 
 import ctypes as C
+from collections import namedtuple
 from pathlib import Path
 
 import numpy as np
@@ -43,6 +44,8 @@ ABI_SYMBOLS = (
     "fmrx_long_last_ms", "fmrx_long_pll_state",
     "fmrx_rds_create", "fmrx_rds_destroy", "fmrx_rds_reset", "fmrx_rds_process", "fmrx_rds_pll_state",
     "fmrx_estimate_psd",
+    "fmrx_scan_create", "fmrx_scan_destroy", "fmrx_scan_reset", "fmrx_scan_process", "fmrx_scan_process_device",
+    "fmrx_scan_read", "fmrx_find_stations",
 )
 
 
@@ -61,6 +64,10 @@ class ModeInfoStruct(C.Structure):
 class ConfigStruct(C.Structure):
     _fields_ = [("mode", C.c_int), ("taps", C.c_int), ("n_captures", C.c_int), ("device", C.c_int),
                 ("chunk_blocks", C.c_int), ("keep_stages", C.c_int), ("n_sets", C.c_int), ("reserved", C.c_int * 3)]
+
+
+class StationStruct(C.Structure):
+    _fields_ = [("offset_hz", C.c_double), ("level_db", C.c_double), ("snr_db", C.c_double)]
 
 
 class ModeInfo:
@@ -130,6 +137,14 @@ def load() -> C.CDLL:
     L.fmrx_set_timing.argtypes = [C.c_void_p, C.c_int]
     L.fmrx_last_timing.argtypes = [C.c_void_p, _f32p]
     L.fmrx_set_tuning.argtypes = [C.c_void_p, C.c_int, C.c_double]
+    L.fmrx_scan_create.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.c_double, C.c_int]
+    L.fmrx_scan_destroy.argtypes = [C.c_void_p]
+    L.fmrx_scan_reset.argtypes = [C.c_void_p]
+    L.fmrx_scan_process.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t]
+    L.fmrx_scan_process_device.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
+    L.fmrx_scan_read.argtypes = [C.c_void_p, C.POINTER(C.c_double), C.c_size_t, C.POINTER(C.c_uint64)]
+    L.fmrx_find_stations.argtypes = [C.POINTER(C.c_double), C.c_int, C.c_double, C.c_double, C.c_double,
+                                     C.POINTER(StationStruct), C.c_int, C.POINTER(C.c_int)]
     _lib = L
     return L
 
@@ -469,3 +484,82 @@ def estimatePSD(samples, freq_bins: int, Fs: float):
     p = np.zeros(freq_bins // 2, np.float32)
     _check(L.fmrx_estimate_psd(_fp(f), _fp(p), _fp(x), len(x), freq_bins, Fs), "fmrx_estimate_psd")
     return f, p
+
+
+# ---- band scan ----------------------------------------------------------------
+
+Station = namedtuple("Station", "offset_hz level_db snr_db")
+
+
+class Scanner:
+    """Welch's averaged periodogram of a complex u8 IQ stream on the device (fmrx_scan_*; the definition is in
+    include/fmrx.h): ``process`` / ``process_device`` feed pairs (the stream continues across calls), ``spectrum``
+    returns ``(freq_hz, psd, n_segments)`` with the bins fft-shifted, DC at ``n_fft // 2``."""
+
+    def __init__(self, rf_fs: float, n_fft: int = 4096, device: int = -1):
+        self._L = load()
+        self.rf_fs = float(rf_fs)
+        self.n_fft = int(n_fft)
+        h = C.c_void_p()
+        _check(self._L.fmrx_scan_create(C.byref(h), self.n_fft, self.rf_fs, device), "fmrx_scan_create")
+        self._h = h
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._L.fmrx_scan_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        self.close()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def reset(self):
+        _check(self._L.fmrx_scan_reset(self._h), "fmrx_scan_reset")
+
+    def process(self, iq):
+        """Host uint8, 1-D, interleaved I,Q (an odd trailing byte is an error)."""
+        iq = np.ascontiguousarray(iq, np.uint8)
+        if iq.ndim != 1 or len(iq) % 2:
+            raise ValueError("iq: a 1-D uint8 array of whole I,Q pairs")
+        _check(self._L.fmrx_scan_process(self._h, iq.ctypes.data, len(iq) // 2), "fmrx_scan_process")
+
+    def process_device(self, iq_ptr: int, n_pairs: int, stream: int = 0):
+        """A device pointer on the scanner's device; ordered on ``stream``, asynchronous w.r.t. the host."""
+        _check(self._L.fmrx_scan_process_device(self._h, iq_ptr, n_pairs, stream), "fmrx_scan_process_device")
+
+    def spectrum(self):
+        psd = np.zeros(self.n_fft, np.float64)
+        n = C.c_uint64(0)
+        _check(self._L.fmrx_scan_read(self._h, psd.ctypes.data_as(C.POINTER(C.c_double)), self.n_fft, C.byref(n)),
+               "fmrx_scan_read")
+        freq = (np.arange(self.n_fft) - self.n_fft // 2) * (self.rf_fs / self.n_fft)
+        return freq, psd, int(n.value)
+
+
+def find_stations(psd, rf_fs: float, threshold_db: float = 10.0, channel_hz: float = 200e3) -> list:
+    """Stations in a spectrum as ``Scanner.spectrum`` returns it (fmrx_find_stations, host code): a list of
+    ``Station(offset_hz, level_db, snr_db)`` in ascending offset."""
+    L = load()
+    psd = np.ascontiguousarray(psd, np.float64)
+    n_fft = len(psd)
+    cap = max(1, n_fft)
+    out = (StationStruct * cap)()
+    found = C.c_int(0)
+    _check(L.fmrx_find_stations(psd.ctypes.data_as(C.POINTER(C.c_double)), n_fft, float(rf_fs), float(threshold_db),
+                                float(channel_hz), out, cap, C.byref(found)), "fmrx_find_stations")
+    return [Station(out[i].offset_hz, out[i].level_db, out[i].snr_db) for i in range(found.value)]
+
+
+def scan(iq, rf_fs: float, n_fft: int = 4096, threshold_db: float = 10.0, channel_hz: float = 200e3,
+         device: int = -1) -> list:
+    """The stations of a host IQ capture (uint8, interleaved I,Q) in one call: ``Scanner`` then ``find_stations``.
+    Their ``offset_hz`` are what ``Pipeline(tune_hz=...)`` takes."""
+    with Scanner(rf_fs, n_fft, device) as s:
+        s.process(iq)
+        _, psd, _ = s.spectrum()
+    return find_stations(psd, rf_fs, threshold_db, channel_hz)

@@ -1588,3 +1588,344 @@ extern "C" int fmrx_estimate_psd(float *freq, float *psd, const float *samples, 
     CU(cudaMemcpy(psd, d_p.p, half * sizeof(float), cudaMemcpyDeviceToHost));
     return FMRX_OK;
 }
+
+// ---------------------------------------------------------------------------
+// Band scan: Welch's averaged periodogram of the complex u8 IQ stream, and the station finder (include/fmrx.h)
+// ---------------------------------------------------------------------------
+// The handle keeps the stream's tail (pairs [n_seg*H, pairs), fewer than N) on the device.  A call first runs the at
+// most two segments that start in that tail, assembled from the tail and the head of the new input, then the segments
+// that lie wholly in the new input, straight from the caller's device buffer (fmrx_scan_process_device) or from
+// device staging chunks (fmrx_scan_process).  Launches cover whole runs (scan_run_segments) counted from the call's
+// first wholly-new segment, and the staging chunks are whole runs too, so both paths add the same partial sums in the
+// same order.
+struct fmrx_scan {
+    int device = 0, n = 0;
+    double fs = 0, win_sq = 0;                 // sum of the double window's squares
+    cudaStream_t st = nullptr, cp = nullptr;   // compute, staging copies (host path)
+    cudaEvent_t ev_in = nullptr, ev_out = nullptr, ev_copied[2] = {}, ev_used[2] = {};
+    float *d_win = nullptr;
+    float2 *d_tw = nullptr;
+    double *d_acc = nullptr, *d_partial = nullptr;
+    size_t partial_runs = 0;                   // capacity of d_partial in runs of N doubles
+    uint8_t *d_tail[2] = {}, *d_asm = nullptr, *d_stage[2] = {};
+    size_t stage_cap = 0;                      // bytes of each d_stage
+    int cur = 0;                               // d_tail[cur] holds the tail
+    uint64_t pairs = 0, n_seg = 0;
+};
+
+namespace {
+
+constexpr size_t kScanPartialDoubles = size_t(1) << 24;   // 128 MB: the largest partial buffer (4096 runs at N = 4096)
+constexpr size_t kScanStageBytes = size_t(1) << 26;       // per host-path staging buffer: 512 runs of 2^16 pairs
+
+bool scan_n_ok(int n_fft) { return n_fft >= 256 && n_fft <= 16384 && (n_fft & (n_fft - 1)) == 0; }
+
+void free_scan(fmrx_scan *s)
+{
+    if (!s)
+        return;
+    cudaSetDevice(s->device);
+    cudaDeviceSynchronize();
+    for (void *q : { (void *)s->d_win, (void *)s->d_tw, (void *)s->d_acc, (void *)s->d_tail[0], (void *)s->d_tail[1],
+                     (void *)s->d_asm, (void *)s->d_partial, (void *)s->d_stage[0], (void *)s->d_stage[1] })
+        if (q)
+            cudaFree(q);
+    for (cudaEvent_t e : { s->ev_in, s->ev_out, s->ev_copied[0], s->ev_copied[1], s->ev_used[0], s->ev_used[1] })
+        if (e)
+            cudaEventDestroy(e);
+    for (cudaStream_t q : { s->st, s->cp })
+        if (q)
+            cudaStreamDestroy(q);
+    delete s;
+}
+
+int scan_create_impl(fmrx_scan *s)
+{
+    const int N = s->n;
+    CU(cudaStreamCreateWithFlags(&s->st, cudaStreamNonBlocking));
+    CU(cudaStreamCreateWithFlags(&s->cp, cudaStreamNonBlocking));
+    for (cudaEvent_t *e : { &s->ev_in, &s->ev_out, &s->ev_copied[0], &s->ev_copied[1], &s->ev_used[0], &s->ev_used[1] })
+        CU(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
+    // the periodic Hann window and the twiddles, in double, rounded to float
+    std::vector<float> win(N);
+    std::vector<float2> tw(N / 2);
+    const double two_pi = 2.0 * 3.14159265358979323846;
+    s->win_sq = 0.0;
+    for (int k = 0; k < N; k++) {
+        const double w = 0.5 - 0.5 * std::cos(two_pi * k / N);
+        win[k] = static_cast<float>(w);
+        s->win_sq += w * w;
+    }
+    for (int k = 0; k < N / 2; k++)
+        tw[k] = make_float2(static_cast<float>(std::cos(two_pi * k / N)), static_cast<float>(-std::sin(two_pi * k / N)));
+    CU(dalloc(&s->d_win, N));
+    CU(dalloc(&s->d_tw, N / 2));
+    CU(dalloc(&s->d_acc, N));
+    CU(dalloc(&s->d_tail[0], 2 * N));
+    CU(dalloc(&s->d_tail[1], 2 * N));
+    CU(dalloc(&s->d_asm, 3 * N));              // the tail and the head of a call: two segments, 3N/2 pairs
+    CU(cudaMemcpy(s->d_win, win.data(), N * sizeof(float), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(s->d_tw, tw.data(), N / 2 * sizeof(float2), cudaMemcpyHostToDevice));
+    CU(cudaMemset(s->d_acc, 0, N * sizeof(double)));
+    return FMRX_OK;
+}
+
+// Segments [0, n_seg) of the pairs at iq (device), added to the accumulator on s->st in launches of whole runs.
+int scan_segments(fmrx_scan *s, const uint8_t *iq, uint64_t n_seg)
+{
+    const int N = s->n, H = N / 2, R = scan_run_segments(N);
+    const uint64_t runs_total = (n_seg + R - 1) / R;
+    const size_t max_runs = kScanPartialDoubles / N;
+    const size_t want = static_cast<size_t>(std::min<uint64_t>(runs_total, max_runs));
+    if (want > s->partial_runs) {
+        if (s->d_partial)
+            CU(cudaFreeAsync(s->d_partial, s->st));
+        s->d_partial = nullptr;
+        s->partial_runs = 0;
+        CU(cudaMallocAsync(reinterpret_cast<void **>(&s->d_partial), want * N * sizeof(double), s->st));
+        s->partial_runs = want;
+    }
+    const uint64_t per_launch = static_cast<uint64_t>(max_runs) * R;
+    for (uint64_t j = 0; j < n_seg; j += per_launch) {
+        const int k = static_cast<int>(std::min<uint64_t>(per_launch, n_seg - j));
+        CU(launch_scan(iq + 2 * j * H, k, N, s->d_win, s->d_tw, s->d_partial, s->d_acc, s->st));
+    }
+    return FMRX_OK;
+}
+
+// One call: `src` is a host pointer (host = true) or a device pointer ordered on s->st.
+int scan_run(fmrx_scan *s, const uint8_t *src, uint64_t n, bool host)
+{
+    const uint64_t N = s->n, H = N / 2;
+    const cudaMemcpyKind in_kind = host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
+    const uint64_t P = s->pairs, start = s->n_seg * H, tl = P - start, end = P + n;
+    // 1. segments that start in the tail: at `start` and `start + H`, whole ones only
+    uint64_t k_str = 0;
+    while (k_str < 2 && start + k_str * H < P && start + k_str * H + N <= end)
+        k_str++;
+    if (k_str) {
+        const uint64_t head = start + (k_str - 1) * H + N - P;
+        CU(cudaMemcpyAsync(s->d_asm, s->d_tail[s->cur], 2 * tl, cudaMemcpyDeviceToDevice, s->st));
+        CU(cudaMemcpyAsync(s->d_asm + 2 * tl, src, 2 * head, in_kind, s->st));
+        const int rc = scan_segments(s, s->d_asm, k_str);
+        if (rc != FMRX_OK)
+            return rc;
+    }
+    // 2. segments wholly in the new input (none if a segment starting in the tail is still incomplete)
+    const uint64_t next = start + k_str * H;
+    uint64_t k_main = 0;
+    if (next >= P && end - next >= N)
+        k_main = (end - next - N) / H + 1;
+    if (k_main) {
+        const uint8_t *base = src + 2 * (next - P);
+        if (!host) {
+            const int rc = scan_segments(s, base, k_main);
+            if (rc != FMRX_OK)
+                return rc;
+        } else {
+            // whole runs per staging chunk, double-buffered: copies on s->cp under the kernels on s->st
+            const uint64_t R = scan_run_segments(s->n);
+            const uint64_t chunk = std::max<uint64_t>(1, kScanStageBytes / (2 * R * H)) * R;   // segments
+            const size_t need = static_cast<size_t>(2 * ((std::min(chunk, k_main) - 1) * H + N));
+            if (need > s->stage_cap) {
+                for (uint8_t *&q : s->d_stage) {
+                    if (q)
+                        CU(cudaFreeAsync(q, s->st));
+                    q = nullptr;
+                }
+                s->stage_cap = 0;
+                for (uint8_t *&q : s->d_stage)
+                    CU(cudaMallocAsync(reinterpret_cast<void **>(&q), need, s->st));
+                s->stage_cap = need;
+            }
+            CU(cudaEventRecord(s->ev_used[0], s->st));        // (the allocations above are ordered on s->st)
+            CU(cudaEventRecord(s->ev_used[1], s->st));
+            int b = 0;
+            for (uint64_t j = 0; j < k_main; j += chunk, b ^= 1) {
+                const uint64_t k = std::min(chunk, k_main - j);
+                CU(cudaStreamWaitEvent(s->cp, s->ev_used[b], 0));
+                CU(cudaMemcpyAsync(s->d_stage[b], base + 2 * j * H, 2 * ((k - 1) * H + N), cudaMemcpyHostToDevice, s->cp));
+                CU(cudaEventRecord(s->ev_copied[b], s->cp));
+                CU(cudaStreamWaitEvent(s->st, s->ev_copied[b], 0));
+                const int rc = scan_segments(s, s->d_stage[b], k);
+                if (rc != FMRX_OK)
+                    return rc;
+                CU(cudaEventRecord(s->ev_used[b], s->st));
+            }
+        }
+    }
+    // 3. the new tail: pairs [n_seg*H, end), from the old tail and the new input
+    s->n_seg += k_str + k_main;
+    const uint64_t ns = s->n_seg * H;
+    uint8_t *dst = s->d_tail[s->cur ^ 1];
+    uint64_t a = 0;
+    if (ns < P) {
+        a = P - ns;
+        CU(cudaMemcpyAsync(dst, s->d_tail[s->cur] + 2 * (ns - start), 2 * a, cudaMemcpyDeviceToDevice, s->st));
+    }
+    const uint64_t from = ns > P ? ns - P : 0;
+    if (n > from)
+        CU(cudaMemcpyAsync(dst + 2 * a, src + 2 * from, 2 * (n - from), in_kind, s->st));
+    s->cur ^= 1;
+    s->pairs = end;
+    return FMRX_OK;
+}
+
+}  // namespace
+
+extern "C" int fmrx_scan_create(fmrx_scan **out, int n_fft, double rf_fs, int device)
+{
+    if (!out || !scan_n_ok(n_fft) || !(rf_fs > 0) || !std::isfinite(rf_fs))
+        return FMRX_ERR_ARG;
+    *out = nullptr;
+    if (fmrx_device_count() < 1) {
+        std::snprintf(g_err, sizeof(g_err), "no CUDA device");
+        return FMRX_ERR_NO_DEVICE;
+    }
+    if (device < 0)
+        CU(cudaGetDevice(&device));
+    CU(cudaSetDevice(device));
+    cudaDeviceProp prop;
+    CU(cudaGetDeviceProperties(&prop, device));
+    if (prop.major != 10) {
+        std::snprintf(g_err, sizeof(g_err), "device %d is sm_%d%d; this library is sm_100a only", device, prop.major,
+                      prop.minor);
+        return FMRX_ERR_NO_DEVICE;
+    }
+    fmrx_scan *s = new (std::nothrow) fmrx_scan();
+    if (!s)
+        return FMRX_ERR_ALLOC;
+    s->device = device;
+    s->n = n_fft;
+    s->fs = rf_fs;
+    const int rc = scan_create_impl(s);
+    if (rc != FMRX_OK) {
+        free_scan(s);
+        return rc;
+    }
+    *out = s;
+    return FMRX_OK;
+}
+
+extern "C" int fmrx_scan_destroy(fmrx_scan *s)
+{
+    free_scan(s);
+    return FMRX_OK;
+}
+
+extern "C" int fmrx_scan_reset(fmrx_scan *s)
+{
+    if (!s)
+        return FMRX_ERR_ARG;
+    CU(cudaSetDevice(s->device));
+    CU(cudaStreamSynchronize(s->st));
+    CU(cudaMemset(s->d_acc, 0, s->n * sizeof(double)));
+    s->pairs = 0;
+    s->n_seg = 0;
+    return FMRX_OK;
+}
+
+extern "C" int fmrx_scan_process(fmrx_scan *s, const uint8_t *iq, size_t n_pairs)
+{
+    if (!s || (!iq && n_pairs))
+        return FMRX_ERR_ARG;
+    if (!n_pairs)
+        return FMRX_OK;
+    CU(cudaSetDevice(s->device));
+    const int rc = scan_run(s, iq, n_pairs, true);
+    CU(cudaStreamSynchronize(s->st));          // the caller may reuse iq on return
+    return rc;
+}
+
+extern "C" int fmrx_scan_process_device(fmrx_scan *s, const uint8_t *iq_dev, size_t n_pairs, void *stream)
+{
+    if (!s || (!iq_dev && n_pairs))
+        return FMRX_ERR_ARG;
+    if (!n_pairs)
+        return FMRX_OK;
+    CU(cudaSetDevice(s->device));
+    cudaStream_t caller = static_cast<cudaStream_t>(stream);
+    CU(cudaEventRecord(s->ev_in, caller));
+    CU(cudaStreamWaitEvent(s->st, s->ev_in, 0));
+    const int rc = scan_run(s, iq_dev, n_pairs, false);
+    CU(cudaEventRecord(s->ev_out, s->st));
+    CU(cudaStreamWaitEvent(caller, s->ev_out, 0));
+    return rc;
+}
+
+extern "C" int fmrx_scan_read(fmrx_scan *s, double *psd, size_t n, uint64_t *n_segments)
+{
+    if (!s || !psd || n < static_cast<size_t>(s->n))
+        return FMRX_ERR_ARG;
+    CU(cudaSetDevice(s->device));
+    CU(cudaStreamSynchronize(s->st));
+    CU(cudaMemcpy(psd, s->d_acc, s->n * sizeof(double), cudaMemcpyDeviceToHost));
+    const double norm = s->n_seg ? 1.0 / (static_cast<double>(s->n_seg) * s->fs * s->win_sq) : 0.0;
+    for (int m = 0; m < s->n; m++)
+        psd[m] = s->n_seg ? psd[m] * norm : 0.0;
+    if (n_segments)
+        *n_segments = s->n_seg;
+    return FMRX_OK;
+}
+
+extern "C" int fmrx_find_stations(const double *psd, int n_fft, double rf_fs, double threshold_db, double channel_hz,
+                                  fmrx_station *out, int max_out, int *n_found)
+{
+    if (!psd || !n_found || max_out < 0 || (!out && max_out) || !scan_n_ok(n_fft) || !(rf_fs > 0) ||
+        !std::isfinite(rf_fs) || !std::isfinite(threshold_db) || !std::isfinite(channel_hz))
+        return FMRX_ERR_ARG;
+    if (threshold_db <= 0)
+        threshold_db = 10.0;
+    if (channel_hz <= 0)
+        channel_hz = 200e3;
+    const int N = n_fft;
+    const double df = rf_fs / N;
+    const double hh = std::floor(channel_hz / (2.0 * df) + 0.5);
+    if (!(hh >= 1) || 2 * hh + 1 > N)
+        return FMRX_ERR_ARG;
+    const int h = static_cast<int>(hh);
+    std::vector<double> sorted(psd, psd + N);
+    std::sort(sorted.begin(), sorted.end());
+    const double floor_ = sorted[static_cast<size_t>(std::floor(0.1 * (N - 1)))];
+    const double thr = floor_ * std::pow(10.0, threshold_db / 10.0);
+    struct Cand { int m; double mean; };
+    std::vector<Cand> cand;
+    for (int m = h; m <= N - 1 - h; m++) {
+        double sum = 0.0;
+        for (int k = m - h; k <= m + h; k++)
+            sum += psd[k];
+        const double mean = sum / (2 * h + 1);
+        if (mean >= thr && mean > 0)
+            cand.push_back({ m, mean });
+    }
+    std::sort(cand.begin(), cand.end(), [](const Cand &a, const Cand &b) {
+        return a.mean != b.mean ? a.mean > b.mean : a.m < b.m;
+    });
+    std::vector<Cand> acc;
+    for (const Cand &c : cand) {
+        bool ok = true;
+        for (const Cand &a : acc)
+            if (std::abs(c.m - a.m) * df < channel_hz) {
+                ok = false;
+                break;
+            }
+        if (ok)
+            acc.push_back(c);
+    }
+    std::vector<fmrx_station> st;
+    for (const Cand &c : acc) {
+        double sq = 0.0, sfq = 0.0, sp = 0.0;
+        for (int k = c.m - h; k <= c.m + h; k++) {
+            const double q = std::max(psd[k] - floor_, 0.0);
+            sq += q;
+            sfq += (k - N / 2) * df * q;
+            sp += psd[k];
+        }
+        st.push_back({ sfq / sq, 10.0 * std::log10(sp * df), 10.0 * std::log10(c.mean / floor_) });
+    }
+    std::sort(st.begin(), st.end(), [](const fmrx_station &a, const fmrx_station &b) { return a.offset_hz < b.offset_hz; });
+    *n_found = static_cast<int>(st.size());
+    for (int i = 0; i < max_out && i < static_cast<int>(st.size()); i++)
+        out[i] = st[i];
+    return FMRX_OK;
+}

@@ -119,4 +119,12 @@ cudaError_t launch_rds_mix(float *out, const float *trig, const float *chan, con
 // spectrum tap: the reference's estimatePSD (src/fourier.cpp:35-117); freq_bins * 20 bytes of dynamic shared memory
 cudaError_t launch_psd(float *psd, const float *samples, int n_seg, int freq_bins, float Fs, cudaStream_t s);
 
+// band scan (fmrx_scan.cu): Welch segments of n_fft pairs, hop n_fft/2.  Segment j of a launch covers pairs
+// [j*n_fft/2, j*n_fft/2 + n_fft) of iq.  The launch sums runs of scan_run_segments(n_fft) consecutive segments into
+// partial[run][n_fft] (fft-shifted) and then adds the runs, in order, to acc[n_fft]; partial must hold
+// ceil(n_seg / scan_run_segments(n_fft)) * n_fft doubles.  win: n_fft floats; tw: n_fft/2 float2, e^{-2 pi i k/n_fft}.
+int scan_run_segments(int n_fft);
+cudaError_t launch_scan(const uint8_t *iq, int n_seg, int n_fft, const float *win, const float2 *tw, double *partial,
+                        double *acc, cudaStream_t s);
+
 }  // namespace fmrx

@@ -2,9 +2,19 @@
 //
 //   project                      mode 0 (message says "mono", like the reference)
 //   project <mode 0-3> <1|2|m|s> [--taps N] [--chunk-blocks K] [--device D] [--tune HZ] [--stats]
+//   project <mode 0-3> <1|2|m|s> --scan SECONDS [--fft N] [--threshold DB] [--device D]
 //
 // --tune HZ: decode the station HZ (an integer, may be negative) above the capture's centre
 // frequency (fmrx_set_tuning); |HZ| < rf_fs/2 of the mode, else the usage message and exit 1.
+//
+// --scan SECONDS: decode nothing; find the stations in up to SECONDS of signal at the mode's
+// RF rate (0: until EOF), read and scanned chunk by chunk (fmrx_scan_process, so a live
+// rtl_sdr pipe works), and print one line per station on stdout in ascending offset:
+// offset_hz<TAB>level_db<TAB>snr_db, the offset an integer, the levels to 0.1 dB
+// (fmrx_find_stations) -- the offsets are what --tune takes.  Exit status 0.  --fft N: the
+// Welch segment length, a power of two in 256..16384 (default 4096); --threshold DB: the
+// detection threshold above the noise floor (default 10).  Malformed values, --fft or
+// --threshold without --scan, and --scan with --tune: the usage message and exit 1.
 //
 // stdin : raw interleaved u8 I/Q at the mode's RF rate
 // stdout: raw s16le PCM, interleaved R,L, 48 or 44.1 kS/s -- for either channel
@@ -24,7 +34,9 @@
 // processing chunk i and writing chunk i-1 overlap (live use: rtl_sdr | project | aplay,
 // src/project.cpp:392-393).  --stats prints the sustained real-time factor and the
 // per-chunk latency (last input byte read -> last PCM byte written) on stderr.
+#include <algorithm>
 #include <chrono>
+#include <cmath>
 #include <condition_variable>
 #include <cstdint>
 #include <cstdio>
@@ -43,8 +55,9 @@ namespace {
 [[noreturn]] void usage(const char *argv0)
 {
     std::fprintf(stderr, "Usage: %s\nor \nUsage %s <mode> <channels>\n"
-                         "\t\t<mode> is a value from 0 to 3\n\t\t   <channels> is either 1 or 2\n",
-                 argv0, argv0);
+                         "\t\t<mode> is a value from 0 to 3\n\t\t   <channels> is either 1 or 2\n"
+                         "or\nUsage %s <mode> <channels> --scan SECONDS [--fft N] [--threshold DB]\n",
+                 argv0, argv0, argv0);
     std::exit(1);
 }
 
@@ -58,6 +71,50 @@ size_t read_full(int fd, uint8_t *dst, size_t want)
         got += static_cast<size_t>(r);
     }
     return got;
+}
+
+// --scan: the stations in up to `seconds` of stdin (0: until EOF); exit status 0
+int scan_stdin(const fmrx_mode_info &mi, int device, double seconds, int fft, double threshold_db)
+{
+    fmrx_scan *sc = nullptr;
+    int rc = fmrx_scan_create(&sc, fft, mi.rf_fs, device);
+    if (rc != FMRX_OK) {
+        std::fprintf(stderr, "fmrx_scan_create: %s (%s)\n", fmrx_strerror(rc), fmrx_last_error());
+        return 1;
+    }
+    const uint64_t limit = seconds > 0 ? static_cast<uint64_t>(seconds * mi.rf_fs) : UINT64_MAX;
+    const size_t chunk = static_cast<size_t>(0.2 * mi.rf_fs);      // pairs per read: about 0.2 s of signal
+    void *buf = nullptr;
+    if (fmrx_host_alloc(&buf, 2 * chunk) != FMRX_OK) {
+        std::fprintf(stderr, "pinned allocation failed (%s)\n", fmrx_last_error());
+        return 1;
+    }
+    for (uint64_t done = 0; done < limit;) {
+        const size_t want = static_cast<size_t>(std::min<uint64_t>(chunk, limit - done));
+        const size_t got = read_full(STDIN_FILENO, static_cast<uint8_t *>(buf), 2 * want) / 2;   // whole pairs
+        if (got && (rc = fmrx_scan_process(sc, static_cast<const uint8_t *>(buf), got)) != FMRX_OK) {
+            std::fprintf(stderr, "fmrx_scan_process: %s (%s)\n", fmrx_strerror(rc), fmrx_last_error());
+            return 1;
+        }
+        done += got;
+        if (got < want)
+            break;
+    }
+    std::vector<double> psd(fft);
+    uint64_t n_seg = 0;
+    std::vector<fmrx_station> st(fft);
+    int found = 0;
+    if ((rc = fmrx_scan_read(sc, psd.data(), psd.size(), &n_seg)) != FMRX_OK ||
+        (rc = fmrx_find_stations(psd.data(), fft, mi.rf_fs, threshold_db, 0.0, st.data(), fft, &found)) != FMRX_OK) {
+        std::fprintf(stderr, "band scan: %s (%s)\n", fmrx_strerror(rc), fmrx_last_error());
+        return 1;
+    }
+    for (int i = 0; i < found; i++)
+        std::printf("%lld\t%.1f\t%.1f\n", std::llround(st[i].offset_hz), st[i].level_db, st[i].snr_db);
+    std::fflush(stdout);
+    fmrx_host_free(buf);
+    fmrx_scan_destroy(sc);
+    return 0;
 }
 
 bool write_full(int fd, const uint8_t *src, size_t n)
@@ -78,7 +135,9 @@ int main(int argc, char *argv[])
 {
     int mode = 0, channels = 1, taps = 51, chunk_blocks = 0, device = -1;
     long long tune_hz = 0;
-    bool stats = false;
+    bool stats = false, tuned = false, scan = false, scan_opts = false;
+    double scan_s = 0.0, threshold_db = 10.0;
+    int fft = 4096;
     // positional part, as src/project.cpp:278-299
     int npos = 0;
     const char *pos[2] = { nullptr, nullptr };
@@ -96,6 +155,29 @@ int main(int argc, char *argv[])
             char *end = nullptr;
             tune_hz = std::strtoll(argv[++i], &end, 10);
             if (end == argv[i] || *end) usage(argv[0]);
+            tuned = true;
+        }
+        else if (a == "--scan" || a == "--threshold") {
+            if (i + 1 >= argc) usage(argv[0]);
+            char *end = nullptr;
+            const double v = std::strtod(argv[++i], &end);
+            if (end == argv[i] || *end || !std::isfinite(v)) usage(argv[0]);
+            if (a == "--scan") {
+                if (v < 0) usage(argv[0]);
+                scan = true;
+                scan_s = v;
+            } else {
+                threshold_db = v;
+                scan_opts = true;
+            }
+        }
+        else if (a == "--fft") {
+            if (i + 1 >= argc) usage(argv[0]);
+            char *end = nullptr;
+            const long v = std::strtol(argv[++i], &end, 10);
+            if (end == argv[i] || *end || v < 256 || v > 16384 || (v & (v - 1))) usage(argv[0]);
+            fft = static_cast<int>(v);
+            scan_opts = true;
         }
         else if (a == "--stats") stats = true;
         else if (npos < 2) pos[npos++] = argv[i];
@@ -117,6 +199,8 @@ int main(int argc, char *argv[])
             return 1;
         }
     }
+    if ((scan && tuned) || (scan_opts && !scan))
+        usage(argv[0]);
     std::fprintf(stderr, "Operating in mode %d, %s\n", mode, channels == 1 ? "mono" : "stereo");
 
     fmrx_mode_info mi;
@@ -126,6 +210,8 @@ int main(int argc, char *argv[])
     }
     if (!(std::llabs(tune_hz) < mi.rf_fs / 2))
         usage(argv[0]);
+    if (scan)
+        return scan_stdin(mi, device, scan_s, fft, threshold_db);
     if (chunk_blocks <= 0) {
         // about 0.2 s of signal per call: low latency for a live rtl_sdr pipe
         chunk_blocks = static_cast<int>(0.2 * mi.rf_fs * 2 / mi.block_size);
