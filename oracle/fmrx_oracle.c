@@ -274,6 +274,10 @@ struct orc_chain {
     /* scratch */
     float *iq, *ib, *qb, *i_ds, *q_ds, *demod, *chan, *pilot, *trig, *mixer;
     float *mono, *mono_shift, *stereo, *left, *right;
+    /* tuning mixer (orc_chain_set_tuning): the chain is tuned iff cos_t is set */
+    float *cos_t, *sin_t;
+    uint32_t inc;
+    uint64_t pairs_done;             /* pairs run since create */
 };
 
 static float *zalloc_f(size_t n)
@@ -327,13 +331,34 @@ void orc_chain_destroy(orc_chain *c)
                      c->st_i, c->st_q, c->st_chan, c->st_pilot, c->st_audio,
                      c->iq, c->ib, c->qb, c->i_ds, c->q_ds, c->demod, c->chan,
                      c->pilot, c->trig, c->mixer, c->mono, c->mono_shift,
-                     c->stereo, c->left, c->right };
+                     c->stereo, c->left, c->right, c->cos_t, c->sin_t };
     for (size_t i = 0; i < sizeof(all) / sizeof(all[0]); i++)
         free(all[i]);
     free(c);
 }
 
 const orc_mode *orc_chain_mode(const orc_chain *c) { return &c->m; }
+
+/* The tuning mixer, defined in fmrx_oracle.h.  Its tables are built here,
+ * apart from the product's (fmrx_taps.cpp). */
+#define ORC_TUNE_TABLE 65536
+
+int orc_chain_set_tuning(orc_chain *c, double offset_hz)
+{
+    if (!(fabs(offset_hz) < (double)c->m.rf_fs / 2.0) || c->pairs_done != 0)
+        return -1;
+    if (!c->cos_t) {
+        c->cos_t = zalloc_f(ORC_TUNE_TABLE);
+        c->sin_t = zalloc_f(ORC_TUNE_TABLE);
+        for (int k = 0; k < ORC_TUNE_TABLE; k++) {
+            const double a = 6.283185307179586 * (double)k / 65536.0;
+            c->cos_t[k] = (float)cos(a);
+            c->sin_t[k] = (float)sin(a);
+        }
+    }
+    c->inc = (uint32_t)llrint(offset_hz * 4294967296.0 / (double)c->m.rf_fs);
+    return 0;
+}
 
 static void put(float *dst, const float *src, int n)
 {
@@ -354,6 +379,17 @@ void orc_chain_block(orc_chain *c, const uint8_t *iq, int16_t *pcm,
         c->ib[j] = c->iq[2 * j];
         c->qb[j] = c->iq[2 * j + 1];
     }
+    if (c->cos_t) {                      /* the tuning mixer: x * e^{-j theta(n)}; not in the reference */
+        for (int j = 0; j < npairs; j++) {
+            const uint32_t ph = (uint32_t)(c->pairs_done + (uint64_t)j) * c->inc;
+            const float cs = c->cos_t[ph >> 16], sn = c->sin_t[ph >> 16];
+            const float i = c->ib[j], q = c->qb[j];
+            const float ic = i * cs, qs = q * sn, qc = q * cs, is = i * sn;
+            c->ib[j] = ic + qs;
+            c->qb[j] = qc - is;
+        }
+    }
+    c->pairs_done += (uint64_t)npairs;
     orc_resample(c->i_ds, c->st_i, T - 1, c->ib, npairs, c->rf_coeff, T, 1, m->rf_decim);  /* :65 */
     orc_resample(c->q_ds, c->st_q, T - 1, c->qb, npairs, c->rf_coeff, T, 1, m->rf_decim);  /* :66 */
     orc_fmdemod(c->demod, &c->prev_i, &c->prev_q, c->i_ds, c->q_ds, nif);                 /* :69 */

@@ -89,6 +89,21 @@ orc_chain *orc_chain_create(int mode, int taps);
 void orc_chain_destroy(orc_chain *c);
 const orc_mode *orc_chain_mode(const orc_chain *c);
 
+/* Tune the chain to the station offset_hz above the capture's centre, as
+ * fmrx_set_tuning (include/fmrx.h) defines it.  Between the de-interleave and
+ * the RF filter, pair n of the stream (counted from create) becomes
+ * x * e^{-j theta(n)}:
+ *   inc = (uint32) llrint(offset_hz * 2^32 / rf_fs),  ph = (uint32)(n * inc),
+ *   k = ph >> 16,  cos_t[k] = (float)cos(a), sin_t[k] = (float)sin(a),
+ *   a = 2 pi k / 65536 in double,
+ *   I' = i*c + q*s,  Q' = q*c - i*s  (one IEEE float operation each).
+ * The zero filter history in front of the first pair is not rotated.  The
+ * reference has no mixer: a chain is untuned unless this is called, and the
+ * pins against the reference cover the untuned chain.  A tuned chain runs the
+ * mixer even at offset 0, where it is the identity.  Returns nonzero, and
+ * changes nothing, when !(|offset_hz| < rf_fs/2) or a block has already run. */
+int orc_chain_set_tuning(orc_chain *c, double offset_hz);
+
 /* Optional per-block stage taps; any pointer may be NULL. Sizes per block:
  * i_ds,q_ds,demod,chan,pilot,trig,nco,mixer: if_per_block floats;
  * mono,mono_shift,stereo,left,right: audio_per_block floats. */
@@ -105,7 +120,9 @@ void orc_chain_run(orc_chain *c, const uint8_t *iq, size_t n_blocks,
                    int16_t *pcm, const orc_stage_dump *dump);
 
 /* Carried state, flattened (what a time-shard hands to the next):
- * layout and length are reported by orc_chain_state_len(). */
+ * layout and length are reported by orc_chain_state_len().  It does not
+ * carry the tuning mixer's pair counter, so a tuned chain runs from its
+ * stream's start. */
 size_t orc_chain_state_len(const orc_chain *c);
 void orc_chain_get_state(const orc_chain *c, float *out);
 void orc_chain_set_state(orc_chain *c, const float *in);

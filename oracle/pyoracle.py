@@ -194,6 +194,8 @@ class Port(_OpsMixin):
         L.orc_chain_destroy.argtypes = [C.c_void_p]
         L.orc_chain_mode.restype = C.POINTER(_Mode)
         L.orc_chain_mode.argtypes = [C.c_void_p]
+        L.orc_chain_set_tuning.argtypes = [C.c_void_p, C.c_double]
+        L.orc_chain_set_tuning.restype = C.c_int
         L.orc_chain_run.argtypes = [C.c_void_p, _u8p, C.c_size_t, _i16p, C.POINTER(_Dump)]
         L.orc_chain_run.restype = None
         L.orc_chain_state_len.restype = C.c_size_t
@@ -239,18 +241,21 @@ class Port(_OpsMixin):
         f(out.ctypes.data_as(_i16p), _fp(left), _fp(right), len(left))
         return out
 
-    def chain(self, mode, taps=51):
-        return PortChain(self, mode, taps)
+    def chain(self, mode, taps=51, tune_hz=None):
+        return PortChain(self, mode, taps, tune_hz)
 
 
 class PortChain:
-    """Block loop of the restatement, with carried state."""
+    """Block loop of the restatement, with carried state; tuned to the station ``tune_hz`` above the capture's
+    centre when that is given (orc_chain_set_tuning)."""
 
-    def __init__(self, port: Port, mode: int, taps: int):
+    def __init__(self, port: Port, mode: int, taps: int, tune_hz: float | None = None):
         self.port = port
         self.h = port.lib.orc_chain_create(mode, taps)
         if not self.h:
             raise ValueError(f"bad mode/taps {mode}/{taps}")
+        if tune_hz is not None and port.lib.orc_chain_set_tuning(self.h, float(tune_hz)) != 0:
+            raise ValueError(f"tune_hz {tune_hz} outside +-rf_fs/2")
         self.info = ModeInfo(port.lib.orc_chain_mode(self.h).contents)
 
     def __del__(self):

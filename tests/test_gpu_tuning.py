@@ -9,7 +9,6 @@ import pytest
 
 from conftest import assert_bits_equal
 import pyoracle
-from tuned_oracle import TunedChain
 
 pytestmark = pytest.mark.gpu
 
@@ -38,7 +37,7 @@ def test_tuned_stages_bit_identical_to_the_tuned_oracle(fm, port, synth, mode, t
     with fm.Pipeline(mode, taps, 3, device=0, chunk_blocks=chunk, keep_stages=True, tune_hz=offs) as p:
         pcm, st = p.process_stages(np.stack([iq] * 3), ALL_STAGES)
     for c, off in enumerate(offs):
-        ref, rst = TunedChain(mode, taps, off).run(iq, stages=ALL_STAGES)
+        ref, rst = port.chain(mode, taps, tune_hz=off).run(iq, stages=ALL_STAGES)
         for s in ALL_STAGES:
             assert_bits_equal(st[s][c], rst[s], f"m{mode} t{taps} capture {c} ({off} Hz) {s}")
         assert np.array_equal(pcm[c], ref), (mode, taps, c)
@@ -51,7 +50,7 @@ def test_split_calls_and_state_blobs_continue_one_pass(fm, port, synth, mode):
     nb = 23
     iq = _stream(synth, info, nb, [(off, 8, "stereo", 100), (150e3, 9, "stereo", 100)])
     bs = info.block_size
-    ref, _ = TunedChain(mode, 51, off).run(iq)
+    ref, _ = port.chain(mode, 51, tune_hz=off).run(iq)
     with fm.Pipeline(mode, 51, 1, device=0, chunk_blocks=4, tune_hz=off) as p:
         parts = [p.process(iq[a * bs:b * bs]) for a, b in ((0, 1), (1, 8), (8, 19), (19, nb))]
     assert np.array_equal(np.concatenate(parts, axis=1)[0], ref)
@@ -83,7 +82,7 @@ def test_five_stations_from_one_stream_host_and_device(fm, port, synth):
         torch.cuda.synchronize()
         dev = d_pcm.cpu().numpy()
     for c, off in enumerate(offs):
-        ref, _ = TunedChain(0, 51, off).run(iq)
+        ref, _ = port.chain(0, 51, tune_hz=off).run(iq)
         with fm.Pipeline(0, 51, 1, device=0, tune_hz=off) as one:
             alone = one.process(iq)[0]
         assert np.array_equal(host[c], ref), c
@@ -120,7 +119,7 @@ def test_three_stations_across_the_counter_saturation(fm, port, synth):
     del d_iq, d_pcm
 
     def check(c):
-        ref, _ = TunedChain(0, 51, offs[c]).run(iq)
+        ref, _ = port.chain(0, 51, tune_hz=offs[c]).run(iq)
         return int(np.count_nonzero(pcm[c] != ref))
     with ThreadPoolExecutor(3) as ex:
         assert list(ex.map(check, range(3))) == [0, 0, 0]
@@ -159,7 +158,7 @@ def test_cli_tune_matches_the_library(fm, port, synth):
                        capture_output=True, timeout=300)
     assert r.returncode == 1 and b"End of input stream reached!" in r.stderr
     assert np.array_equal(np.frombuffer(r.stdout, np.int16), lib)
-    assert np.array_equal(lib, TunedChain(0, 51, -300e3).run(iq)[0])
+    assert np.array_equal(lib, port.chain(0, 51, tune_hz=-300e3).run(iq)[0])
     for bad in ("1200000", "-1200000", "12x", "0.5"):
         r = subprocess.run([str(CLI), "0", "s", "--tune", bad], input=b"", capture_output=True, timeout=60)
         assert r.returncode == 1 and b"Usage" in r.stderr, bad

@@ -1,4 +1,4 @@
-"""Tuning to stations off the capture's centre, on the CPU: the tuned oracle (tests/tuned_chain.c), the
+"""Tuning to stations off the capture's centre, on the CPU: the oracle's tuning mixer (orc_chain_set_tuning), the
 multi-station synthesiser, and what a tuned chain decodes out of a stream that holds three stations."""
 import ctypes
 
@@ -7,7 +7,6 @@ import pytest
 
 from conftest import assert_bits_equal
 import pyoracle
-from tuned_oracle import TunedChain
 
 ALL_STAGES = pyoracle.STAGES
 
@@ -21,12 +20,12 @@ def _three_stations(mode):
 @pytest.mark.parametrize("mode,n_blocks", [(0, 6), (1, 6), (2, 2), (3, 2)])
 def test_tuned_oracle_at_offset_zero_equals_untuned(port, synth, mode, n_blocks):
     """cos_t[0] = 1, sin_t[0] = 0 and the pairs are never -0, so the mixer at offset 0 is the identity: checked on
-    every stage, not assumed.  This also pins the tuned restatement to the oracle's own block loop."""
+    every stage, not assumed.  A chain tuned to offset 0 runs the mixer, so this pins the mixer itself."""
     info = port.mode(mode, 51)
     iq = synth.synth_iq_exact_multi(n_blocks * info.block_size // 2, float(info.rf_fs),
                                     [(-250e3, 3, "stereo", 120), (0.0, 5, "stereo", 120)])
     pcm0, st0 = port.chain(mode, 51).run(iq, stages=ALL_STAGES)
-    pcm1, st1 = TunedChain(mode, 51, 0.0).run(iq, stages=ALL_STAGES)
+    pcm1, st1 = port.chain(mode, 51, tune_hz=0.0).run(iq, stages=ALL_STAGES)
     for s in ALL_STAGES:
         assert_bits_equal(st1[s], st0[s], f"mode {mode} {s}")
     assert np.array_equal(pcm1, pcm0)
@@ -35,11 +34,11 @@ def test_tuned_oracle_at_offset_zero_equals_untuned(port, synth, mode, n_blocks)
 def test_tuned_oracle_rejects_offsets_beyond_half_the_rf_rate(port):
     for mode in range(4):
         half = port.mode(mode, 51).rf_fs / 2
-        TunedChain(mode, 51, half - 1.0)
-        TunedChain(mode, 51, -(half - 1.0))
+        port.chain(mode, 51, tune_hz=half - 1.0)
+        port.chain(mode, 51, tune_hz=-(half - 1.0))
         for bad in (half, -half, 1e9, float("nan")):
             with pytest.raises(ValueError):
-                TunedChain(mode, 51, bad)
+                port.chain(mode, 51, tune_hz=bad)
 
 
 def test_multi_synth_with_one_centred_station_is_synth_iq_exact(synth):
@@ -83,7 +82,7 @@ def test_tuned_chain_decodes_each_of_three_stations(port, synth, mode):
     tones = [t for _, k, _, _ in stations for t in synth.station_tones(k)]
     for off, k, kind, gain in stations:
         f_l, f_r = synth.station_tones(k)
-        pcm, _ = TunedChain(mode, 51, off).run(iq)
+        pcm, _ = port.chain(mode, 51, tune_hz=off).run(iq)
         alone = synth.synth_iq_exact_multi(n_pairs, float(info.rf_fs), [(0.0, k, kind, gain)])
         ref = _tone_levels_db(port.chain(mode, 51).run(alone)[0], tones)
         got = _tone_levels_db(pcm, tones)
@@ -95,7 +94,7 @@ def test_tuned_chain_decodes_each_of_three_stations(port, synth, mode):
             assert lv[want] - max(others) >= 30.0, (mode, off, ch, lv[want], max(others))
         if off:
             # the sign convention: the mirror offset does not hold this station
-            mirror = _tone_levels_db(TunedChain(mode, 51, -off).run(iq)[0], tones)
+            mirror = _tone_levels_db(port.chain(mode, 51, tune_hz=-off).run(iq)[0], tones)
             for ch, want in ((0, f_r), (1, f_l)):
                 assert mirror[ch][1][want] < ref[ch][1][want] - 30.0, (mode, off, ch)
 

@@ -26,7 +26,6 @@ from pathlib import Path
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT))
 sys.path.insert(0, str(ROOT / "oracle"))
-sys.path.insert(0, str(ROOT / "tests"))
 
 MODE, TAPS, SECONDS = 0, 51, 60.0
 OFFSETS = [-875e3 + 250e3 * k for k in range(8)]
@@ -133,12 +132,13 @@ def main():
     del host_shared, host_sep, host_pcm
 
     # whole-run parity of every tuned station (S = 8) against the live oracle
-    from tuned_oracle import TunedChain
+    import pyoracle
+    port = pyoracle.Port()
     iq = shared.cpu().numpy()
     t0 = time.perf_counter()
 
     def check(c):
-        ref, _ = TunedChain(MODE, TAPS, OFFSETS[c]).run(iq)
+        ref, _ = port.chain(MODE, TAPS, tune_hz=OFFSETS[c]).run(iq)
         return int(np.count_nonzero(tuned8[c] != ref))
     with ThreadPoolExecutor(8) as ex:
         diff = list(ex.map(check, range(8)))
