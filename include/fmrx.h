@@ -175,6 +175,77 @@ int fmrx_process_device(fmrx_pipeline *p, const uint8_t *iq_dev, size_t iq_strid
  * a tuned checkpoint: fmrx_create, fmrx_set_tuning, fmrx_set_state. */
 int fmrx_set_tuning(fmrx_pipeline *p, int capture, double offset_hz);
 
+/* RDS (IEC 62106) of `capture`, decoded on the device beside the PLL from its
+ * demodulated signal d[n] (FMRX_STAGE_DEMOD, fs = bp_fs), so tuned captures work
+ * unchanged.  n counts from the stream's first sample (0 after create or reset)
+ * and continues across calls, chunks and state blobs.  Per mode (fs 240 000,
+ * 288 000, 240 000, 256 000):
+ *   mix     z[n] = d[n] e^{-2 pi i k/P}, k = (q n) mod P, q/P = 57000/fs in
+ *           lowest terms (P = 80, 96, 80, 256); the table is cos/sin in double
+ *           rounded to float;
+ *   FIR     u[m] = sum_t h[t] z[mD - t], D = 12 at 288 kHz else 10, so
+ *           fs2 = fs/D = 24 000 or 25 600; only n = mD from the stream's start;
+ *           h = Blackman-windowed sinc, cutoff 4 kHz, 2 floor(63 fs/240000 + 1/2)
+ *           + 1 taps (127, 153, 127, 135), unit DC gain, double rounded to float;
+ *   biphase y[m] = sum_{i<L} u[m-i] - sum_{L<=i<2L} u[m-i], L = round(fs2/2375);
+ *   timing  windows of M = fs2/10 samples from m = 0; once window w is complete,
+ *           c_w = sum_{m in w} |y[m]|^2 e^{-2 pi i m 1187.5/fs2} (fixed order),
+ *           tau_w = -arg(c_w)/2 pi, unwrapped against tau_{w-1} into (-1/2, 1/2];
+ *           tau(t) is linear between window centres wM + M/2 (constant beyond
+ *           the first and the latest); sps = fs2/1187.5;
+ *   bits    bit j at t_j = (j + tau(t'))sps, t' = (j + tau(t''))sps,
+ *           t'' = t_{j-1} + sps (j sps for the first bit); s_j = y linearly
+ *           interpolated at t_j; b_j = 1 iff Re(s_j conj(s_{j-1})) < 0.  A bit is
+ *           decided once the window after the one holding t_j is complete, so
+ *           groups lag the input by about two windows (0.2 s);
+ *   blocks  26 bits, g(x) = x^10+x^8+x^7+x^5+x^4+x^3+1, offset words A B C C' D.
+ *           Search: sync when a block matching offset X ends 26 bits after one
+ *           matching the offset before X in A->B->(C|C')->D->A.  In sync, every 26
+ *           bits is the next block, valid iff its syndrome is the expected
+ *           offset's (C' accepted for C); 8 invalid blocks in a row lose sync.
+ *           No error correction: an invalid block is reported, never guessed;
+ *   groups  four blocks from an A position, emitted at their D position if one
+ *           of them is valid.  if_index = round(t D) of the group's first bit.
+ * Configuration, not state: only at the start of the capture's stream (after
+ * create or reset), else FMRX_ERR_STATE; it survives fmrx_reset, which clears
+ * the decoder and its ring.  Not in the state blob: fmrx_set_state on a capture
+ * with RDS on restarts its decoder (search, empty ring) at the restored position.
+ * With RDS off for every capture nothing is launched.  enable 0 or 1, else
+ * FMRX_ERR_ARG.  The PCM and every stage are the same with RDS on or off. */
+int fmrx_set_rds(fmrx_pipeline *p, int capture, int enable);
+
+typedef struct {
+    uint64_t if_index;     /* IF sample (FMRX_STAGE_DEMOD index from the stream's start) of the first bit */
+    uint16_t block[4];     /* information words A, B, C (or C'), D */
+    uint8_t valid;         /* bit i: block[i] had its offset's syndrome */
+    uint8_t c_prime;       /* block 2 was received with offset C' */
+    uint16_t reserved;
+} fmrx_rds_group;
+
+/* Drain up to max groups of `capture` in stream order into out; *n_out = groups
+ * written.  Each capture keeps the last 8192 groups (about 12 minutes); older
+ * ones are dropped and counted in *n_lost (since create, reset or restart; may
+ * be NULL).  Waits for the pipeline's work in flight. */
+int fmrx_read_rds(fmrx_pipeline *p, int capture, fmrx_rds_group *out, size_t max, size_t *n_out,
+                  uint64_t *n_lost);
+
+typedef struct {
+    int pi_valid;          /* a PI value has appeared in two valid A blocks */
+    uint16_t pi;           /* the first such value */
+    int pty, tp;           /* from the last valid B block; -1 before any */
+    char ps[9];            /* programme service name; segments not received are spaces */
+    uint8_t ps_seen;       /* bit k: PS segment k (characters 2k, 2k+1) received */
+    char rt[65];           /* radio text, cut at the first 0x0D; segments not received are spaces */
+    uint16_t rt_seen;      /* bit k: RT segment k received (since the last A/B flag change) */
+    uint64_t groups, blocks_valid, blocks_total;
+} fmrx_rds_info;
+
+/* Host code, deterministic; no device needed.  PI: see pi_valid.  PS: from 0A/0B
+ * groups with B and D valid, segment B & 3.  RT: 2A groups with B, C and D valid
+ * (4 characters at segment B & 15) and 2B groups with B and D valid (2
+ * characters); a change of the A/B flag (B bit 4) clears it. */
+int fmrx_rds_summarise(const fmrx_rds_group *g, size_t n, fmrx_rds_info *out);
+
 /* Stage intermediates of the LAST fmrx_process* call (keep_stages=1 only). */
 typedef enum {
     FMRX_STAGE_DEMOD = 0,  /* IF rate */
@@ -259,7 +330,8 @@ int fmrx_long_last_ms(const fmrx_long_capture *h, float *ms);
 int fmrx_long_pll_state(fmrx_long_capture *h, float out[6]);
 
 /* ---------------------------------------------------------------------- */
-/* The reference's RDS sketch, src/project.cpp:200-271 (rds_thread: compiled */
+/* The reference's RDS sketch (not a decoder: fmrx_set_rds decodes RDS),    */
+/* src/project.cpp:200-271 (rds_thread: compiled                            */
 /* into the reference, never started): 54-60 kHz channel band-pass, squarer, */
 /* 113.5-114.5 kHz band-pass, PLL(114000, bp_fs, 0.5, 0, 0.01), the channel   */
 /* delayed by channel_delay samples, mixer.  One call = one block of          */

@@ -39,7 +39,7 @@ ABI_SYMBOLS = (
     "fmrx_process", "fmrx_process_device", "fmrx_read_stage",
     "fmrx_state_size", "fmrx_get_state", "fmrx_set_state", "fmrx_get_pll_state",
     "fmrx_host_alloc", "fmrx_host_free", "fmrx_kernel_launches", "fmrx_set_timing",
-    "fmrx_last_timing", "fmrx_set_tuning",
+    "fmrx_last_timing", "fmrx_set_tuning", "fmrx_set_rds", "fmrx_read_rds", "fmrx_rds_summarise",
     "fmrx_long_create", "fmrx_long_destroy", "fmrx_long_shard", "fmrx_long_process", "fmrx_long_process_device",
     "fmrx_long_last_ms", "fmrx_long_pll_state",
     "fmrx_rds_create", "fmrx_rds_destroy", "fmrx_rds_reset", "fmrx_rds_process", "fmrx_rds_pll_state",
@@ -68,6 +68,25 @@ class ConfigStruct(C.Structure):
 
 class StationStruct(C.Structure):
     _fields_ = [("offset_hz", C.c_double), ("level_db", C.c_double), ("snr_db", C.c_double)]
+
+
+class RdsGroupStruct(C.Structure):
+    _fields_ = [("if_index", C.c_uint64), ("block", C.c_uint16 * 4), ("valid", C.c_uint8), ("c_prime", C.c_uint8),
+                ("reserved", C.c_uint16)]
+
+
+class RdsInfoStruct(C.Structure):
+    _fields_ = [("pi_valid", C.c_int), ("pi", C.c_uint16), ("pty", C.c_int), ("tp", C.c_int), ("ps", C.c_char * 9),
+                ("ps_seen", C.c_uint8), ("rt", C.c_char * 65), ("rt_seen", C.c_uint16), ("groups", C.c_uint64),
+                ("blocks_valid", C.c_uint64), ("blocks_total", C.c_uint64)]
+
+
+# fmrx_rds_group as numpy sees it (Pipeline.rds_groups)
+RDS_GROUP_DTYPE = np.dtype([("if_index", "<u8"), ("block", "<u2", (4,)), ("valid", "u1"), ("c_prime", "u1"),
+                            ("reserved", "<u2")], align=True)
+assert RDS_GROUP_DTYPE.itemsize == C.sizeof(RdsGroupStruct)
+
+RdsInfo = namedtuple("RdsInfo", "pi pty tp ps ps_seen rt rt_seen groups blocks_valid blocks_total")
 
 
 class ModeInfo:
@@ -137,6 +156,10 @@ def load() -> C.CDLL:
     L.fmrx_set_timing.argtypes = [C.c_void_p, C.c_int]
     L.fmrx_last_timing.argtypes = [C.c_void_p, _f32p]
     L.fmrx_set_tuning.argtypes = [C.c_void_p, C.c_int, C.c_double]
+    L.fmrx_set_rds.argtypes = [C.c_void_p, C.c_int, C.c_int]
+    L.fmrx_read_rds.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t),
+                                C.POINTER(C.c_uint64)]
+    L.fmrx_rds_summarise.argtypes = [C.c_void_p, C.c_size_t, C.POINTER(RdsInfoStruct)]
     L.fmrx_scan_create.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.c_double, C.c_int]
     L.fmrx_scan_destroy.argtypes = [C.c_void_p]
     L.fmrx_scan_reset.argtypes = [C.c_void_p]
@@ -255,10 +278,11 @@ def pcm_pack(left, right) -> np.ndarray:
 
 class Pipeline:
     """The block loop of src/project.cpp for ``n_captures`` captures at once.  ``tune_hz``: the station's offset from
-    the capture's centre frequency (fmrx_set_tuning), one for all captures or one per capture; None: untuned."""
+    the capture's centre frequency (fmrx_set_tuning), one for all captures or one per capture; None: untuned.
+    ``rds``: decode RDS (fmrx_set_rds) on every capture (True), none (False) or per capture (a list of bools)."""
 
     def __init__(self, mode: int = 0, taps: int = 51, n_captures: int = 1, device: int = -1,
-                 chunk_blocks: int = 0, keep_stages: bool = False, tune_hz=None):
+                 chunk_blocks: int = 0, keep_stages: bool = False, tune_hz=None, rds=False):
         self._L = load()
         cfg = ConfigStruct(mode, taps, n_captures, device, chunk_blocks, int(keep_stages))
         h = C.c_void_p()
@@ -276,6 +300,29 @@ class Pipeline:
                 raise ValueError(f"tune_hz: {len(hz)} offsets for {n_captures} captures")
             for c, f in enumerate(hz):
                 self.set_tuning(c, f)
+        on = list(rds) if np.ndim(rds) else [bool(rds)] * n_captures
+        if len(on) != n_captures:
+            self.close()
+            raise ValueError(f"rds: {len(on)} flags for {n_captures} captures")
+        for c, f in enumerate(on):
+            if f:
+                self.set_rds(c, True)
+        self.rds_lost = [0] * n_captures
+
+    def set_rds(self, capture: int, on: bool):
+        """RDS decoding of ``capture`` on or off; only at the start of its stream (after creation or reset)."""
+        _check(self._L.fmrx_set_rds(self._h, capture, int(bool(on))), "fmrx_set_rds")
+
+    def rds_groups(self, capture: int = 0, max_groups: int = 1 << 20) -> np.ndarray:
+        """Drain the RDS groups decoded so far for ``capture``: a structured array of RDS_GROUP_DTYPE in stream order.
+        ``rds_lost[capture]`` becomes the count of groups dropped because nobody drained them in time."""
+        out = np.zeros(max_groups, RDS_GROUP_DTYPE)
+        n = C.c_size_t(0)
+        lost = C.c_uint64(0)
+        _check(self._L.fmrx_read_rds(self._h, capture, out.ctypes.data, max_groups, C.byref(n), C.byref(lost)),
+               "fmrx_read_rds")
+        self.rds_lost[capture] = int(lost.value)
+        return out[:n.value].copy()
 
     def set_tuning(self, capture: int, hz: float):
         """Tune ``capture`` to the station ``hz`` above its stream's centre (negative: below); only at the start of
@@ -474,6 +521,17 @@ class RdsFront:
         st = np.zeros(6, np.float32)
         _check(self._L.fmrx_rds_pll_state(self._h, _fp(st)), "fmrx_rds_pll_state")
         return st
+
+
+def rds_summarise(groups) -> RdsInfo:
+    """PI, PTY, TP, PS and RT of a run of groups (fmrx_rds_summarise, host code).  ``pi`` is None until a value has
+    appeared in two valid A blocks; ``pty``/``tp`` -1 before a valid B block."""
+    g = np.ascontiguousarray(groups, RDS_GROUP_DTYPE)
+    s = RdsInfoStruct()
+    _check(load().fmrx_rds_summarise(g.ctypes.data if len(g) else None, len(g), C.byref(s)), "fmrx_rds_summarise")
+    raw_ps = bytes(C.string_at(C.addressof(s) + RdsInfoStruct.ps.offset, 8))
+    return RdsInfo(int(s.pi) if s.pi_valid else None, int(s.pty), int(s.tp), raw_ps.decode("latin-1"), int(s.ps_seen),
+                   s.rt.decode("latin-1"), int(s.rt_seen), int(s.groups), int(s.blocks_valid), int(s.blocks_total))
 
 
 def estimatePSD(samples, freq_bins: int, Fs: float):

@@ -17,6 +17,7 @@
 #include <cstdio>
 #include <cstring>
 #include <memory>
+#include <numeric>
 #include <new>
 #include <type_traits>
 #include <vector>
@@ -486,6 +487,20 @@ struct fmrx_pipeline {
     dptr<RfTune> d_tune;                  // [C]
     dptr<float2> d_tune_cs;               // the mixer table (65536 cos, sin), allocated when a capture is first tuned
     bool tuned = false;                   // some capture has a nonzero phase step: K1 runs its tuned variant
+    // RDS (fmrx_set_rds): configuration like tuning.  The decoder's buffers are allocated when a capture first turns
+    // it on; its kernels run on the front stream after front_done, so every buffer has one user at a time.
+    std::vector<int> rds_on;              // [C]
+    std::vector<int> rds_caps;            // the captures with RDS on, mirrored in d_rds_caps
+    dptr<int> d_rds_caps;
+    RdsParams rds_prm{};
+    dptr<float> d_rds_taps, d_rds_dtail;  // dtail: [C][rds_dtail_len] demod samples before the chunk
+    dptr<float2> d_rds_mix, d_rds_y;      // y: [C][rds_y_len]
+    dptr<double2> d_rds_phase;
+    dptr<RdsDecState> d_rds_state;        // [C]
+    dptr<fmrx_rds_group> d_rds_ring;      // [C][kRdsRing]
+    int rds_dtail_len = 0, rds_ytail_len = 0;
+    size_t rds_y_len = 0;
+    std::vector<uint64_t> rds_read, rds_lost;   // per capture: groups drained / dropped since (re)start
     size_t mem_pitch = 0;       // cudaDeviceProp::memPitch: the largest pitch cudaMemcpy2D takes
     uint64_t launches = 0;
 
@@ -508,6 +523,29 @@ struct fmrx_pipeline {
 
 namespace {
 
+// The RDS decoder of `capture` from its stream position blocks_done[capture]: search, no bits, zero history, empty
+// ring.  The device must be idle.
+int rds_restart(fmrx_pipeline *p, int capture)
+{
+    const RdsParams &P = p->rds_prm;
+    const long long n = p->blocks_done[capture] * p->mi.if_per_block;
+    const long long m = (n + P.D - 1) / P.D;                 // the first kept sample from here
+    RdsDecState st;
+    std::memset(&st, 0, sizeof(st));
+    st.n_offset = (p->blocks_done[capture] - p->blocks_run) * p->mi.if_per_block;
+    st.w_first = st.w_next = m / P.M;
+    st.j = static_cast<long long>(std::ceil(static_cast<double>(m) / (P.fs2 / 1187.5)));
+    for (auto &h : st.last_hit)
+        h = kRdsNoHit;
+    CU(cudaMemcpy(p->d_rds_state.get() + capture, &st, sizeof(st), cudaMemcpyHostToDevice));
+    CU(cudaMemset(p->d_rds_dtail.get() + static_cast<size_t>(capture) * p->rds_dtail_len, 0,
+                  p->rds_dtail_len * sizeof(float)));
+    CU(cudaMemset(p->d_rds_y.get() + static_cast<size_t>(capture) * p->rds_y_len, 0, p->rds_y_len * sizeof(float2)));
+    p->rds_read[capture] = 0;
+    p->rds_lost[capture] = 0;
+    return FMRX_OK;
+}
+
 int reset_state(fmrx_pipeline *p)
 {
     const size_t C = p->C;
@@ -524,6 +562,12 @@ int reset_state(fmrx_pipeline *p)
     for (auto &t : p->tune)
         t.pair_offset = 0;
     CU(cudaMemcpy(p->d_tune.get(), p->tune.data(), C * sizeof(RfTune), cudaMemcpyHostToDevice));
+    for (size_t c = 0; c < C; c++)
+        if (p->rds_on[c]) {
+            const int rc = rds_restart(p, static_cast<int>(c));
+            if (rc != FMRX_OK)
+                return rc;
+        }
     return FMRX_OK;
 }
 
@@ -728,6 +772,42 @@ int run(fmrx_pipeline *p, const uint8_t *iq, size_t iq_stride, size_t n_blocks, 
         CU(copy2d(p->d_tail_demod.get(), fH, S.demod.get() + n_if, if_pitch, fH, C, p->s_front.get()));
         CU(copy2d(p->d_tail_chan.get(), fH, S.chan.get() + n_if, if_pitch, fH, C, p->s_front.get()));
         CU(cudaEventRecord(S.front_done.get(), p->s_front.get()));
+        if (!p->rds_caps.empty() && !feedforward_only) {
+            // RDS beside K3: on the front stream after front_done, so that K3 does not wait for it
+            const long long if_run = p->blocks_run * mi.if_per_block;
+            RdsBasebandArgs b{};
+            b.prm = p->rds_prm;
+            b.caps = p->d_rds_caps.get();
+            b.state = p->d_rds_state.get();
+            b.demod = S.demod.get();
+            b.if_stride = p->if_stride;
+            b.if_off = H;
+            b.n_if = n_if;
+            b.if_run = if_run;
+            b.dtail = p->d_rds_dtail.get();
+            b.dtail_len = p->rds_dtail_len;
+            b.taps = p->d_rds_taps.get();
+            b.mix = p->d_rds_mix.get();
+            b.ybuf = p->d_rds_y.get();
+            b.ybuf_len = p->rds_y_len;
+            b.ytail_len = p->rds_ytail_len;
+            RdsBitsArgs r{};
+            r.prm = p->rds_prm;
+            r.caps = p->d_rds_caps.get();
+            r.state = p->d_rds_state.get();
+            r.n_if = n_if;
+            r.if_run = if_run;
+            r.ybuf = p->d_rds_y.get();
+            r.ybuf_len = p->rds_y_len;
+            r.ytail_len = p->rds_ytail_len;
+            r.bitphase = p->d_rds_phase.get();
+            r.ring = p->d_rds_ring.get();
+            CU(launch_rds(b, r, static_cast<int>(p->rds_caps.size()), p->s_front.get()));
+            p->launches += 2;
+            const size_t dt = static_cast<size_t>(p->rds_dtail_len) * sizeof(float);
+            CU(copy2d(p->d_rds_dtail.get(), dt, S.demod.get() + H + n_if - p->rds_dtail_len, if_pitch, dt, C,
+                      p->s_front.get()));
+        }
         if (feedforward_only) {
             CU(cudaEventRecord(S.free_ev.get(), p->s_front.get()));
             S.free_pending = true;
@@ -939,6 +1019,9 @@ extern "C" int fmrx_create(fmrx_pipeline **out, const fmrx_config *cfg)
     CU(dalloc(p->d_pll_state, C * 8));
     CU(dalloc(p->d_tune, C));
     p->tune.assign(C, RfTune{ 0, 0 });
+    p->rds_on.assign(C, 0);
+    p->rds_read.assign(C, 0);
+    p->rds_lost.assign(C, 0);
     for (auto &s : p->sets) {
         CU(dalloc(s.demod, C * p->if_stride));
         CU(dalloc(s.chan, C * p->if_stride));
@@ -1114,6 +1197,92 @@ extern "C" int fmrx_set_state(fmrx_pipeline *p, int capture, const void *blob, s
         p->tune[capture].pair_offset = (h.blocks_done - p->blocks_run) * (p->mi.block_size / 2);
         CU(cudaMemcpy(p->d_tune.get() + capture, &p->tune[capture], sizeof(RfTune), cudaMemcpyHostToDevice));
     }
+    if (p->rds_on[capture])
+        return rds_restart(p, capture);
+    return FMRX_OK;
+}
+
+extern "C" int fmrx_set_rds(fmrx_pipeline *p, int capture, int enable)
+{
+    if (!p || capture < 0 || capture >= p->C || (enable != 0 && enable != 1))
+        return FMRX_ERR_ARG;
+    if (p->blocks_done[capture] != 0)
+        return FMRX_ERR_STATE;
+    CU(cudaSetDevice(p->device));
+    CU(cudaDeviceSynchronize());   // the RDS kernels of calls still in flight read d_rds_caps
+    const size_t C = p->C;
+    if (enable && !p->d_rds_state) {
+        const RdsParams P = rds_params(p->mi.bp_fs);
+        std::vector<float> taps(P.taps);
+        std::vector<float2> mix(P.P);
+        std::vector<double2> ph(P.Q);
+        rds_tables(P, taps.data(), mix.data(), ph.data());
+        // demod history: the FIR input of the first u a tile needs; y history: two windows and a bit of slack
+        // (the bits still to be decided lie at most two windows back)
+        const int dtail = ((2 * P.L + 1) * P.D + P.taps + 31) / 32 * 32;
+        const int ytail = 2 * P.M + 64;
+        const size_t y_len = ytail + static_cast<size_t>(p->chunk_if) / P.D + 2;
+        if (dtail > p->mi.if_per_block)
+            return FMRX_ERR_ARG;
+        CU(dalloc(p->d_rds_taps, taps.size()));
+        CU(dalloc(p->d_rds_mix, mix.size()));
+        CU(dalloc(p->d_rds_phase, ph.size()));
+        CU(dalloc(p->d_rds_dtail, C * dtail));
+        CU(dalloc(p->d_rds_y, C * y_len));
+        CU(dalloc(p->d_rds_ring, C * kRdsRing));
+        CU(dalloc(p->d_rds_caps, C));
+        CU(cudaMemcpy(p->d_rds_taps.get(), taps.data(), taps.size() * sizeof(float), cudaMemcpyHostToDevice));
+        CU(cudaMemcpy(p->d_rds_mix.get(), mix.data(), mix.size() * sizeof(float2), cudaMemcpyHostToDevice));
+        CU(cudaMemcpy(p->d_rds_phase.get(), ph.data(), ph.size() * sizeof(double2), cudaMemcpyHostToDevice));
+        CU(dalloc(p->d_rds_state, C));     // last: it marks the decoder's buffers as present
+        p->rds_prm = P;
+        p->rds_dtail_len = dtail;
+        p->rds_ytail_len = ytail;
+        p->rds_y_len = y_len;
+    }
+    p->rds_on[capture] = enable;
+    p->rds_caps.clear();
+    for (size_t c = 0; c < C; c++)
+        if (p->rds_on[c])
+            p->rds_caps.push_back(static_cast<int>(c));
+    if (!p->rds_caps.empty())
+        CU(cudaMemcpy(p->d_rds_caps.get(), p->rds_caps.data(), p->rds_caps.size() * sizeof(int),
+                      cudaMemcpyHostToDevice));
+    return enable ? rds_restart(p, capture) : FMRX_OK;
+}
+
+extern "C" int fmrx_read_rds(fmrx_pipeline *p, int capture, fmrx_rds_group *out, size_t max, size_t *n_out,
+                             uint64_t *n_lost)
+{
+    if (!p || capture < 0 || capture >= p->C || !out || !n_out)
+        return FMRX_ERR_ARG;
+    *n_out = 0;
+    if (n_lost)
+        *n_lost = p->rds_lost[capture];
+    if (!p->rds_on[capture])
+        return FMRX_OK;
+    CU(cudaSetDevice(p->device));
+    CU(cudaStreamSynchronize(p->s_front.get()));
+    uint64_t written = 0;
+    CU(cudaMemcpy(&written, &p->d_rds_state.get()[capture].written, sizeof(written), cudaMemcpyDeviceToHost));
+    uint64_t &rd = p->rds_read[capture];
+    if (written - rd > static_cast<uint64_t>(kRdsRing)) {
+        p->rds_lost[capture] += written - rd - kRdsRing;
+        rd = written - kRdsRing;
+    }
+    const fmrx_rds_group *ring = p->d_rds_ring.get() + static_cast<size_t>(capture) * kRdsRing;
+    size_t k = static_cast<size_t>(std::min<uint64_t>(written - rd, max));
+    size_t done = 0;
+    while (done < k) {
+        const size_t at = static_cast<size_t>((rd + done) % kRdsRing);
+        const size_t run = std::min(k - done, static_cast<size_t>(kRdsRing) - at);
+        CU(cudaMemcpy(out + done, ring + at, run * sizeof(fmrx_rds_group), cudaMemcpyDeviceToHost));
+        done += run;
+    }
+    rd += k;
+    *n_out = k;
+    if (n_lost)
+        *n_lost = p->rds_lost[capture];
     return FMRX_OK;
 }
 
@@ -1898,5 +2067,125 @@ extern "C" int fmrx_find_stations(const double *psd, int n_fft, double rf_fs, do
     *n_found = static_cast<int>(st.size());
     for (int i = 0; i < max_out && i < static_cast<int>(st.size()); i++)
         out[i] = st[i];
+    return FMRX_OK;
+}
+
+// ---------------------------------------------------------------------------
+// RDS decoder: constants and tables (include/fmrx.h, fmrx_set_rds), and the group summary
+// ---------------------------------------------------------------------------
+
+namespace fmrx {
+
+RdsParams rds_params(int fs)
+{
+    RdsParams P{};
+    P.fs = fs;
+    P.D = fs == 288000 ? 12 : 10;
+    P.fs2 = fs / P.D;
+    P.L = static_cast<int>(P.fs2 / 2375.0 + 0.5);
+    P.M = P.fs2 / 10;
+    P.taps = 2 * static_cast<int>(63.0 * fs / 240000.0 + 0.5) + 1;
+    const int g = std::gcd(57000, fs);
+    P.P = fs / g;
+    P.q = 57000 / g;
+    const int g2 = std::gcd(2375, 2 * P.fs2);      // 1187.5 / fs2 = 2375 / (2 fs2)
+    P.Q = 2 * P.fs2 / g2;
+    P.q2 = 2375 / g2;
+    return P;
+}
+
+void rds_tables(const RdsParams &P, float *taps, float2 *mix, double2 *bitphase)
+{
+    const double pi = 3.14159265358979323846;
+    const int N = P.taps;
+    const double fc = 2.0 * 4000.0 / P.fs;
+    std::vector<double> h(N);
+    double sum = 0.0;
+    for (int n = 0; n < N; n++) {
+        const double x = n - (N - 1) / 2.0;
+        const double sinc = x == 0.0 ? 1.0 : std::sin(pi * fc * x) / (pi * fc * x);
+        const double w = 0.42 - 0.5 * std::cos(2 * pi * n / (N - 1)) + 0.08 * std::cos(4 * pi * n / (N - 1));
+        h[n] = fc * sinc * w;
+        sum += h[n];
+    }
+    for (int n = 0; n < N; n++)
+        taps[n] = static_cast<float>(h[n] / sum);
+    for (int k = 0; k < P.P; k++) {
+        const double a = 2 * pi * k / P.P;
+        mix[k] = make_float2(static_cast<float>(std::cos(a)), -static_cast<float>(std::sin(a)));
+    }
+    for (int k = 0; k < P.Q; k++) {
+        const double a = 2 * pi * k / P.Q;
+        bitphase[k] = make_double2(std::cos(a), -std::sin(a));
+    }
+}
+
+}  // namespace fmrx
+
+extern "C" int fmrx_rds_summarise(const fmrx_rds_group *g, size_t n, fmrx_rds_info *out)
+{
+    if (!out || (n && !g))
+        return FMRX_ERR_ARG;
+    std::memset(out, 0, sizeof(*out));
+    out->pty = out->tp = -1;
+    std::memset(out->ps, ' ', 8);
+    std::memset(out->rt, ' ', 64);
+    std::vector<uint16_t> pi_seen;
+    int ab = -1;
+    for (size_t i = 0; i < n; i++) {
+        const fmrx_rds_group &x = g[i];
+        out->groups++;
+        out->blocks_total += 4;
+        for (int b = 0; b < 4; b++)
+            out->blocks_valid += (x.valid >> b) & 1u;
+        if ((x.valid & 1u) && !out->pi_valid) {
+            if (std::find(pi_seen.begin(), pi_seen.end(), x.block[0]) != pi_seen.end()) {
+                out->pi_valid = 1;
+                out->pi = x.block[0];
+            } else {
+                pi_seen.push_back(x.block[0]);
+            }
+        }
+        if (!(x.valid & 2u))
+            continue;
+        const uint16_t B = x.block[1];
+        out->pty = (B >> 5) & 31;
+        out->tp = (B >> 10) & 1;
+        const int type = B >> 12, version_b = (B >> 11) & 1;
+        if (type == 0 && (x.valid & 8u)) {
+            const int seg = B & 3;
+            out->ps[2 * seg] = static_cast<char>(x.block[3] >> 8);
+            out->ps[2 * seg + 1] = static_cast<char>(x.block[3] & 0xFF);
+            out->ps_seen |= static_cast<uint8_t>(1u << seg);
+        } else if (type == 2) {
+            const int flag = (B >> 4) & 1, seg = B & 15;
+            if (version_b ? !(x.valid & 8u) : (x.valid & 12u) != 12u)
+                continue;
+            if (flag != ab) {
+                if (ab >= 0) {
+                    std::memset(out->rt, ' ', 64);
+                    out->rt_seen = 0;
+                }
+                ab = flag;
+            }
+            if (version_b) {
+                out->rt[2 * seg] = static_cast<char>(x.block[3] >> 8);
+                out->rt[2 * seg + 1] = static_cast<char>(x.block[3] & 0xFF);
+            } else {
+                out->rt[4 * seg] = static_cast<char>(x.block[2] >> 8);
+                out->rt[4 * seg + 1] = static_cast<char>(x.block[2] & 0xFF);
+                out->rt[4 * seg + 2] = static_cast<char>(x.block[3] >> 8);
+                out->rt[4 * seg + 3] = static_cast<char>(x.block[3] & 0xFF);
+            }
+            out->rt_seen |= static_cast<uint16_t>(1u << seg);
+        }
+    }
+    out->ps[8] = 0;
+    out->rt[64] = 0;
+    for (int k = 0; k < 64; k++)
+        if (out->rt[k] == 0x0D) {
+            out->rt[k] = 0;
+            break;
+        }
     return FMRX_OK;
 }

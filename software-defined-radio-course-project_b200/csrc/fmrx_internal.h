@@ -5,6 +5,7 @@
 #include <cstdint>
 #include <cuda_runtime.h>
 
+#include "fmrx.h"
 #include "fmrx_device.cuh"
 
 namespace fmrx {
@@ -126,5 +127,67 @@ cudaError_t launch_psd(float *psd, const float *samples, int n_seg, int freq_bin
 int scan_run_segments(int n_fft);
 cudaError_t launch_scan(const uint8_t *iq, int n_seg, int n_fft, const float *win, const float2 *tw, double *partial,
                         double *acc, cudaStream_t s);
+
+// RDS decoder (fmrx_rds_dec.cu; fmrx_set_rds): the constants of include/fmrx.h for one demod rate fs
+struct RdsParams {
+    int fs, D, fs2, L, M, taps;   // decimation, decimated rate, matched-filter half length, window, FIR taps
+    int P, q;                     // mixer: sample n uses mix[(q * (n mod P)) mod P]
+    int Q, q2;                    // window sums: sample m uses bitphase[(q2 * (m mod Q)) mod Q]
+};
+RdsParams rds_params(int fs);
+void rds_tables(const RdsParams &P, float *taps, float2 *mix, double2 *bitphase);
+
+constexpr int kRdsRing = 8192;        // groups per capture: about 12 minutes
+constexpr int kRdsBitRing = 128;      // bit instants kept: a group is 104 bits
+constexpr long long kRdsNoHit = -(1ll << 40);
+
+// One capture's decoder state between chunks (device memory; k_rds_bits works on a copy in shared memory).
+struct RdsDecState {
+    long long n_offset;           // the capture's IF index minus the pipeline's (nonzero after fmrx_set_state)
+    long long w_first, w_next;    // the decoder's first window; the next window to complete
+    long long j;                  // next bit index
+    long long nbits;              // bits decided since (re)start
+    long long last_hit[4];        // search: bit count at the last block matching offset position 0..3
+    long long t_ring[kRdsBitRing];   // IF index of bit count k at [k & 127]
+    unsigned long long reg;       // the last 52 decided bits, newest in bit 0
+    unsigned long long written;   // groups written to the ring since (re)start
+    double tau[4];                // tau of window w at [w & 3]
+    double t_prev;
+    double2 s_prev;
+    int have_prev, synced, pos, in_block, bad, pad_;
+    fmrx_rds_group cur;           // the group being assembled
+};
+
+struct RdsBasebandArgs {
+    RdsParams prm;
+    const int *caps;              // the captures with RDS on, one per blockIdx.y
+    const RdsDecState *state;     // [C] (n_offset)
+    const float *demod;           // as BandpassArgs: capture c at demod + c*if_stride, sample k at [if_off + k]
+    size_t if_stride;
+    int if_off;
+    int n_if;
+    long long if_run;             // IF samples in front of this chunk, counted by the pipeline since create/reset
+    const float *dtail;           // [C][dtail_len]: the demod samples before this chunk
+    int dtail_len;
+    const float *taps;            // [prm.taps]
+    const float2 *mix;            // [prm.P]: e^{-2 pi i k / P}
+    float2 *ybuf;                 // [C][ybuf_len]: y of m_lo - ytail_len + i at [i]
+    size_t ybuf_len;
+    int ytail_len;
+};
+struct RdsBitsArgs {
+    RdsParams prm;
+    const int *caps;
+    RdsDecState *state;
+    int n_if;
+    long long if_run;
+    float2 *ybuf;
+    size_t ybuf_len;
+    int ytail_len;
+    const double2 *bitphase;      // [prm.Q]: e^{-2 pi i k / Q}
+    fmrx_rds_group *ring;         // [C][kRdsRing]
+};
+int rds_baseband_smem(const RdsParams &P);
+cudaError_t launch_rds(const RdsBasebandArgs &b, const RdsBitsArgs &r, int n_caps, cudaStream_t s);
 
 }  // namespace fmrx

@@ -2,7 +2,7 @@
 //
 //   project                      mode 0 (message says "mono", like the reference)
 //   project <mode 0-3> <1|2|m|s> [--taps N] [--chunk-blocks K] [--device D] [--tune HZ] [--stats]
-//   project <mode 0-3> <1|2|m|s> --scan SECONDS [--fft N] [--threshold DB] [--device D]
+//   project <mode 0-3> <1|2|m|s> --scan SECONDS [--fft N] [--threshold DB] [--device D] [--rds]
 //
 // --tune HZ: decode the station HZ (an integer, may be negative) above the capture's centre
 // frequency (fmrx_set_tuning); |HZ| < rf_fs/2 of the mode, else the usage message and exit 1.
@@ -15,6 +15,11 @@
 // Welch segment length, a power of two in 256..16384 (default 4096); --threshold DB: the
 // detection threshold above the noise floor (default 10).  Malformed values, --fft or
 // --threshold without --scan, and --scan with --tune: the usage message and exit 1.
+//
+// --rds (with --scan only): then decode every station found from the same bytes (one pipeline, a capture tuned to
+// each station, one shared stream, RDS on; the PCM is discarded) and add two columns: pi (4 hex digits, or -) and
+// ps (8 characters; '_' where no segment arrived, '.' for bytes outside 0x20-0x7E).  --rds without --scan: the usage
+// message and exit 1.
 //
 // stdin : raw interleaved u8 I/Q at the mode's RF rate
 // stdout: raw s16le PCM, interleaved R,L, 48 or 44.1 kS/s -- for either channel
@@ -56,7 +61,7 @@ namespace {
 {
     std::fprintf(stderr, "Usage: %s\nor \nUsage %s <mode> <channels>\n"
                          "\t\t<mode> is a value from 0 to 3\n\t\t   <channels> is either 1 or 2\n"
-                         "or\nUsage %s <mode> <channels> --scan SECONDS [--fft N] [--threshold DB]\n",
+                         "or\nUsage %s <mode> <channels> --scan SECONDS [--fft N] [--threshold DB] [--rds]\n",
                  argv0, argv0, argv0);
     std::exit(1);
 }
@@ -73,8 +78,59 @@ size_t read_full(int fd, uint8_t *dst, size_t want)
     return got;
 }
 
+// --scan --rds: PI and PS of every station, decoded from the bytes the scan read (whole blocks)
+int rds_columns(const fmrx_mode_info &mi, int device, const std::vector<uint8_t> &iq, const fmrx_station *st, int n,
+                std::vector<std::string> &cols)
+{
+    cols.assign(n, "-\t________");
+    const size_t nb = iq.size() / mi.block_size;
+    if (n == 0 || nb == 0)
+        return 0;
+    fmrx_config cfg{};
+    cfg.mode = mi.mode;
+    cfg.taps = mi.taps;
+    cfg.n_captures = n;
+    cfg.device = device;
+    fmrx_pipeline *p = nullptr;
+    int rc = fmrx_create(&p, &cfg);
+    std::vector<int16_t> pcm;
+    for (int c = 0; rc == FMRX_OK && c < n; c++)
+        if ((rc = fmrx_set_tuning(p, c, std::round(st[c].offset_hz))) == FMRX_OK)
+            rc = fmrx_set_rds(p, c, 1);
+    if (rc == FMRX_OK) {
+        pcm.resize(static_cast<size_t>(n) * nb * 2 * mi.audio_per_block);
+        rc = fmrx_process(p, iq.data(), 0, nb, pcm.data(), nb * 2 * mi.audio_per_block);
+    }
+    std::vector<fmrx_rds_group> g(8192);
+    for (int c = 0; rc == FMRX_OK && c < n; c++) {
+        size_t got = 0;
+        fmrx_rds_info info;
+        if ((rc = fmrx_read_rds(p, c, g.data(), g.size(), &got, nullptr)) != FMRX_OK ||
+            (rc = fmrx_rds_summarise(g.data(), got, &info)) != FMRX_OK)
+            break;
+        char buf[32];
+        std::string ps;
+        for (int k = 0; k < 8; k++) {
+            const unsigned char ch = static_cast<unsigned char>(info.ps[k]);
+            ps += !((info.ps_seen >> (k / 2)) & 1) ? '_' : (ch >= 0x20 && ch <= 0x7E) ? static_cast<char>(ch) : '.';
+        }
+        if (info.pi_valid)
+            std::snprintf(buf, sizeof(buf), "%04X", info.pi);
+        else
+            std::snprintf(buf, sizeof(buf), "-");
+        cols[c] = std::string(buf) + "\t" + ps;
+    }
+    if (p)
+        fmrx_destroy(p);
+    if (rc != FMRX_OK) {
+        std::fprintf(stderr, "RDS: %s (%s)\n", fmrx_strerror(rc), fmrx_last_error());
+        return 1;
+    }
+    return 0;
+}
+
 // --scan: the stations in up to `seconds` of stdin (0: until EOF); exit status 0
-int scan_stdin(const fmrx_mode_info &mi, int device, double seconds, int fft, double threshold_db)
+int scan_stdin(const fmrx_mode_info &mi, int device, double seconds, int fft, double threshold_db, bool rds)
 {
     fmrx_scan *sc = nullptr;
     int rc = fmrx_scan_create(&sc, fft, mi.rf_fs, device);
@@ -89,6 +145,7 @@ int scan_stdin(const fmrx_mode_info &mi, int device, double seconds, int fft, do
         std::fprintf(stderr, "pinned allocation failed (%s)\n", fmrx_last_error());
         return 1;
     }
+    std::vector<uint8_t> kept;    // --rds: the bytes read, decoded after the scan
     for (uint64_t done = 0; done < limit;) {
         const size_t want = static_cast<size_t>(std::min<uint64_t>(chunk, limit - done));
         const size_t got = read_full(STDIN_FILENO, static_cast<uint8_t *>(buf), 2 * want) / 2;   // whole pairs
@@ -96,6 +153,8 @@ int scan_stdin(const fmrx_mode_info &mi, int device, double seconds, int fft, do
             std::fprintf(stderr, "fmrx_scan_process: %s (%s)\n", fmrx_strerror(rc), fmrx_last_error());
             return 1;
         }
+        if (rds)
+            kept.insert(kept.end(), static_cast<const uint8_t *>(buf), static_cast<const uint8_t *>(buf) + 2 * got);
         done += got;
         if (got < want)
             break;
@@ -109,8 +168,14 @@ int scan_stdin(const fmrx_mode_info &mi, int device, double seconds, int fft, do
         std::fprintf(stderr, "band scan: %s (%s)\n", fmrx_strerror(rc), fmrx_last_error());
         return 1;
     }
-    for (int i = 0; i < found; i++)
-        std::printf("%lld\t%.1f\t%.1f\n", std::llround(st[i].offset_hz), st[i].level_db, st[i].snr_db);
+    const int shown = std::min(found, fft);
+    std::vector<std::string> cols;
+    if (rds && rds_columns(mi, device, kept, st.data(), shown, cols) != 0)
+        return 1;
+    for (int i = 0; i < shown; i++) {
+        std::printf("%lld\t%.1f\t%.1f", std::llround(st[i].offset_hz), st[i].level_db, st[i].snr_db);
+        std::printf(rds ? "\t%s\n" : "\n", rds ? cols[i].c_str() : "");
+    }
     std::fflush(stdout);
     fmrx_host_free(buf);
     fmrx_scan_destroy(sc);
@@ -135,7 +200,7 @@ int main(int argc, char *argv[])
 {
     int mode = 0, channels = 1, taps = 51, chunk_blocks = 0, device = -1;
     long long tune_hz = 0;
-    bool stats = false, tuned = false, scan = false, scan_opts = false;
+    bool stats = false, tuned = false, scan = false, scan_opts = false, rds = false;
     double scan_s = 0.0, threshold_db = 10.0;
     int fft = 4096;
     // positional part, as src/project.cpp:278-299
@@ -157,6 +222,7 @@ int main(int argc, char *argv[])
             if (end == argv[i] || *end) usage(argv[0]);
             tuned = true;
         }
+        else if (a == "--rds") rds = true;
         else if (a == "--scan" || a == "--threshold") {
             if (i + 1 >= argc) usage(argv[0]);
             char *end = nullptr;
@@ -199,7 +265,7 @@ int main(int argc, char *argv[])
             return 1;
         }
     }
-    if ((scan && tuned) || (scan_opts && !scan))
+    if ((scan && tuned) || (scan_opts && !scan) || (rds && !scan))
         usage(argv[0]);
     std::fprintf(stderr, "Operating in mode %d, %s\n", mode, channels == 1 ? "mono" : "stereo");
 
@@ -211,7 +277,7 @@ int main(int argc, char *argv[])
     if (!(std::llabs(tune_hz) < mi.rf_fs / 2))
         usage(argv[0]);
     if (scan)
-        return scan_stdin(mi, device, scan_s, fft, threshold_db);
+        return scan_stdin(mi, device, scan_s, fft, threshold_db, rds);
     if (chunk_blocks <= 0) {
         // about 0.2 s of signal per call: low latency for a live rtl_sdr pipe
         chunk_blocks = static_cast<int>(0.2 * mi.rf_fs * 2 / mi.block_size);

@@ -17,6 +17,8 @@ statistics, not the same bytes).
 """
 from __future__ import annotations
 
+from collections import namedtuple
+
 import numpy as np
 
 PILOT_HZ = 19000.0
@@ -266,6 +268,95 @@ def synth_iq_exact_torch(n_pairs: int, n_captures: int, device, rf_fs: float = 2
 
 
 # ----------------------------------------------------------------------------------------
+# RDS (IEC 62106): the block code, and a station's group stream as a bit table
+# ----------------------------------------------------------------------------------------
+#
+# A station that broadcasts RDS adds  c * biphase(e_k) * sin(3 * pilot phase)  to its integer multiplex (Q45 like
+# the rest, c = rint(0.03 * 2^15): 3 % of the deviation).  The bit clock is the pilot's phase accumulator divided by
+# 16 (n * inc_p in 2^-32 turns, unwrapped: bit k = (n * inc_p) >> 36), so it is locked to the pilot as the standard
+# requires; biphase is + for the first half of a bit and - for the second, rectangular; e_k is the differentially
+# encoded data, e_k = d_k xor e_{k-1}.  The group cycle is 0A (PS segments 0..3) four times, then one 2A (the next
+# RT segment), so PS is complete after 4 groups (0.35 s) and RT after 5 per segment.
+
+RdsProgram = namedtuple("RdsProgram", "pi pty ps rt")   # pi: 16 bits, pty: 0..31, ps: <= 8 chars, rt: <= 64 chars
+
+RDS_POLY = 0x5B9                                         # g(x) = x^10 + x^8 + x^7 + x^5 + x^4 + x^3 + 1
+RDS_OFFSETS = {"A": 0x0FC, "B": 0x198, "C": 0x168, "C'": 0x350, "D": 0x1B4}
+# the parity-check matrix of IEC 62106 Annex B, first transmitted bit first: syndrome = xor of the rows of set bits
+RDS_H = (0x200, 0x100, 0x080, 0x040, 0x020, 0x010, 0x008, 0x004, 0x002, 0x001, 0x2DC, 0x16E, 0x0B7, 0x287, 0x39F,
+         0x313, 0x355, 0x376, 0x1BB, 0x201, 0x3DC, 0x1EE, 0x0F7, 0x2A7, 0x38F, 0x31B)
+RDS_SYNDROMES = {"A": 0x3D8, "B": 0x3D4, "C": 0x25C, "C'": 0x3CC, "D": 0x258}
+RDS_LEVEL = 983
+
+
+def rds_checkword(info: int) -> int:
+    """info(x) * x^10 mod g(x): the 10 check bits of a 16-bit information word, before the offset word."""
+    v = (info & 0xFFFF) << 10
+    for i in range(25, 9, -1):
+        if v >> i & 1:
+            v ^= RDS_POLY << (i - 10)
+    return v
+
+
+def rds_block(info: int, offset: str) -> int:
+    """The 26-bit block, first transmitted bit in bit 25."""
+    return ((info & 0xFFFF) << 10) | (rds_checkword(info) ^ RDS_OFFSETS[offset])
+
+
+def rds_syndrome(block: int) -> int:
+    s = 0
+    for i in range(26):
+        if block >> (25 - i) & 1:
+            s ^= RDS_H[i]
+    return s
+
+
+def _rds_rt(rt: str) -> bytes:
+    b = rt.encode("latin-1")[:64]
+    return b + b"\r" if len(b) < 64 else b
+
+
+def rds_group(prog: RdsProgram, g: int) -> tuple:
+    """Information words (A, B, C, D) of group g of the station's cycle: 0A x 4 (PS), then 2A (RT)."""
+    tp = 0
+    if g % 5 < 4:
+        seg = g % 5
+        ps = prog.ps.encode("latin-1")[:8].ljust(8)
+        b = (0 << 12) | (tp << 10) | (prog.pty << 5) | seg
+        return prog.pi, b, 0xE0CD, (ps[2 * seg] << 8) | ps[2 * seg + 1]
+    rt = _rds_rt(prog.rt)
+    n_seg = (len(rt) + 3) // 4
+    seg = (g // 5) % n_seg
+    txt = rt[4 * seg:4 * seg + 4].ljust(4)
+    b = (2 << 12) | (tp << 10) | (prog.pty << 5) | seg
+    return prog.pi, b, (txt[0] << 8) | txt[1], (txt[2] << 8) | txt[3]
+
+
+def rds_cycle_groups(prog: RdsProgram) -> int:
+    return 5 * ((len(_rds_rt(prog.rt)) + 3) // 4)
+
+
+def rds_bit_table(prog: RdsProgram) -> dict:
+    """The differentially encoded bits e_k of one period of the group cycle, and the parity that each further period
+    flips them by."""
+    bits = []
+    for g in range(rds_cycle_groups(prog)):
+        for info, off in zip(rds_group(prog, g), ("A", "B", "C", "D")):
+            blk = rds_block(info, off)
+            bits.extend((blk >> (25 - i)) & 1 for i in range(26))
+    e = np.bitwise_xor.accumulate(np.array(bits, np.int64))
+    return {"e": e, "period": len(bits), "flip": int(e[-1])}
+
+
+def _rds_mpx(n, inc_p, rds, sin12):
+    ph = n * inc_p                          # the pilot's phase accumulator, 2^-32 turns, unwrapped
+    k = ph >> 36                            # bit index: 16 pilot cycles per bit
+    e = rds["e"][k % rds["period"]] ^ ((k // rds["period"]) & rds["flip"])
+    sign = 1 - 2 * (e ^ ((ph >> 35) & 1))  # biphase: the second half of a bit is inverted
+    return RDS_LEVEL * sign * sin12[((ph * 3) & 0xFFFFFFFF) >> 20] * 32768
+
+
+# ----------------------------------------------------------------------------------------
 # Several stations in one stream (what one RTL-SDR capture of the FM band holds)
 # ----------------------------------------------------------------------------------------
 #
@@ -279,10 +370,15 @@ def synth_iq_exact_torch(n_pairs: int, n_captures: int, device, rf_fs: float = 2
 
 def _multi_plans(rf_fs: float, stations):
     plans = []
-    for off, idx, kind, gain in stations:
+    for st in stations:
+        off, idx, kind, gain = st[:4]
+        rds = st[4] if len(st) > 4 else None
         if not abs(off) < rf_fs / 2:
             raise ValueError(f"offset {off} outside +-rf_fs/2")
-        plans.append((_exact_plan(rf_fs, idx, kind, None, None, None), int(round(off / rf_fs * 2.0 ** 40)), int(gain)))
+        plan = _exact_plan(rf_fs, idx, kind, None, None, None)
+        if rds is not None:
+            plan = dict(plan, rds=rds_bit_table(rds))
+        plans.append((plan, int(round(off / rf_fs * 2.0 ** 40)), int(gain)))
     if not plans:
         raise ValueError("no stations")
     return plans
@@ -299,6 +395,8 @@ def _multi_iq(n, plans, carries, tables, consts, cumsum):
             return sin12[((n * inc) & 0xFFFFFFFF) >> 20]
         sl, sr, sp, s38 = tone(p["inc_l"]), tone(p["inc_r"]), tone(p["inc_p"]), tone(p["inc_38"])
         mpx = (p["a"] * (sl + sr) + p["b"] * sp) * 32768 + p["a"] * (sl - sr) * s38
+        if "rds" in p:
+            mpx = mpx + _rds_mpx(n, p["inc_p"], p["rds"], sin12)
         dphi = ((mpx * p["kdev"] + (1 << 62)) >> 25) - (1 << 37)
         phi = cumsum(dphi) + carry
         new_carries.append(phi[-1])
@@ -320,7 +418,8 @@ def _multi_iq(n, plans, carries, tables, consts, cumsum):
 
 class ExactMultiSynth:
     """Stateful numpy generator of several stations in one stream: ``stations`` is a list of
-    ``(offset_hz, station_index, kind, gain)``; ``read(n_pairs)`` returns the next ``2*n_pairs``
+    ``(offset_hz, station_index, kind, gain)``, or of ``(offset_hz, station_index, kind, gain, RdsProgram)`` for a
+    station that broadcasts RDS; ``read(n_pairs)`` returns the next ``2*n_pairs``
     bytes (any split into reads gives the same bytes)."""
 
     def __init__(self, rf_fs: float, stations):
@@ -358,6 +457,9 @@ def synth_iq_exact_multi_torch(n_pairs: int, rf_fs: float, stations, device, chu
 
     dev = torch.device(device)
     plans = _multi_plans(rf_fs, stations)
+    for p, _, _ in plans:
+        if "rds" in p:
+            p["rds"] = dict(p["rds"], e=torch.from_numpy(p["rds"]["e"]).to(dev))
     tables = tuple(torch.from_numpy(t).to(dev) for t in _exact_tables())
     consts = tuple(torch.tensor(_s64(v), dtype=torch.int64, device=dev)
                    for v in (_GOLD, _MIX1, _MIX2, plans[0][0]["seed_mix"]))
