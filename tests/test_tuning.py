@@ -1,5 +1,5 @@
-"""Tuning to stations off the capture's centre, on the CPU: the oracle's tuning mixer (orc_chain_set_tuning), the
-multi-station synthesiser, and what a tuned chain decodes out of a stream that holds three stations."""
+"""Tuning to stations off the capture's centre, on the CPU: the oracle's tuning mixer (orc_chain_set_tuning) and
+what a tuned chain decodes out of a stream that holds three stations."""
 import ctypes
 
 import numpy as np
@@ -39,26 +39,6 @@ def test_tuned_oracle_rejects_offsets_beyond_half_the_rf_rate(port):
         for bad in (half, -half, 1e9, float("nan")):
             with pytest.raises(ValueError):
                 port.chain(mode, 51, tune_hz=bad)
-
-
-def test_multi_synth_with_one_centred_station_is_synth_iq_exact(synth):
-    n = 400_003
-    for kind in synth.KINDS_EXACT:
-        a = synth.synth_iq_exact(n, 2.4e6, station=7, kind=kind)
-        b = synth.synth_iq_exact_multi(n, 2.4e6, [(0.0, 7, kind, 256)], chunk=1 << 17)
-        assert np.array_equal(a, b), kind
-
-
-def test_multi_synth_numpy_and_torch_generate_identical_bytes(synth):
-    torch = pytest.importorskip("torch")
-    n = 700_001
-    st = [(-875e3, 2, "stereo", 60), (125e3, 11, "stereo", 60), (0.0, 0, "noise", 60), (875e3, 30, "offtune", 60)]
-    a = synth.synth_iq_exact_multi(n, 2.4e6, st, chunk=1 << 18)
-    b = synth.synth_iq_exact_multi_torch(n, 2.4e6, st, "cpu", chunk=(1 << 19) + 13).numpy()
-    assert np.array_equal(a, b)
-    g = synth.ExactMultiSynth(2.4e6, st)
-    c = np.concatenate([g.read(1), g.read(99_999), g.read(n - 100_000)])
-    assert np.array_equal(a, c)
 
 
 def _tone_levels_db(pcm, tones):

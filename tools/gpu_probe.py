@@ -19,7 +19,6 @@ ap.add_argument("--mode", type=int, default=0)
 ap.add_argument("--taps", type=int, default=51)
 ap.add_argument("--chunk", type=int, default=0)
 ap.add_argument("--reps", type=int, default=3)
-ap.add_argument("--gpu-synth", action="store_true", help="generate the capture on the GPU (long captures)")
 ap.add_argument("--kind", default="", help="integer synthesiser kind (stereo, noise, offtune, nopilot): made on the GPU")
 ap.add_argument("--split", type=float, default=0.0, help="seconds processed in a first call (timed separately)")
 a = ap.parse_args()
@@ -29,8 +28,6 @@ nb = max(1, int(a.seconds * info.rf_fs * 2 / info.block_size))
 C = a.captures
 if a.kind:
     one = pkg.synth.synth_iq_exact_torch(nb * info.block_size // 2, 1, torch.device("cuda"), float(info.rf_fs), kinds=[a.kind])[0]
-elif a.gpu_synth:
-    one = pkg.synth.synth_iq_torch(nb * info.block_size // 2, 1, torch.device("cuda"), info.rf_fs, seed=0)[0]
 else:
     one = torch.from_numpy(pkg.synth.synth_iq(nb * info.block_size // 2, info.rf_fs, seed=0)).cuda()
 iq = one.unsqueeze(0).repeat(C, 1).contiguous()
