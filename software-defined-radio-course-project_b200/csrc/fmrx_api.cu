@@ -10,8 +10,8 @@
 //     back  : K4 audio -> [D2H]
 // Chunk i+1's front stage and chunk i-1's back stage run under chunk i's PLL.
 // Buffers rotate over kSets sets; the FIR history each stage needs from the
-// previous chunk is kept in small per-capture "tail" arrays owned by the stream
-// that produces the data, and copied in front of the next chunk's buffer.
+// previous chunk is kept in a small per-capture "tail" (CarryLayout), written by
+// the stream that produces the data, and copied in front of the next chunk's buffer.
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
@@ -324,6 +324,7 @@ extern "C" int fmrx_pll(float *inout, size_t n, float freq, float Fs, float nco_
     a.if_off = 0;
     a.n_if = static_cast<int>(n);
     a.state = d_state.as<float>();
+    a.state_stride = 8;
     a.prm = make_pll_params(freq, Fs, nco_scale, phase_adjust, norm_bandwidth);
     CU(launch_pll(a, 1, 0));
     CU(launch_nco(d_x.as<float>(), d_trig.as<float>(), n, nco_scale, phase_adjust, 0));
@@ -434,6 +435,37 @@ PipelineSizes pipeline_sizes(const fmrx_mode_info &mi)
              std::min<long long>(((1ll << 26) - 1) / mi.if_per_block, ((1ll << 31) - 1) / mi.block_size) };
 }
 
+// What a capture carries from one chunk to the next: one record per capture (fmrx_pipeline::d_carry) holding the bytes
+// that follow StateHeader in its blob, in the same order, padded to `pitch` on the device only:
+//     [IQ history: 2*hist_pairs bytes, padded to 4][demod tail: H f32][chan tail: H f32] [trig tail: H f32][PLL: 8 f32]
+// The first three are FMRX_STATE_FEEDFORWARD, the last two FMRX_STATE_PLL, which is also what a time shard hands on.
+struct ByteRange {
+    size_t off, len;
+};
+struct CarryLayout {
+    size_t hist_bytes;              // the IQ history, at offset 0
+    size_t demod, chan, trig, pll;  // offsets
+    ByteRange feedforward, pll_part;
+    size_t body;                    // a blob is sizeof(StateHeader) + body bytes
+    size_t pitch;                   // body rounded up to 16 bytes: every record is 16-byte aligned
+};
+
+CarryLayout carry_layout(int hist_pairs, int H)
+{
+    const size_t fH = static_cast<size_t>(H) * sizeof(float);
+    CarryLayout l;
+    l.hist_bytes = 2 * static_cast<size_t>(hist_pairs);
+    l.demod = (l.hist_bytes + 3) & ~static_cast<size_t>(3);
+    l.chan = l.demod + fH;
+    l.trig = l.chan + fH;
+    l.pll = l.trig + fH;
+    l.body = l.pll + 8 * sizeof(float);
+    l.pitch = (l.body + 15) & ~static_cast<size_t>(15);
+    l.feedforward = { 0, l.trig };
+    l.pll_part = { l.trig, l.body - l.trig };
+    return l;
+}
+
 // What every handle's creator does first: refuse without a device, resolve -1 to the current device, make `dev`
 // current and refuse anything but sm_100.
 int open_device(int &dev, size_t *mem_pitch = nullptr)
@@ -469,11 +501,10 @@ struct fmrx_pipeline {
     size_t if_stride = 0;       // H + chunk_if
     bool keep_stages = false, timing = false;
     PllParams pll_prm{};
+    CarryLayout carry{};
 
     dptr<float> d_rf_taps, d_pilot_taps, d_chan_taps, d_audio_pm;
-    dptr<uint8_t> d_hist_iq;                              // [C][2*hist_pairs]
-    dptr<float> d_tail_demod, d_tail_chan, d_tail_trig;   // [C][H]
-    dptr<float> d_pll_state;                              // [C][8]
+    dptr<uint8_t> d_carry;          // [C][carry.pitch]: each capture's carried state
     std::vector<BufferSet> sets;    // the ring of chunk buffers (fmrx_config.n_sets; 3 by default)
     stream_ptr s_front, s_pll, s_back;
     stream_ptr s_h2d;               // host path: the H2D copies, so that chunk i+1 comes in under K1/K2 of chunk i
@@ -546,17 +577,46 @@ int rds_restart(fmrx_pipeline *p, int capture)
     return FMRX_OK;
 }
 
+// Copy `rows` rows of `width` bytes between pitched device arrays.
+cudaError_t copy2d(void *dst, size_t dpitch, const void *src, size_t spitch, size_t width,
+                   size_t rows, cudaStream_t s, cudaMemcpyKind kind = cudaMemcpyDeviceToDevice, size_t max_pitch = 0)
+{
+    // one row, or a pitch beyond what cudaMemcpy2D takes (cudaDeviceProp::memPitch, ~2 GiB: 7.5 minutes
+    // of mode-0 IQ per capture): plain copies, row by row
+    if (rows == 1 || (max_pitch && (dpitch > max_pitch || spitch > max_pitch))) {
+        for (size_t r = 0; r < rows; r++) {
+            cudaError_t e = cudaMemcpyAsync(static_cast<char *>(dst) + r * dpitch, static_cast<const char *>(src) + r * spitch,
+                                            width, kind, s);
+            if (e != cudaSuccess)
+                return e;
+        }
+        return cudaSuccess;
+    }
+    return cudaMemcpy2DAsync(dst, dpitch, src, spitch, width, rows, kind, s);
+}
+
+// Rows 1 .. rows-1 of a pitched device array, each a copy of the first `width` bytes of row 0: log2(rows) doubling
+// copies (what copy2d cannot do: cudaMemcpy2DAsync refuses a source pitch of 0).
+cudaError_t broadcast_rows(uint8_t *dst, size_t pitch, size_t width, size_t rows, cudaStream_t s)
+{
+    cudaError_t e = cudaSuccess;
+    for (size_t k = 1; k < rows && e == cudaSuccess; k *= 2)
+        e = copy2d(dst + k * pitch, pitch, dst, pitch, width, std::min(k, rows - k), s);
+    return e;
+}
+
 int reset_state(fmrx_pipeline *p)
 {
     const size_t C = p->C;
-    CU(cudaMemset(p->d_hist_iq.get(), 0x80, C * 2 * p->hist_pairs));      // u8 128 == 0.0f
-    CU(cudaMemset(p->d_tail_demod.get(), 0, C * p->H * sizeof(float)));
-    CU(cudaMemset(p->d_tail_chan.get(), 0, C * p->H * sizeof(float)));
-    CU(cudaMemset(p->d_tail_trig.get(), 0, C * p->H * sizeof(float)));
-    std::vector<float> st(C * 8);
-    for (size_t c = 0; c < C; c++)
-        std::copy(kPllInitState, kPllInitState + 8, st.begin() + 8 * c);
-    CU(cudaMemcpy(p->d_pll_state.get(), st.data(), st.size() * sizeof(float), cudaMemcpyHostToDevice));
+    const CarryLayout &L = p->carry;
+    std::vector<uint8_t> rec(L.pitch, 0);
+    std::fill_n(rec.begin(), L.hist_bytes, uint8_t{ 0x80 });      // u8 128 == 0.0f
+    std::memcpy(rec.data() + L.pll, kPllInitState, sizeof(kPllInitState));
+    // on the front stream, which runs first in every chunk; done before return, since a time shard's hand-off
+    // writes into record 0 from another stream
+    CU(cudaMemcpyAsync(p->d_carry.get(), rec.data(), L.pitch, cudaMemcpyHostToDevice, p->s_front.get()));
+    CU(broadcast_rows(p->d_carry.get(), L.pitch, L.pitch, C, p->s_front.get()));
+    CU(cudaStreamSynchronize(p->s_front.get()));
     p->blocks_done.assign(C, 0);
     p->blocks_run = 0;
     for (auto &t : p->tune)
@@ -603,34 +663,6 @@ int ensure_stage_storage(fmrx_pipeline *p, size_t n_blocks)
     return FMRX_OK;
 }
 
-// Copy `rows` rows of `width` bytes between pitched device arrays.
-cudaError_t copy2d(void *dst, size_t dpitch, const void *src, size_t spitch, size_t width,
-                   size_t rows, cudaStream_t s, cudaMemcpyKind kind = cudaMemcpyDeviceToDevice, size_t max_pitch = 0)
-{
-    // one row, or a pitch beyond what cudaMemcpy2D takes (cudaDeviceProp::memPitch, ~2 GiB: 7.5 minutes
-    // of mode-0 IQ per capture): plain copies, row by row
-    if (rows == 1 || (max_pitch && (dpitch > max_pitch || spitch > max_pitch))) {
-        for (size_t r = 0; r < rows; r++) {
-            cudaError_t e = cudaMemcpyAsync(static_cast<char *>(dst) + r * dpitch, static_cast<const char *>(src) + r * spitch,
-                                            width, kind, s);
-            if (e != cudaSuccess)
-                return e;
-        }
-        return cudaSuccess;
-    }
-    return cudaMemcpy2DAsync(dst, dpitch, src, spitch, width, rows, kind, s);
-}
-
-// `rows` contiguous device rows of `width` bytes, each a copy of one source row: one copy, then doubling
-// (what copy2d cannot do: cudaMemcpy2DAsync refuses a source pitch of 0).
-cudaError_t broadcast_rows(uint8_t *dst, const uint8_t *src, size_t width, size_t rows, cudaStream_t s)
-{
-    cudaError_t e = cudaMemcpyAsync(dst, src, width, cudaMemcpyDeviceToDevice, s);
-    for (size_t k = 1; k < rows && e == cudaSuccess; k *= 2)
-        e = cudaMemcpyAsync(dst + k * width, dst, std::min(k, rows - k) * width, cudaMemcpyDeviceToDevice, s);
-    return e;
-}
-
 // The chunk loop shared by the host- and device-pointer entry points.
 // feedforward_only: K1 and K2 only -- what a time shard runs over the blocks in FRONT of its own (its halo), from the
 // zero state, to arrive at the IQ / demod / channel histories the stream has at the shard's first block.
@@ -641,6 +673,8 @@ int run(fmrx_pipeline *p, const uint8_t *iq, size_t iq_stride, size_t n_blocks, 
     const int C = p->C, T = mi.taps, H = p->H;
     const size_t fH = static_cast<size_t>(H) * sizeof(float);
     const size_t if_pitch = p->if_stride * sizeof(float);
+    const CarryLayout &L = p->carry;
+    uint8_t *const carry = p->d_carry.get();
 
     if (host_io) {
         const int rc = ensure_host_staging(p);
@@ -714,14 +748,15 @@ int run(fmrx_pipeline *p, const uint8_t *iq, size_t iq_stride, size_t n_blocks, 
             iq_dev_stride = iq_stride;
         }
         if (te) CU(cudaEventRecord(te[0].get(), p->s_front.get()));
-        CU(copy2d(S.demod.get(), if_pitch, p->d_tail_demod.get(), fH, fH, C, p->s_front.get()));
-        CU(copy2d(S.chan.get(), if_pitch, p->d_tail_chan.get(), fH, fH, C, p->s_front.get()));
+        CU(copy2d(S.demod.get(), if_pitch, carry + L.demod, L.pitch, fH, C, p->s_front.get()));
+        CU(copy2d(S.chan.get(), if_pitch, carry + L.chan, L.pitch, fH, C, p->s_front.get()));
         {
             RfDemodArgs a{};
             a.iq = iq_dev;
             a.iq_stride = iq_dev_stride;
-            a.hist = p->d_hist_iq.get();
+            a.hist = carry;
             a.hist_pairs = p->hist_pairs;
+            a.hist_stride = static_cast<int>(L.pitch);
             a.taps = p->d_rf_taps.get();
             a.T = T;
             a.decim = mi.rf_decim;
@@ -742,12 +777,10 @@ int run(fmrx_pipeline *p, const uint8_t *iq, size_t iq_stride, size_t n_blocks, 
         if (te) CU(cudaEventRecord(te[1].get(), p->s_front.get()));
         // IQ history for the next chunk: the last hist_pairs pairs of this chunk (per capture, also when the
         // captures share one stream: state blobs are per capture)
-        const size_t hist_bytes = 2 * static_cast<size_t>(p->hist_pairs);
-        if (iq_dev_stride)
-            CU(copy2d(p->d_hist_iq.get(), hist_bytes, iq_dev + chunk_bytes - hist_bytes, iq_dev_stride, hist_bytes, C,
-                      p->s_front.get()));
-        else
-            CU(broadcast_rows(p->d_hist_iq.get(), iq_dev + chunk_bytes - hist_bytes, hist_bytes, C, p->s_front.get()));
+        CU(copy2d(carry, L.pitch, iq_dev + chunk_bytes - L.hist_bytes, iq_dev_stride, L.hist_bytes, iq_dev_stride ? C : 1,
+                  p->s_front.get()));
+        if (!iq_dev_stride)
+            CU(broadcast_rows(carry, L.pitch, L.hist_bytes, C, p->s_front.get()));
         if (host_io) {
             CU(cudaEventRecord(S.iq_free.get(), p->s_front.get()));
             S.iq_free_pending = true;
@@ -769,8 +802,8 @@ int run(fmrx_pipeline *p, const uint8_t *iq, size_t iq_stride, size_t n_blocks, 
         }
         if (te) CU(cudaEventRecord(te[2].get(), p->s_front.get()));
         // tails for the next chunk's front stage
-        CU(copy2d(p->d_tail_demod.get(), fH, S.demod.get() + n_if, if_pitch, fH, C, p->s_front.get()));
-        CU(copy2d(p->d_tail_chan.get(), fH, S.chan.get() + n_if, if_pitch, fH, C, p->s_front.get()));
+        CU(copy2d(carry + L.demod, L.pitch, S.demod.get() + n_if, if_pitch, fH, C, p->s_front.get()));
+        CU(copy2d(carry + L.chan, L.pitch, S.chan.get() + n_if, if_pitch, fH, C, p->s_front.get()));
         CU(cudaEventRecord(S.front_done.get(), p->s_front.get()));
         if (!p->rds_caps.empty() && !feedforward_only) {
             // RDS beside K3: on the front stream after front_done, so that K3 does not wait for it
@@ -817,7 +850,7 @@ int run(fmrx_pipeline *p, const uint8_t *iq, size_t iq_stride, size_t n_blocks, 
 
         // ---------------- pll: K3 ----------------
         CU(cudaStreamWaitEvent(p->s_pll.get(), S.front_done.get(), 0));
-        CU(copy2d(S.trig.get(), if_pitch, p->d_tail_trig.get(), fH, fH, C, p->s_pll.get()));
+        CU(copy2d(S.trig.get(), if_pitch, carry + L.trig, L.pitch, fH, C, p->s_pll.get()));
         if (te) CU(cudaEventRecord(te[3].get(), p->s_pll.get()));
         {
             PllArgs a{};
@@ -827,13 +860,14 @@ int run(fmrx_pipeline *p, const uint8_t *iq, size_t iq_stride, size_t n_blocks, 
             a.if_stride = p->if_stride;
             a.if_off = H;
             a.n_if = n_if;
-            a.state = p->d_pll_state.get();
+            a.state = reinterpret_cast<float *>(carry + L.pll);
+            a.state_stride = static_cast<int>(L.pitch / sizeof(float));
             a.prm = p->pll_prm;
             CU(launch_pll(a, C, p->s_pll.get()));
             p->launches++;
         }
         if (te) CU(cudaEventRecord(te[4].get(), p->s_pll.get()));
-        CU(copy2d(p->d_tail_trig.get(), fH, S.trig.get() + n_if, if_pitch, fH, C, p->s_pll.get()));
+        CU(copy2d(carry + L.trig, L.pitch, S.trig.get() + n_if, if_pitch, fH, C, p->s_pll.get()));
         CU(cudaEventRecord(S.pll_done.get(), p->s_pll.get()));
 
         // ---------------- back: K4 [D2H] ----------------
@@ -974,6 +1008,7 @@ extern "C" int fmrx_create(fmrx_pipeline **out, const fmrx_config *cfg)
     p->hist_pairs = T - 1 + mi.rf_decim;
     if (mi.if_per_block < p->H || mi.block_size / 2 < p->hist_pairs)
         return FMRX_ERR_ARG;
+    p->carry = carry_layout(p->hist_pairs, p->H);
     const long long cb_max = sz.max_chunk_blocks;
     if (cb_max < 1)
         return FMRX_ERR_ARG;
@@ -1012,11 +1047,7 @@ extern "C" int fmrx_create(fmrx_pipeline **out, const fmrx_config *cfg)
     CU(cudaMemcpy(p->d_chan_taps.get(), ch.data(), T * sizeof(float), cudaMemcpyHostToDevice));
     CU(cudaMemcpy(p->d_audio_pm.get(), au_pm.data(), au_pm.size() * sizeof(float), cudaMemcpyHostToDevice));
 
-    CU(dalloc(p->d_hist_iq, C * 2 * p->hist_pairs));
-    CU(dalloc(p->d_tail_demod, C * p->H));
-    CU(dalloc(p->d_tail_chan, C * p->H));
-    CU(dalloc(p->d_tail_trig, C * p->H));
-    CU(dalloc(p->d_pll_state, C * 8));
+    CU(dalloc(p->d_carry, C * p->carry.pitch));
     CU(dalloc(p->d_tune, C));
     p->tune.assign(C, RfTune{ 0, 0 });
     p->rds_on.assign(C, 0);
@@ -1127,8 +1158,7 @@ extern "C" size_t fmrx_state_size(const fmrx_pipeline *p)
 {
     if (!p)
         return 0;
-    const size_t iq = (2 * static_cast<size_t>(p->hist_pairs) + 3) & ~static_cast<size_t>(3);
-    return sizeof(StateHeader) + iq + 3 * static_cast<size_t>(p->H) * sizeof(float) + 8 * sizeof(float);
+    return sizeof(StateHeader) + p->carry.body;
 }
 
 extern "C" int fmrx_get_state(fmrx_pipeline *p, int capture, void *blob, size_t blob_size)
@@ -1137,24 +1167,14 @@ extern "C" int fmrx_get_state(fmrx_pipeline *p, int capture, void *blob, size_t 
         return FMRX_ERR_ARG;
     CU(cudaSetDevice(p->device));
     CU(cudaDeviceSynchronize());
-    uint8_t *b = static_cast<uint8_t *>(blob);
-    std::memset(b, 0, fmrx_state_size(p));
+    const CarryLayout &L = p->carry;
     StateHeader h{ kStateMagic, static_cast<uint32_t>(p->mi.mode), static_cast<uint32_t>(p->mi.taps),
                    static_cast<uint32_t>(p->H), static_cast<uint32_t>(p->hist_pairs), 0, p->blocks_done[capture] };
-    std::memcpy(b, &h, sizeof(h));
-    b += sizeof(h);
-    const size_t iqb = 2 * static_cast<size_t>(p->hist_pairs);
-    CU(cudaMemcpy(b, p->d_hist_iq.get() + capture * iqb, iqb, cudaMemcpyDeviceToHost));
-    b += (iqb + 3) & ~static_cast<size_t>(3);
-    const size_t fH = static_cast<size_t>(p->H) * sizeof(float);
-    CU(cudaMemcpy(b, p->d_tail_demod.get() + static_cast<size_t>(capture) * p->H, fH, cudaMemcpyDeviceToHost));
-    b += fH;
-    CU(cudaMemcpy(b, p->d_tail_chan.get() + static_cast<size_t>(capture) * p->H, fH, cudaMemcpyDeviceToHost));
-    b += fH;
-    CU(cudaMemcpy(b, p->d_tail_trig.get() + static_cast<size_t>(capture) * p->H, fH, cudaMemcpyDeviceToHost));
-    b += fH;
-    CU(cudaMemcpy(b, p->d_pll_state.get() + 8 * static_cast<size_t>(capture), 8 * sizeof(float),
-                  cudaMemcpyDeviceToHost));
+    std::memcpy(blob, &h, sizeof(h));
+    uint8_t *b = static_cast<uint8_t *>(blob) + sizeof(h);
+    CU(cudaMemcpy(b, p->d_carry.get() + capture * L.pitch, L.body, cudaMemcpyDeviceToHost));
+    // the padding after the IQ history is not state: zeros, whatever a blob given to fmrx_set_state held there
+    std::memset(b + L.hist_bytes, 0, L.demod - L.hist_bytes);
     return FMRX_OK;
 }
 
@@ -1174,25 +1194,12 @@ extern "C" int fmrx_set_state(fmrx_pipeline *p, int capture, const void *blob, s
     CU(cudaSetDevice(p->device));
     CU(cudaDeviceSynchronize());
     b += sizeof(h);
-    const size_t iqb = 2 * static_cast<size_t>(p->hist_pairs);
-    const size_t fH = static_cast<size_t>(p->H) * sizeof(float);
-    const uint8_t *b_iq = b;
-    const uint8_t *b_demod = b_iq + ((iqb + 3) & ~static_cast<size_t>(3));
-    const uint8_t *b_chan = b_demod + fH;
-    const uint8_t *b_trig = b_chan + fH;
-    const uint8_t *b_pll = b_trig + fH;
-    if (parts & FMRX_STATE_FEEDFORWARD) {
-        CU(cudaMemcpy(p->d_hist_iq.get() + capture * iqb, b_iq, iqb, cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(p->d_tail_demod.get() + static_cast<size_t>(capture) * p->H, b_demod, fH,
-                      cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(p->d_tail_chan.get() + static_cast<size_t>(capture) * p->H, b_chan, fH,
-                      cudaMemcpyHostToDevice));
-    }
+    uint8_t *rec = p->d_carry.get() + capture * p->carry.pitch;
+    const ByteRange &ff = p->carry.feedforward, &pll = p->carry.pll_part;
+    if (parts & FMRX_STATE_FEEDFORWARD)
+        CU(cudaMemcpy(rec + ff.off, b + ff.off, ff.len, cudaMemcpyHostToDevice));
     if (parts & FMRX_STATE_PLL) {
-        CU(cudaMemcpy(p->d_tail_trig.get() + static_cast<size_t>(capture) * p->H, b_trig, fH,
-                      cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(p->d_pll_state.get() + 8 * static_cast<size_t>(capture), b_pll, 8 * sizeof(float),
-                      cudaMemcpyHostToDevice));
+        CU(cudaMemcpy(rec + pll.off, b + pll.off, pll.len, cudaMemcpyHostToDevice));
         p->blocks_done[capture] = h.blocks_done;
         p->tune[capture].pair_offset = (h.blocks_done - p->blocks_run) * (p->mi.block_size / 2);
         CU(cudaMemcpy(p->d_tune.get() + capture, &p->tune[capture], sizeof(RfTune), cudaMemcpyHostToDevice));
@@ -1313,10 +1320,8 @@ extern "C" int fmrx_get_pll_state(fmrx_pipeline *p, int capture, float out[6])
         return FMRX_ERR_ARG;
     CU(cudaSetDevice(p->device));
     CU(cudaDeviceSynchronize());
-    float st[8];
-    CU(cudaMemcpy(st, p->d_pll_state.get() + 8 * static_cast<size_t>(capture), sizeof(st),
+    CU(cudaMemcpy(out, p->d_carry.get() + capture * p->carry.pitch + p->carry.pll, 6 * sizeof(float),
                   cudaMemcpyDeviceToHost));
-    std::memcpy(out, st, 6 * sizeof(float));
     return FMRX_OK;
 }
 
@@ -1530,14 +1535,13 @@ extern "C" int fmrx_long_process_device(fmrx_long_capture *L, const uint8_t *con
             if (rc != FMRX_OK)
                 return rc;
         }
-        // hand the PLL state on: behind this shard's last K3 (and its trigArg tail copy) on the PLL stream
+        // hand the PLL part of the carried state on (what FMRX_STATE_PLL restores): behind this shard's last K3 and
+        // its trigArg tail copy on the PLL stream
         if (r + 1 < L->n) {
             const TimeShard &next = *L->shard[r + 1];
-            fmrx_pipeline *q = next.pipe.get();
-            CU(cudaMemcpyPeerAsync(q->d_pll_state.get(), next.device, p->d_pll_state.get(), s.device, 8 * sizeof(float),
-                                   p->s_pll.get()));
-            CU(cudaMemcpyPeerAsync(q->d_tail_trig.get(), next.device, p->d_tail_trig.get(), s.device,
-                                   static_cast<size_t>(p->H) * sizeof(float), p->s_pll.get()));
+            const ByteRange &pll = p->carry.pll_part;
+            CU(cudaMemcpyPeerAsync(next.pipe->d_carry.get() + pll.off, next.device, p->d_carry.get() + pll.off, s.device,
+                                   pll.len, p->s_pll.get()));
             CU(cudaEventRecord(s.handed.get(), p->s_pll.get()));
         }
         // gather: this shard's PCM to the first device, behind its K4
@@ -1726,6 +1730,7 @@ extern "C" int fmrx_rds_process(fmrx_rds *r, const float *demod, size_t n, float
     a.if_off = 0;
     a.n_if = ni;
     a.state = r->d_pll_state.get();
+    a.state_stride = 8;
     a.prm = r->prm;
     CU(launch_pll(a, 1, 0));                                                                             // :256
     CU(launch_rds_mix(d_out, d_trig, d_chan, r->d_shift_state.get(), r->delay, n, r->prm.scale, r->prm.adjust, 0));   // :259-263, :269

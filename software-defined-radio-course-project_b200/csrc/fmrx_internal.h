@@ -20,8 +20,9 @@ constexpr int kMaxTaps = 512;
 struct RfDemodArgs {
     const uint8_t *iq;      // capture c at iq + c*iq_stride; chunk-local pair m at byte 2m
     size_t iq_stride;       // bytes
-    const uint8_t *hist;    // capture c at hist + c*2*hist_pairs; the pairs before this chunk
+    const uint8_t *hist;    // capture c at hist + c*hist_stride; the pairs before this chunk
     int hist_pairs;         // >= taps-1+decim
+    int hist_stride;        // bytes, a multiple of 2
     const float *taps;      // device, T floats
     int T, decim;
     int n_if;               // IF outputs per capture in this chunk
@@ -69,9 +70,10 @@ struct PllArgs {
     size_t if_stride;
     int if_off;
     int n_if;
-    float *state;           // capture c at state + 8*c: integ, phase, fbI, fbQ, ncoLast, trigOffset
+    float *state;           // capture c at state + c*state_stride: integ, phase, fbI, fbQ, ncoLast, trigOffset, 2 diagnostics
     PllParams prm;
     pllcore::TrigK kconst;  // filled by launch_pll: read as constant-bank operands in the loop
+    int state_stride;       // floats (last, so that the loop's constant-bank operands keep their offsets)
 };
 cudaError_t launch_pll(const PllArgs &a, int n_captures, cudaStream_t s);
 

@@ -136,7 +136,7 @@ __global__ void __launch_bounds__(RFW_THREADS) k_rf_demod_win(const RfDemodArgs 
     const int tid = threadIdx.x;
     const long long n_pairs = (long long)a.n_if * D;
     const uint8_t *iq = a.iq + (size_t)c * a.iq_stride;
-    const uint8_t *hist = a.hist + (size_t)c * 2 * a.hist_pairs;
+    const uint8_t *hist = a.hist + (size_t)c * a.hist_stride;
     const uint16_t *iq16 = reinterpret_cast<const uint16_t *>(iq);
     const uint16_t *hist16 = reinterpret_cast<const uint16_t *>(hist);
     const int padl0 = Tpad - T;
@@ -1172,7 +1172,7 @@ __global__ void __launch_bounds__(PLL_THREADS) k_pll(const PllArgs a)
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const float *p = a.pilot + (size_t)c * a.pilot_stride;
     float *tr = a.trig + (size_t)c * a.if_stride + a.if_off;
-    float *st = a.state + 8 * (size_t)c;
+    float *st = a.state + (size_t)c * a.state_stride;
     const int n = a.n_if;
 
     Consts k;
