@@ -209,7 +209,10 @@ int fmrx_set_tuning(fmrx_pipeline *p, int capture, double offset_hz);
  * Configuration, not state: only at the start of the capture's stream (after
  * create or reset), else FMRX_ERR_STATE; it survives fmrx_reset, which clears
  * the decoder and its ring.  Not in the state blob: fmrx_set_state on a capture
- * with RDS on restarts its decoder (search, empty ring) at the restored position.
+ * with RDS on restarts its decoder (search, empty ring) at the restored position
+ * n_r: the demod before n_r counts as zero; windows stay aligned to m = 0, the
+ * first being w_r = floor(m_r/M), m_r = ceil(n_r/D); tau is constant before
+ * window w_r and is not unwrapped at it; the first bit is j = ceil(m_r/sps).
  * With RDS off for every capture nothing is launched.  enable 0 or 1, else
  * FMRX_ERR_ARG.  The PCM and every stage are the same with RDS on or off. */
 int fmrx_set_rds(fmrx_pipeline *p, int capture, int enable);
@@ -228,6 +231,33 @@ typedef struct {
  * be NULL).  Waits for the pipeline's work in flight. */
 int fmrx_read_rds(fmrx_pipeline *p, int capture, fmrx_rds_group *out, size_t max, size_t *n_out,
                   uint64_t *n_lost);
+
+typedef struct {
+    uint64_t m_end;        /* ceil(n/D) at the stream position n: y[m] is final for m < m_end */
+    int64_t w_next;        /* the next window to complete */
+    int64_t j;             /* the next bit index */
+    int64_t nbits;         /* bits decided since (re)start */
+    uint64_t written;      /* groups emitted since (re)start */
+    uint64_t reg;          /* the last 52 decided bits, newest in bit 0 */
+    double t_prev;         /* t of bit j - 1 (units of 1/fs2); NaN before the first */
+    double tau;            /* tau of window w_next - 1; NaN before the first window */
+    int32_t synced;        /* 1 in sync, 0 in search */
+    int32_t reserved;
+} fmrx_rds_probe_info;
+
+/* A read-only view of `capture`'s decoder, for tests and diagnostics: its scalar
+ * state, and y[m] for m in [m_end - *y_n, m_end) (the history it keeps for the
+ * bits still to be decided) as interleaved (re, im) floats into y, at most y_max
+ * samples, the newest kept.  y may be NULL when y_max is 0; *y_n (may be NULL)
+ * is then the history's length.  Copies only: nothing of the decoder's layout is
+ * part of the ABI.  Waits for the pipeline's work in flight.  FMRX_ERR_ARG for a
+ * bad capture or a NULL out; FMRX_ERR_STATE when RDS is off for the capture.
+ * Bits are decided a window at a time (M outputs, about 119 bits), so reg holds
+ * the last 52 bits of the latest window, not every bit since the last probe.
+ * tests/test_gpu_rds_parity.py compares y, the scalars and those 52 bits with
+ * the float64 oracle after every call. */
+int fmrx_rds_probe(fmrx_pipeline *p, int capture, fmrx_rds_probe_info *out, float *y, size_t y_max,
+                   size_t *y_n);
 
 typedef struct {
     int pi_valid;          /* a PI value has appeared in two valid A blocks */

@@ -39,7 +39,8 @@ ABI_SYMBOLS = (
     "fmrx_process", "fmrx_process_device", "fmrx_read_stage",
     "fmrx_state_size", "fmrx_get_state", "fmrx_set_state", "fmrx_get_pll_state",
     "fmrx_host_alloc", "fmrx_host_free", "fmrx_kernel_launches", "fmrx_set_timing",
-    "fmrx_last_timing", "fmrx_set_tuning", "fmrx_set_rds", "fmrx_read_rds", "fmrx_rds_summarise",
+    "fmrx_last_timing", "fmrx_set_tuning", "fmrx_set_rds", "fmrx_read_rds", "fmrx_rds_probe",
+    "fmrx_rds_summarise",
     "fmrx_long_create", "fmrx_long_destroy", "fmrx_long_shard", "fmrx_long_process", "fmrx_long_process_device",
     "fmrx_long_last_ms", "fmrx_long_pll_state",
     "fmrx_rds_create", "fmrx_rds_destroy", "fmrx_rds_reset", "fmrx_rds_process", "fmrx_rds_pll_state",
@@ -75,6 +76,12 @@ class RdsGroupStruct(C.Structure):
                 ("reserved", C.c_uint16)]
 
 
+class RdsProbeStruct(C.Structure):
+    _fields_ = [("m_end", C.c_uint64), ("w_next", C.c_int64), ("j", C.c_int64), ("nbits", C.c_int64),
+                ("written", C.c_uint64), ("reg", C.c_uint64), ("t_prev", C.c_double), ("tau", C.c_double),
+                ("synced", C.c_int32), ("reserved", C.c_int32)]
+
+
 class RdsInfoStruct(C.Structure):
     _fields_ = [("pi_valid", C.c_int), ("pi", C.c_uint16), ("pty", C.c_int), ("tp", C.c_int), ("ps", C.c_char * 9),
                 ("ps_seen", C.c_uint8), ("rt", C.c_char * 65), ("rt_seen", C.c_uint16), ("groups", C.c_uint64),
@@ -86,6 +93,7 @@ RDS_GROUP_DTYPE = np.dtype([("if_index", "<u8"), ("block", "<u2", (4,)), ("valid
                             ("reserved", "<u2")], align=True)
 assert RDS_GROUP_DTYPE.itemsize == C.sizeof(RdsGroupStruct)
 
+RdsProbe = namedtuple("RdsProbe", "m_lo m_end y w_next j nbits written reg t_prev tau synced")
 RdsInfo = namedtuple("RdsInfo", "pi pty tp ps ps_seen rt rt_seen groups blocks_valid blocks_total")
 
 
@@ -159,6 +167,8 @@ def load() -> C.CDLL:
     L.fmrx_set_rds.argtypes = [C.c_void_p, C.c_int, C.c_int]
     L.fmrx_read_rds.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t),
                                 C.POINTER(C.c_uint64)]
+    L.fmrx_rds_probe.argtypes = [C.c_void_p, C.c_int, C.POINTER(RdsProbeStruct), _f32p, C.c_size_t,
+                                 C.POINTER(C.c_size_t)]
     L.fmrx_rds_summarise.argtypes = [C.c_void_p, C.c_size_t, C.POINTER(RdsInfoStruct)]
     L.fmrx_scan_create.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.c_double, C.c_int]
     L.fmrx_scan_destroy.argtypes = [C.c_void_p]
@@ -323,6 +333,18 @@ class Pipeline:
                "fmrx_read_rds")
         self.rds_lost[capture] = int(lost.value)
         return out[:n.value].copy()
+
+    def rds_probe(self, capture: int = 0) -> RdsProbe:
+        """A copy of ``capture``'s RDS decoder state (fmrx_rds_probe): the scalars, and ``y`` (complex64) for m in
+        ``[m_lo, m_end)``, the matched filter's output the decoder keeps."""
+        st = RdsProbeStruct()
+        n = C.c_size_t(0)
+        _check(self._L.fmrx_rds_probe(self._h, capture, C.byref(st), None, 0, C.byref(n)), "fmrx_rds_probe")
+        y = np.zeros(n.value, np.complex64)
+        _check(self._L.fmrx_rds_probe(self._h, capture, C.byref(st), y.view(np.float32).ctypes.data_as(_f32p), len(y),
+                                      C.byref(n)), "fmrx_rds_probe")
+        return RdsProbe(int(st.m_end) - len(y), int(st.m_end), y, int(st.w_next), int(st.j), int(st.nbits),
+                        int(st.written), int(st.reg), float(st.t_prev), float(st.tau), int(st.synced))
 
     def set_tuning(self, capture: int, hz: float):
         """Tune ``capture`` to the station ``hz`` above its stream's centre (negative: below); only at the start of

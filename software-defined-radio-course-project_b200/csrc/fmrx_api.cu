@@ -1293,6 +1293,39 @@ extern "C" int fmrx_read_rds(fmrx_pipeline *p, int capture, fmrx_rds_group *out,
     return FMRX_OK;
 }
 
+extern "C" int fmrx_rds_probe(fmrx_pipeline *p, int capture, fmrx_rds_probe_info *out, float *y, size_t y_max,
+                              size_t *y_n)
+{
+    if (!p || capture < 0 || capture >= p->C || !out || (!y && y_max))
+        return FMRX_ERR_ARG;
+    if (!p->rds_on[capture])
+        return FMRX_ERR_STATE;
+    CU(cudaSetDevice(p->device));
+    CU(cudaStreamSynchronize(p->s_front.get()));
+    RdsDecState st;
+    CU(cudaMemcpy(&st, p->d_rds_state.get() + capture, sizeof(st), cudaMemcpyDeviceToHost));
+    const RdsParams &P = p->rds_prm;
+    const long long n = p->blocks_done[capture] * p->mi.if_per_block;
+    std::memset(out, 0, sizeof(*out));
+    out->m_end = static_cast<uint64_t>((n + P.D - 1) / P.D);
+    out->w_next = st.w_next;
+    out->j = st.j;
+    out->nbits = st.nbits;
+    out->written = st.written;
+    out->reg = st.reg & ((1ull << 52) - 1);
+    out->t_prev = st.have_prev ? st.t_prev : std::nan("");
+    out->tau = st.w_next > st.w_first ? st.tau[(st.w_next - 1) & 3] : std::nan("");
+    out->synced = st.synced;
+    // after every chunk the buffer starts with y[m_end - ytail_len .. m_end)
+    const size_t k = std::min(y_max, static_cast<size_t>(p->rds_ytail_len));
+    if (k)
+        CU(cudaMemcpy(y, p->d_rds_y.get() + static_cast<size_t>(capture) * p->rds_y_len + (p->rds_ytail_len - k),
+                      k * sizeof(float2), cudaMemcpyDeviceToHost));
+    if (y_n)
+        *y_n = y_max ? k : static_cast<size_t>(p->rds_ytail_len);
+    return FMRX_OK;
+}
+
 extern "C" int fmrx_set_tuning(fmrx_pipeline *p, int capture, double offset_hz)
 {
     if (!p || capture < 0 || capture >= p->C || !(std::fabs(offset_hz) < 0.5 * p->mi.rf_fs))

@@ -7,8 +7,10 @@ table are the library's (designed in double, rounded to float); everything after
 """
 from __future__ import annotations
 
+import bisect
 import importlib
 import math
+from collections import namedtuple
 
 import numpy as np
 
@@ -70,10 +72,12 @@ class BlockSync:
 
     def __init__(self):
         self.groups = []
+        self.stamps = []           # per group: the bit count - 1 of the bit whose instant stamps it
         self.reg = 0               # the last 52 bits, newest in bit 0
         self.nbits = 0
         self.t_ring = {}
         self.synced = False
+        self.losses = 0            # times sync was lost
         self.last_hit = [-(1 << 40)] * 4
         self.pos = 0
         self.in_block = 0
@@ -84,10 +88,12 @@ class BlockSync:
         if self.cur["valid"]:
             g = self.cur
             self.groups.append((g["if_index"], tuple(g["block"]), g["valid"], g["c_prime"]))
+            self.stamps.append(g["stamp"])
 
     def _start_group(self, first_bit):
         # a group that began before the decoder's first bit takes that bit's instant
-        self.cur = {"if_index": self.t_ring[max(first_bit, 1)], "block": [0, 0, 0, 0], "valid": 0, "c_prime": 0}
+        self.cur = {"if_index": self.t_ring[max(first_bit, 1)], "block": [0, 0, 0, 0], "valid": 0, "c_prime": 0,
+                    "stamp": max(first_bit, 1) - 1}
 
     def push(self, bit: int, if_index: int):
         self.reg = ((self.reg << 1) | bit) & ((1 << 52) - 1)
@@ -144,27 +150,57 @@ class BlockSync:
             self._emit()
         if self.bad >= 8:
             self.synced = False
+            self.losses += 1
             self.last_hit = [-(1 << 40)] * 4
 
 
 class RdsOracle:
+    """``run(demod, start_n=0)`` keeps what a comparison with the device needs: ``y`` (from m = 0), ``c`` and ``tau``
+    (dicts by window index), and ``records``, one ``BitRecord`` per decided bit.  Each run starts from scratch, so
+    what an instance holds is always its latest run's."""
+
     def __init__(self, bp_fs):
         self.prm = RdsParams(bp_fs)
-        self.margins = []       # |Re(s_j s*_{j-1})| of every decided bit, for the decision-margin check
+        self._clear()
 
-    def run(self, demod: np.ndarray):
+    def _clear(self):
+        self.margins = []       # |Re(s_j s*_{j-1})| of every decided bit, for the decision-margin check
+        self.records = []
+        self.y = None
+        self.c, self.tau = {}, {}
+        self.w_first = self.j0 = 0
+        self.first = None       # (t, W) of bit j0, which only serves as the reference of bit j0 + 1
+        self.trace = []         # (synced, groups emitted) after each decided bit
+        self.sync = None
+
+    def run(self, demod: np.ndarray, start_n: int = 0):
+        """Decode ``demod`` (indexed from the stream's first sample).  ``start_n`` > 0 is the decoder restarted at
+        that sample, as fmrx_set_state does (rds_restart in fmrx_api.cu): the demod before start_n counts as zero;
+        windows stay aligned to m = 0, the first being w_first = m_r // M with m_r = ceil(start_n / D); tau is constant
+        before window w_first and is not unwrapped at it; the first bit is j0 = ceil(m_r / sps); the search starts
+        with an empty register."""
+        self._clear()
         prm = self.prm
-        y = baseband(prm, demod)
-        c = window_sums(prm, y)
+        d = np.asarray(demod, np.float64)
+        if start_n:
+            d = d.copy()
+            d[:start_n] = 0.0
+        m_r = -(-int(start_n) // prm.D)
         M, sps = prm.M, prm.sps
-        taus = []
-        sync = BlockSync()
-        j, t_prev, s_prev = 0, None, None
+        w_first = m_r // M
+        j = math.ceil(m_r / sps)
+        self.w_first, self.j0 = w_first, j
+        y = baseband(prm, d)
+        c = window_sums(prm, y)
+        self.y = y
+        taus = self.tau
+        sync = self.sync = BlockSync()
+        t_prev, s_prev = None, None
 
         def tau_at(t, W):
             a = math.floor((t - M / 2) / M)
-            if a < 0:
-                return taus[0]
+            if a < w_first:
+                return taus[w_first]
             if a >= W - 1:
                 return taus[W - 1]
             f = (t - (a * M + M / 2)) / M
@@ -173,14 +209,15 @@ class RdsOracle:
         def y_at(i):
             return y[i] if 0 <= i < len(y) else 0.0
 
-        for w in range(len(c)):
+        for w in range(w_first, len(c)):
+            self.c[w] = c[w]
             raw = -math.atan2(c[w].imag, c[w].real) / (2 * math.pi)
-            if w == 0:
-                taus.append(raw)
+            if w == w_first:
+                taus[w] = raw
             else:
-                dlt = raw - taus[-1]
+                dlt = raw - taus[w - 1]
                 dlt -= math.ceil(dlt - 0.5)
-                taus.append(taus[-1] + dlt)
+                taus[w] = taus[w - 1] + dlt
             W = w + 1
             while True:
                 t0 = t_prev + sps if t_prev is not None else j * sps
@@ -194,10 +231,57 @@ class RdsOracle:
                 if s_prev is not None:
                     r = (s * np.conj(s_prev)).real
                     self.margins.append(abs(r))
-                    sync.push(1 if r < 0 else 0, math.floor(t * prm.D + 0.5))
+                    x = t * prm.D + 0.5
+                    bit = 1 if r < 0 else 0
+                    self.records.append(BitRecord(j, t, bit, abs(r), math.floor(x), abs(x - round(x)), W))
+                    sync.push(bit, math.floor(x))
+                    self.trace.append((sync.synced, len(sync.groups)))
+                else:
+                    self.first = (t, W)
                 s_prev, t_prev = s, t
                 j += 1
         return sync.groups
+
+    def state_at(self, m_end: int) -> dict:
+        """The decoder's scalars once y[m] is known for m < m_end, as fmrx_rds_probe reports them (after run)."""
+        W_end = max(self.w_first, m_end // self.prm.M)
+        k = bisect.bisect_right([r.W for r in self.records], W_end)
+        first = self.first is not None and self.first[1] <= W_end
+        reg = 0
+        for r in self.records[max(0, k - 52):k]:
+            reg = (reg << 1) | r.bit
+        synced, written = self.trace[k - 1] if k else (False, 0)
+        return {"w_next": W_end, "j": self.j0 + int(first) + k, "nbits": k, "written": written, "reg": reg,
+                "synced": int(synced),
+                "t_prev": self.records[k - 1].t if k else (self.first[0] if first else math.nan),
+                "tau": self.tau[W_end - 1] if W_end > self.w_first else math.nan}
+
+
+BitRecord = namedtuple("BitRecord", "j t bit margin if_index tie W")
+"""One decided bit: its index j, instant t_j (units of 1/fs2), value, |Re(s_j s*_{j-1})|, if_index = floor(t_j D + 1/2),
+the distance of t_j D + 1/2 from an integer (how close if_index is to rounding the other way), and W: the bit was
+decided once windows 0 .. W-1 were complete."""
+
+
+def close_bits(records, eps_m=1e-4, span=129):
+    """Indices of the decided bits whose margin is below eps_m times the typical margin around them: the median of
+    the ``span`` bits centred on each (local, so that in a stream of quiet and loud parts each bit is judged against
+    its own part)."""
+    if not records:
+        return []
+    m = np.array([r.margin for r in records])
+    k = min(span, len(m))
+    windows = np.lib.stride_tricks.sliding_window_view(np.pad(m, (k // 2, k - 1 - k // 2), mode="edge"), k)
+    return list(np.nonzero(m < eps_m * np.median(windows, axis=1))[0])
+
+
+def well_posed(records, eps_m=1e-4, eps_t=1e-3, stamps=None):
+    """The bits of a run are far from every decision that float rounding could change: no bit with a margin below
+    eps_m times the local median margin (close_bits), and no group stamp (the bits ``stamps`` lists: BlockSync.stamps)
+    whose if_index is within eps_t of rounding the other way.  Returns (ok, indices into records of the close bits)."""
+    close = close_bits(records, eps_m)
+    ties = [k for k in (range(len(records)) if stamps is None else stamps) if records[k].tie < eps_t]
+    return not close and not ties, sorted(set(close) | set(ties))
 
 
 def decode(demod, bp_fs):

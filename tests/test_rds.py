@@ -6,6 +6,7 @@ import numpy as np
 import pytest
 
 import rds_oracle
+import test_gpu_rds_parity as parity
 
 synth = rds_oracle.synth
 OFFSETS = ("A", "B", "C", "C'", "D")
@@ -214,3 +215,100 @@ def test_rds_pipeline_without_a_device(pkg):
     with pytest.raises(fm.FmrxError) as e:
         fm.Pipeline(0, 51, 1, rds=True)
     assert e.value.status == fm.ERR_NO_DEVICE
+
+
+# ---- the oracle's records, its restart, and the inputs of tests/test_gpu_rds_parity.py -----------------------------
+
+def test_records_and_start_zero(pkg, port):
+    info, d = _demod(port, 0, 2.5, [(0.0, 2, "stereo", 256, _prog(1))])
+    o = rds_oracle.RdsOracle(info.bp_fs)
+    groups = o.run(d, start_n=0)
+    assert groups == rds_oracle.decode(d, info.bp_fs)
+    _check_stream(groups, _prog(1))
+    assert [r.j for r in o.records] == list(range(1, len(o.records) + 1))
+    assert [g[0] for g in groups] == [o.records[k].if_index for k in o.sync.stamps]
+    assert sorted(o.tau) == list(range(len(o.y) // o.prm.M))
+    end = o.state_at(len(o.y))
+    assert end["nbits"] == len(o.records) and end["written"] == len(groups) and end["synced"] == 1
+
+
+@pytest.mark.parametrize("cut", [1, 37, 38, 75])
+def test_restart_at_a_block_boundary(pkg, port, cut):
+    """run(demod, start_n): what precedes start_n is ignored, y is zero before m_r and the plain y once the filters
+    reach past start_n, the first decided bit is j0 + 1, and once in sync again the groups are the plain run's."""
+    info, d = _demod(port, 0, 3.0, [(0.0, 2, "stereo", 256, _prog(8))])
+    start_n = cut * info.if_per_block
+    plain = rds_oracle.RdsOracle(info.bp_fs)
+    all_groups = plain.run(d)
+    o = rds_oracle.RdsOracle(info.bp_fs)
+    groups = o.run(d, start_n=start_n)
+    prm = o.prm
+    m_r = -(-start_n // prm.D)
+    assert o.w_first == m_r // prm.M and o.j0 == int(np.ceil(m_r / prm.sps))
+    assert min(o.tau) == o.w_first
+    garbage = d.copy()
+    garbage[:start_n] = np.random.default_rng(cut).normal(0, 1, start_n)
+    g2 = rds_oracle.RdsOracle(info.bp_fs)
+    assert g2.run(garbage, start_n=start_n) == groups and np.array_equal(g2.y, o.y)
+    assert not np.any(o.y[:m_r])
+    reach = m_r + (prm.n_taps + prm.D - 1) // prm.D + 2 * prm.L
+    assert np.array_equal(o.y[reach:], plain.y[reach:])
+    assert o.records[0].j == o.j0 + 1 and o.state_at(m_r)["j"] == o.j0
+    assert len(groups) >= 20 and groups[0][0] >= start_n
+    tail = groups[2:]
+    k = all_groups.index(tail[0])
+    assert all_groups[k:k + len(tail)] == tail
+
+
+ORACLE_INPUTS = parity.oracle_inputs()
+
+
+@pytest.mark.parametrize("name", sorted(ORACLE_INPUTS))
+def test_gpu_parity_inputs_are_well_posed(pkg, port, name):
+    """Every fixed input tests/test_gpu_rds_parity.py compares the device with the oracle on: no bit too close to
+    call, no group stamp too close to a rounding tie, so that float rounding on the device cannot change what is
+    compared.  The chain oracle's demod is the device's, bit for bit."""
+    mode, taps, tune, make_iq, cut = ORACLE_INPUTS[name]
+    _, st = port.chain(mode, taps, tune_hz=tune).run(make_iq(), stages=("demod",))
+    o = rds_oracle.RdsOracle(port.mode(mode, taps).bp_fs)
+    groups = o.run(st["demod"], start_n=cut * port.mode(mode, taps).if_per_block)
+    ok, close = rds_oracle.well_posed(o.records, stamps=o.sync.stamps)
+    invalid = sum(4 - bin(g[2]).count("1") for g in groups)
+    print(f"{name}: {len(groups)} groups, {invalid} invalid blocks, sync lost {o.sync.losses} times, "
+          f"close bits {[(int(k), o.records[k].margin, o.records[k].tie) for k in close]}")
+    assert ok, close
+
+
+def _mutated_baseband(kind, chunk_if):
+    """rds_oracle.baseband with one kernel-like error: the mixer index one sample late, one inner tap 0.1 % high, the
+    decimation phase one sample late, or the last demod sample before every chunk boundary read as zero."""
+    def bb(prm, d):
+        d = np.asarray(d, np.float64)
+        n = np.arange(len(d), dtype=np.int64) + (1 if kind == "mix_index" else 0)
+        z = d * prm.table[(prm.q * (n % prm.P)) % prm.P]
+        taps = prm.taps.copy()
+        if kind == "tap":
+            taps[len(taps) // 2 + 5] *= 1.001
+        if kind == "tail":
+            z[np.arange(chunk_if, len(d), chunk_if) - 1] = 0.0
+        u = np.convolve(z, taps)[:len(d)][(1 if kind == "phase" else 0)::prm.D][:-(-len(d) // prm.D)]
+        return np.convolve(u, np.concatenate([np.ones(prm.L), -np.ones(prm.L)]))[:len(u)]
+    return bb
+
+
+@pytest.mark.parametrize("kind", ["mix_index", "tap", "phase", "tail"])
+def test_baseband_bound_catches_kernel_like_errors(pkg, port, monkeypatch, kind):
+    """Each error, applied to the oracle in place of the same bug in k_rds_baseband, breaks the y bound of
+    tests/test_gpu_rds_parity.py by far.  Whether it also changes the groups is printed: the mixer index and the tap
+    leave them unchanged, which is why the groups alone are not enough."""
+    info, d = _demod(port, 0, 3.0, [(0.0, 2, "stereo", 256, _prog(1))])
+    o = rds_oracle.RdsOracle(info.bp_fs)
+    groups = o.run(d)
+    y = o.y
+    monkeypatch.setattr(rds_oracle, "baseband", _mutated_baseband(kind, 16 * info.if_per_block))
+    bad = rds_oracle.RdsOracle(info.bp_fs)
+    bad_groups = bad.run(d)
+    dy = np.max(np.abs(bad.y - y)) / np.sqrt(np.mean(np.abs(y) ** 2))
+    print(f"{kind}: max|dy|/rms {dy:.3g}; groups {'unchanged' if bad_groups == groups else 'changed'}")
+    assert len(bad.y) == len(y)
+    assert dy > 10 * parity.EPS_Y
